@@ -21,6 +21,9 @@ maps, 5..15 pedestrians, map re-drawn at reset; every N -- at N=8 this IS config
 and her (the HER batch kernel with its HBM roofline; N=1).
 `--impl reference` times the CPU restatement of the reference's path (oracle/, OpenMP over all
 host cores) on the same world with the same 4096 environments per step.
+`--dump-outputs DIR` writes what the last timed step of the headline leg returned to its caller
+(obs, reward, done and the info fields) as DIR/<name>.npy in float32; inputs are seeded, so two
+builds run with the same arguments can be compared output for output.
 """
 import argparse
 import json
@@ -34,6 +37,7 @@ import numpy as np
 
 ROOT = os.path.dirname(os.path.abspath(__file__))
 sys.path.insert(0, ROOT)
+sys.dont_write_bytecode = True   # the benchmark leaves the tree it runs from untouched
 
 ENVS_PER_GPU = 4096
 NB = 512
@@ -201,6 +205,31 @@ def device_leg(torch, env, policy, K, W, flush=None, barrier=None):
     else:
         torch.cuda.synchronize(env.device)
     return np.array([s.elapsed_time(e) for s, e in ev]), int(lib.navgym_launch_count() - l0)
+
+
+DUMP_BYTES = 60 << 20   # --dump-outputs budget, all files together
+
+
+def step_outputs(env):
+    """Host copies, as float32, of what env.step returned: the env's own buffers (obs, reward,
+    done, info), which the next step overwrites.  Flags and step counts are exact in float32."""
+    out = {'obs': env.obs, 'reward': env.reward, 'done': env.done, 'is_success': env.is_success,
+           'is_crash': env.is_crash, 'distance': env.distance, 'episode_step': env.steps,
+           'truncated': env.truncated}
+    return {k: v.float().cpu().numpy() for k, v in out.items()}
+
+
+def dump_outputs(out_dir, arrays):
+    """arrays: {name: [B, ...]} -> out_dir/<name>.npy.  Beyond DUMP_BYTES in all, every array keeps
+    the same environments: a fixed, seeded sample of rows in ascending order."""
+    B = len(arrays['obs'])
+    row_bytes = sum(a[:1].nbytes for a in arrays.values())
+    rows = np.arange(B)
+    if B * row_bytes > DUMP_BYTES:
+        rows = np.sort(np.random.RandomState(0).choice(B, DUMP_BYTES // row_bytes, replace=False))
+    os.makedirs(out_dir, exist_ok=True)
+    for name, a in arrays.items():
+        np.save(os.path.join(out_dir, name + '.npy'), np.ascontiguousarray(a[rows]))
 
 
 def gather_block(B, ms, gathers_per_env_step, source):
@@ -381,7 +410,11 @@ def main():
     ap.add_argument('--no-flush', action='store_true')
     ap.add_argument('--no-configs', action='store_true', help='skip the c3 / c4 / c5 block')
     ap.add_argument('--no-e2e', action='store_true', help='skip the host-buffer legs (profiling runs)')
+    ap.add_argument('--dump-outputs', metavar='DIR',
+                    help="write the last timed step's outputs (rank 0's environments) as DIR/<name>.npy")
     a = ap.parse_args()
+    if a.dump_outputs and a.impl != 'native':
+        ap.error('--dump-outputs writes the outputs of the native arm')
     a.warmup = max(a.warmup, 3)
     rank = int(os.environ.get('RANK', '0'))
     world = int(os.environ.get('WORLD_SIZE', '1'))
@@ -467,6 +500,7 @@ def main():
     total_ms = float(step_ms.sum())
     crash_frac = float(env.is_crash.float().mean().item())
     done_frac = float(env.done.float().mean().item())
+    outputs = step_outputs(env) if a.dump_outputs and rank == 0 else None   # before the e2e legs step env
 
     # ---- end-to-end legs: HOST buffers, copies inside the timed region ----------------------
     # (a) rollout: the env groups rotate in C (navgym_host_rollout): per group H2D actions ->
@@ -631,6 +665,8 @@ def main():
         line["configs"] = cfg
     if not a.no_cpu_baseline and world == 1:
         line["cpu_baseline"] = cpu_baseline_block()
+    if outputs is not None:
+        dump_outputs(a.dump_outputs, outputs)
     print(json.dumps(line))
     if world > 1:
         dist.destroy_process_group()

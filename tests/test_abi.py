@@ -50,8 +50,14 @@ def test_no_cpu_fallback(lib):
         BatchedNavGym(1, [m])
 
 
-def test_sass_is_sm100a():
-    out = os.popen('cuobjdump -lelf %s 2>/dev/null' % _lib.SO).read()
+def test_sass_is_sm100a(lib):
+    import subprocess
+    # the cuobjdump of the toolkit whose nvcc built the library, found the same way (PATH or
+    # /usr/local/cuda/bin)
+    nvcc = _lib._nvcc()
+    assert nvcc is not None
+    cuobjdump = os.path.join(os.path.dirname(nvcc), 'cuobjdump')
+    out = subprocess.run([cuobjdump, '-lelf', _lib.SO], capture_output=True, text=True, check=True).stdout
     assert 'sm_100a' in out
 
 
