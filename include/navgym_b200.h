@@ -378,11 +378,11 @@ int navgym_policy_features(const float *scan, int n, const float *w1, const floa
  *   feat = the convolutional front end of navgym_policy_features on the pedestrian's newest scan
  *          (env.py:647 feeds it to all three input frames; the fold is done here from the
  *          reference-shaped act_fea_cv1 weight).
- * Three launches, no library GEMM: the front end (features leave as two f16 halves), act_fc1 on
- * the tcgen05 tensor cores with TMA-fed operands and TMEM accumulators in the "f16x3" scheme
- * (hi/lo f16 splits of both operands, three MMAs per K step: float32-grade results), act_fc2 and
- * the heads on the CUDA cores.  Parameters are float32 device pointers in torch's state_dict
- * layout; they are copied / pre-split into the caller's workspace by navgym_policy_create, so
+ * Three launches, no library GEMM, every contraction on the tcgen05 tensor cores in the "f16x3"
+ * scheme (hi/lo f16 splits of both operands, three MMAs per K step: float32-grade results): the
+ * front end (features leave as two f16 halves), act_fc1 with TMA-fed operands and TMEM
+ * accumulators, act_fc2 with the heads in its epilogue.  Parameters are float32 device pointers
+ * in torch's state_dict layout; they are copied / pre-split into the caller's workspace by navgym_policy_create, so
  * changing the weights means creating a new policy.  workspace: device memory, 1024-byte
  * aligned, navgym_policy_workspace_bytes(max_n) bytes (the feature halves dominate: 16 KB per
  * pedestrian), owned by the caller and kept alive for the policy's lifetime. */
@@ -406,10 +406,10 @@ void navgym_policy_destroy(navgym_policy_t *policy);
  * [n][2] (env.py:641-645), speed f32 [n][2] (the previous clipped mean) -> mean f32 [n][2]. */
 int navgym_policy_mean(navgym_policy_t *policy, const float *scan, const float *goal,
                        const float *speed, int n, float *mean, void *stream);
-/* byte offsets inside the workspace of {features hi, features lo, act_fc1 output as float32 (written
- * by the comparison path NAVGYM_POLICY_FC2=1 only), scales, total, act_fc1 output hi, lo (f16 pairs
- * times scales[6])} (tests compare the intermediate results against a float32 reference) */
-void navgym_policy_workspace_layout(int max_n, uint64_t *out7);
+/* byte offsets inside the workspace of {features hi, features lo, scales, total, act_fc1 output
+ * hi, lo (f16 pairs times scales[6])} (tests compare the intermediate results against a float32
+ * reference) */
+void navgym_policy_workspace_layout(int max_n, uint64_t *out6);
 
 /* ---- inner native boundary: range_libc --------------------------------------------- */
 /* PyOMap(bool[H,W]) + PyRayMarching(omap, max_range) (env.py:337-340): exact Euclidean

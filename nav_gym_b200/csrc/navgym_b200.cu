@@ -231,10 +231,7 @@ navgym_policy_t *navgym_policy_create(const navgym_policy_params_t *p, void *str
          policy_make_map(&pol->tm_w2l, pol->ws + L.w2l, 128, 128, 256) == 0;
     ok = ok && cudaFuncSetAttribute(dense_umma_kernel<pg::Fc1, 0>, cudaFuncAttributeMaxDynamicSharedMemorySize, pg::Fc1::SMEM_BYTES) == cudaSuccess &&
          cudaFuncSetAttribute(dense_umma_kernel<pg::Fc2, 1>, cudaFuncAttributeMaxDynamicSharedMemorySize, pg::Fc2::SMEM_BYTES) == cudaSuccess &&
-         cudaFuncSetAttribute(policy_features_umma_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, pc::SMEM_BYTES) == cudaSuccess &&
-         cudaFuncSetAttribute(policy_features_umma2_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, pf::SMEM_BYTES) == cudaSuccess &&
-         cudaFuncSetAttribute(fc2_heads_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize,
-                              (PF2_IN * 128 + 64 * PF2_ROW) * (int)sizeof(float)) == cudaSuccess;
+         cudaFuncSetAttribute(policy_features_umma2_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, pf::SMEM_BYTES) == cudaSuccess;
     if (ok) {
         policy_prepare_kernel<<<1, 1024, 0, st>>>(*p, pol->ws, L);
         g_launches++;
@@ -256,42 +253,26 @@ int navgym_policy_mean(navgym_policy_t *pol, const float *scan, const float *goa
     uint8_t *ws = pol->ws;
     const policy_ws_t &L = pol->L;
     const float *scales = (const float *)(ws + L.scales);
-    // front end: both convolutions on the tensor cores (2, default) or conv1 on the CUDA cores (1)
-    static const int front = env_int("NAVGYM_POLICY_FRONT", 2);
-    if (front == 2)
-        policy_features_umma2_kernel<<<n < pol->sms ? n : pol->sms, pf::THREADS, pf::SMEM_BYTES, st>>>(
-            scan, n, (const uint4 *)(ws + L.conv1_img), (const uint4 *)(ws + L.conv2_img), (const float *)(ws + L.b2), scales,
-            (__half *)(ws + L.fh), (__half *)(ws + L.fl));
-    else
-        policy_features_umma_kernel<<<n < pol->sms ? n : pol->sms, pc::THREADS, pc::SMEM_BYTES, st>>>(
-            scan, n, (const uint4 *)(ws + L.conv_img), (const float *)(ws + L.w1s), (const float *)(ws + L.b2), scales,
-            (__half *)(ws + L.fh), (__half *)(ws + L.fl));
-    // act_fc1, then act_fc2 + heads: both on the tensor cores (default), or act_fc2 + heads on the CUDA cores
-    // from a float32 copy of act_fc1's output (NAVGYM_POLICY_FC2=1, the comparison path)
-    static const int fc2_mode = env_int("NAVGYM_POLICY_FC2", 2);
+    // front end (both convolutions), act_fc1, then act_fc2 + heads: all on the tensor cores
+    policy_features_umma2_kernel<<<n < pol->sms ? n : pol->sms, pf::THREADS, pf::SMEM_BYTES, st>>>(
+        scan, n, (const uint4 *)(ws + L.conv1_img), (const uint4 *)(ws + L.conv2_img), (const float *)(ws + L.b2), scales,
+        (__half *)(ws + L.fh), (__half *)(ws + L.fl));
     const int tiles = (n + pg::BM - 1) / pg::BM, grid = tiles < pol->sms ? tiles : pol->sms;
     dense_umma_kernel<pg::Fc1, 0><<<grid, pg::THREADS, pg::Fc1::SMEM_BYTES, st>>>(
         pol->tm_fh, pol->tm_fl, pol->tm_wh, pol->tm_wl, (const float *)(ws + L.fc1_b), scales, n, tiles,
-        fc2_mode == 2 ? nullptr : (float *)(ws + L.h), (__half *)(ws + L.hh), (__half *)(ws + L.hl), nullptr, nullptr, nullptr);
-    if (fc2_mode == 2) {
-        dense_umma_kernel<pg::Fc2, 1><<<grid, pg::THREADS, pg::Fc2::SMEM_BYTES, st>>>(
-            pol->tm_hh, pol->tm_hl, pol->tm_w2h, pol->tm_w2l, (const float *)(ws + L.fc2_tab), scales, n, tiles,
-            nullptr, nullptr, nullptr, goal, speed, mean);
-    } else {
-        const int tiles2 = (n + 63) / 64;
-        fc2_heads_kernel<<<tiles2 < pol->sms ? tiles2 : pol->sms, 256, (PF2_IN * 128 + 64 * PF2_ROW) * sizeof(float), st>>>(
-            (const float *)(ws + L.h), goal, speed, n, (const float *)(ws + L.w2t), (const float *)(ws + L.fc2_b),
-            (const float *)(ws + L.heads), mean);
-    }
+        (__half *)(ws + L.hh), (__half *)(ws + L.hl), nullptr, nullptr, nullptr);
+    dense_umma_kernel<pg::Fc2, 1><<<grid, pg::THREADS, pg::Fc2::SMEM_BYTES, st>>>(
+        pol->tm_hh, pol->tm_hl, pol->tm_w2h, pol->tm_w2l, (const float *)(ws + L.fc2_tab), scales, n, tiles,
+        nullptr, nullptr, goal, speed, mean);
     g_launches += 3;
     return (int)cudaGetLastError();
 }
 
 /* test hook: byte offsets of the intermediate buffers inside the workspace */
-void navgym_policy_workspace_layout(int max_n, uint64_t *out /* [7]: fh, fl, h (float32, comparison path only), scales, total, hh, hl */)
+void navgym_policy_workspace_layout(int max_n, uint64_t *out /* [6]: fh, fl, scales, total, hh, hl */)
 {
     const policy_ws_t L = policy_ws_layout(max_n);
-    out[0] = L.fh; out[1] = L.fl; out[2] = L.h; out[3] = L.scales; out[4] = L.total; out[5] = L.hh; out[6] = L.hl;
+    out[0] = L.fh; out[1] = L.fl; out[2] = L.scales; out[3] = L.total; out[4] = L.hh; out[5] = L.hl;
 }
 
 int navgym_peds_move(const navgym_move_args_t *args, void *stream)

@@ -1,15 +1,15 @@
 // policy_gemm.cuh -- part of navgym_b200.cu (included there; one translation unit).
-// The dense half of the pedestrian policy (human_policy.py:38-55 `act_fc1`, `act_fc2`, `actor1`,
-// `actor2`; called from env.py:649-656) as sm_100a kernels:
+// The pedestrian policy's action mean (human_policy.py:38-55; called from env.py:649-656) as three
+// sm_100a launches per forward, every contraction on the 5th-generation tensor cores (the weights
+// are laid out for them once, by policy_prepare_kernel):
 //
+//   policy_features_umma2_kernel  the convolutional front end: scan -> features F [n][4096] as f16 pairs.
 //   dense_umma_kernel   <Fc1, 0>: H = relu(F W1^T + b1), F [n][4096], W1 [256][4096]: the big dense contraction of
-//                       the system, on the 5th-generation tensor cores; <Fc2, 1>: act_fc2 + the two heads (N 128, K 256).  tcgen05.mma (kind::f16,
+//                       the system; <Fc2, 1>: act_fc2 + the two heads (N 128, K 256).  tcgen05.mma (kind::f16,
 //                       M 128 x N 256 x K 16 per instruction, issued by one thread), operands staged
-//                       in shared memory by TMA (cp.async.bulk.tensor, 128-byte swizzle),
+//                       in shared memory by TMA (cp.async.bulk.tensor, 64-byte swizzle),
 //                       accumulators in tensor memory (2 x 256 columns: the epilogue of one tile
 //                       overlaps the main loop of the next), read back with tcgen05.ld.
-//   fc2_heads_kernel    mean = (sigmoid, tanh)(actor(relu(fc2([h, goal, speed])))) in float32 on
-//                       the CUDA cores (33 k FMA per pedestrian; 3 % of the policy's arithmetic).
 //
 // Float32-grade results from the f16 tensor pipe ("f16x3"): every float32 operand x is carried as
 // two halves, hi = half(x * s) and lo = half(x * s - hi) with s a power of two chosen from the
@@ -29,20 +29,16 @@
 #include <cuda_fp16.h>
 
 namespace pg {
-#ifndef NAVGYM_FC1_BK
-#define NAVGYM_FC1_BK 32
-#endif
-// K block of a pipeline stage: 64 f16 = 128-byte rows (128-byte swizzle, 2 stages of 96 KB) or
-// 32 f16 = 64-byte rows (64-byte swizzle, 4 stages of 48 KB: the same bytes per MMA cycle, but
-// three stages in flight instead of one while a stage is being multiplied)
-constexpr int BM = 128, BK = NAVGYM_FC1_BK, UK = 16;
-static_assert(BK == 64 || BK == 32, "K block = one swizzle row");
+// K block of a pipeline stage: 32 f16 = 64-byte rows (64-byte swizzle, 4 stages of 48 KB: the same
+// bytes per MMA cycle as 64-wide blocks in 2 stages of 96 KB, but three stages in flight instead of
+// one while a stage is being multiplied)
+constexpr int BM = 128, BK = 32, UK = 16;
 // one dense layer on the tensor cores: BN outputs, KDIM inputs (act_fc1: 256 x 4096; act_fc2: 128 x 256)
 template <int BN_, int KDIM_>
 struct Dense {
     static constexpr int BN = BN_, KDIM = KDIM_, KB = KDIM_ / BK;
     static constexpr int WBOX = BN_ > 128 ? 64 : BN_;   // weight rows per TMA box (a leftover tile's N parts are multiples of it)
-    static constexpr uint32_t A_BYTES = BM * BK * 2;                      // 128 rows x (128 | 64) B
+    static constexpr uint32_t A_BYTES = BM * BK * 2;                      // 128 rows x 64 B
     static constexpr uint32_t B_BYTES = BN_ * BK * 2;
     static constexpr uint32_t STAGE_BYTES = 2 * A_BYTES + 2 * B_BYTES;    // A hi, A lo, W hi, W lo
     static constexpr int STAGES = (192 * 1024) / STAGE_BYTES;
@@ -99,23 +95,13 @@ __device__ __forceinline__ void umma_commit(uint32_t bar)
 {
     asm volatile("tcgen05.commit.cta_group::1.mbarrier::arrive::one.shared::cluster.b64 [%0];" ::"r"(bar) : "memory");
 }
-// Shared-memory matrix descriptor of a K-major tile whose rows are 128 bytes, laid out by TMA
-// with the 128-byte swizzle: 8-row groups 1024 B apart (stride byte offset), descriptor version
-// 1 (sm_100), layout type 2 (SWIZZLE_128B); the leading byte offset is unused for this layout.
-__device__ __forceinline__ uint64_t umma_desc_sw128(uint32_t smem_addr)
-{
-    return (uint64_t)((smem_addr & 0x3FFFFu) >> 4) | ((uint64_t)1 << 16) | ((uint64_t)(1024 >> 4) << 32) |
-           ((uint64_t)1 << 46) | ((uint64_t)2 << 61);
-}
-// The same for 64-byte rows with the 64-byte swizzle: 8-row groups 512 B apart, layout type 4.
+// Shared-memory matrix descriptor of a K-major tile whose rows are 64 bytes, laid out by TMA
+// with the 64-byte swizzle: 8-row groups 512 B apart (stride byte offset), descriptor version
+// 1 (sm_100), layout type 4 (SWIZZLE_64B); the leading byte offset is unused for this layout.
 __device__ __forceinline__ uint64_t umma_desc_sw64(uint32_t smem_addr)
 {
     return (uint64_t)((smem_addr & 0x3FFFFu) >> 4) | ((uint64_t)1 << 16) | ((uint64_t)(512 >> 4) << 32) |
            ((uint64_t)1 << 46) | ((uint64_t)4 << 61);
-}
-__device__ __forceinline__ uint64_t umma_desc_fc1(uint32_t smem_addr)
-{
-    return BK == 64 ? umma_desc_sw128(smem_addr) : umma_desc_sw64(smem_addr);
 }
 __device__ __forceinline__ void tmem_ld32(uint32_t taddr, uint32_t (&v)[32])
 {
@@ -148,8 +134,7 @@ __device__ __forceinline__ void split2(float a, float b, uint32_t &hi, uint32_t 
 // dense_umma_kernel<L, EPI>: Y = A W^T in the f16x3 scheme, A = (a_hi, a_lo) [n][KDIM] and W = (w_hi, w_lo)
 // [BN][KDIM] f16 pairs behind TMA maps; 128-row tiles, persistent over tiles.
 //   EPI 0 (act_fc1): h = relu(Y descale + bias), written as f16 hi/lo pairs times s_h2 -- the A operand of the
-//          act_fc2 launch -- and, if h32 != NULL, as float32 (the comparison path fc2_heads_kernel reads it);
-//          scales[1] = descale, scales[6] = s_h2.
+//          act_fc2 launch; scales[1] = descale, scales[6] = s_h2.
 //   EPI 1 (act_fc2 + heads, human_policy.py:51-55): y = relu(Y descale + b2 + [goal, speed] . w2[:, 256:260]),
 //          mean = (sigmoid(y . a1 + a1_b), tanh(y . a2 + a2_b)); tab = [7][128] b2, the four extra input columns
 //          of fc2's weight, a1_w, a2_w, then a1_b, a2_b; scales[7] = descale.  One thread per pedestrian.
@@ -158,7 +143,7 @@ __global__ void __launch_bounds__(pg::THREADS, 1)
 dense_umma_kernel(const __grid_constant__ CUtensorMap tm_ah, const __grid_constant__ CUtensorMap tm_al,
                   const __grid_constant__ CUtensorMap tm_wh, const __grid_constant__ CUtensorMap tm_wl,
                   const float *__restrict__ bias_or_tab, const float *__restrict__ scales, int n, int num_tiles,
-                  float *__restrict__ h32, __half *__restrict__ h_hi, __half *__restrict__ h_lo,
+                  __half *__restrict__ h_hi, __half *__restrict__ h_lo,
                   const float *__restrict__ goal, const float *__restrict__ speed, float *__restrict__ mean)
 {
     using namespace pg;
@@ -236,8 +221,8 @@ dense_umma_kernel(const __grid_constant__ CUtensorMap tm_ah, const __grid_consta
                     mbar_wait(full0 + 8 * s, ph);
                     tc_fence_after();
                     const uint32_t st = base + s * STAGE_BYTES;
-                    const uint64_t fh = umma_desc_fc1(st), fl = umma_desc_fc1(st + A_BYTES);
-                    const uint64_t wh = umma_desc_fc1(st + 2 * A_BYTES), wl = umma_desc_fc1(st + 2 * A_BYTES + B_BYTES);
+                    const uint64_t fh = umma_desc_sw64(st), fl = umma_desc_sw64(st + A_BYTES);
+                    const uint64_t wh = umma_desc_sw64(st + 2 * A_BYTES), wl = umma_desc_sw64(st + 2 * A_BYTES + B_BYTES);
 #pragma unroll
                     for (int k = 0; k < BK / UK; k++) {
                         const uint64_t adv = (uint64_t)((k * UK * 2) >> 4);   // 32 bytes along K inside the swizzle atom
@@ -279,7 +264,6 @@ dense_umma_kernel(const __grid_constant__ CUtensorMap tm_ah, const __grid_consta
                             o.y = fmaxf(fmaf(__uint_as_float(v[j + 1]), descale, b.y), 0.0f);
                             o.z = fmaxf(fmaf(__uint_as_float(v[j + 2]), descale, b.z), 0.0f);
                             o.w = fmaxf(fmaf(__uint_as_float(v[j + 3]), descale, b.w), 0.0f);
-                            if (h32) *reinterpret_cast<float4 *>(h32 + (size_t)row * BN + col + j) = o;
                             split2(o.x * s_h2, o.y * s_h2, hi[j >> 1], lo[j >> 1]);
                             split2(o.z * s_h2, o.w * s_h2, hi[(j >> 1) + 1], lo[(j >> 1) + 1]);
                         }
@@ -343,95 +327,13 @@ dense_umma_kernel(const __grid_constant__ CUtensorMap tm_ah, const __grid_consta
     }
 }
 
-// ------------------------------------------------------------------ fc2 + actor heads
-// 256 threads = 16 pedestrian groups (4 pedestrians each) x 16 output groups (2 x 4 of the 128 fc2
-// outputs each): a 64-pedestrian tile per pass, the transposed fc2 weight (260 x 128) resident in
-// shared memory for the CTA's lifetime; the two heads are 16-lane shuffle reductions.
-#define PF2_IN 260
-#define PF2_ROW 261   // row pitch of the staged inputs (odd: the 16 pedestrian groups hit different banks)
-__global__ void __launch_bounds__(256, 1)
-fc2_heads_kernel(const float *__restrict__ H, const float *__restrict__ goal, const float *__restrict__ speed, int n,
-                 const float *__restrict__ w2t /* [260][128] */, const float *__restrict__ b2,
-                 const float *__restrict__ heads /* a1_w[128] a2_w[128] a1_b a2_b */, float *__restrict__ mean)
-{
-    extern __shared__ __align__(16) float fsm[];
-    float *ws = fsm;                   // [260][128]
-    float *xs = fsm + PF2_IN * 128;    // [64][261]
-    const int t = threadIdx.x, og = t & 15, pg_ = t >> 4;
-    for (int i = t; i < PF2_IN * 128 / 4; i += 256) reinterpret_cast<float4 *>(ws)[i] = reinterpret_cast<const float4 *>(w2t)[i];
-    float bo[8], h1w[8], h2w[8];
-#pragma unroll
-    for (int j = 0; j < 8; j++) {   // this thread's outputs: 4 og .. 4 og + 3 and 64 + 4 og .. (conflict-free LDS.128)
-        const int o = (j >> 2) * 64 + og * 4 + (j & 3);
-        bo[j] = b2[o]; h1w[j] = heads[o]; h2w[j] = heads[128 + o];
-    }
-    const float hb1 = heads[256], hb2 = heads[257];
-    const int tiles = (n + 63) / 64;
-    for (int tile = blockIdx.x; tile < tiles; tile += gridDim.x) {
-        __syncthreads();
-        const int p0 = tile * 64;
-        for (int i = t; i < 64 * 64; i += 256) {   // 64 rows x 64 float4
-            const int r = i >> 6, c4 = i & 63;
-            float4 v = make_float4(0.f, 0.f, 0.f, 0.f);
-            if (p0 + r < n) v = *reinterpret_cast<const float4 *>(H + (size_t)(p0 + r) * 256 + c4 * 4);
-            float *d = xs + r * PF2_ROW + c4 * 4;
-            d[0] = v.x; d[1] = v.y; d[2] = v.z; d[3] = v.w;
-        }
-        if (t < 64) {   // torch.cat((a, goal, speed)) (human_policy.py:51)
-            float *d = xs + t * PF2_ROW + 256;
-            const bool ok = p0 + t < n;
-            d[0] = ok ? goal[2 * (size_t)(p0 + t)] : 0.f;  d[1] = ok ? goal[2 * (size_t)(p0 + t) + 1] : 0.f;
-            d[2] = ok ? speed[2 * (size_t)(p0 + t)] : 0.f; d[3] = ok ? speed[2 * (size_t)(p0 + t) + 1] : 0.f;
-        }
-        __syncthreads();
-        float acc[4][8];
-#pragma unroll
-        for (int p = 0; p < 4; p++)
-#pragma unroll
-            for (int j = 0; j < 8; j++) acc[p][j] = bo[j];
-        const float *xr = xs + (pg_ * 4) * PF2_ROW;
-#pragma unroll 4
-        for (int k = 0; k < PF2_IN; k++) {
-            const float4 wa = *reinterpret_cast<const float4 *>(ws + k * 128 + og * 4);
-            const float4 wb = *reinterpret_cast<const float4 *>(ws + k * 128 + 64 + og * 4);
-            const float wv[8] = {wa.x, wa.y, wa.z, wa.w, wb.x, wb.y, wb.z, wb.w};
-#pragma unroll
-            for (int p = 0; p < 4; p++) {
-                const float x = xr[p * PF2_ROW + k];
-#pragma unroll
-                for (int j = 0; j < 8; j++) acc[p][j] = fmaf(x, wv[j], acc[p][j]);
-            }
-        }
-#pragma unroll
-        for (int p = 0; p < 4; p++) {
-            float s1 = 0.f, s2 = 0.f;
-#pragma unroll
-            for (int j = 0; j < 8; j++) {
-                const float a = fmaxf(acc[p][j], 0.0f);
-                s1 = fmaf(a, h1w[j], s1);
-                s2 = fmaf(a, h2w[j], s2);
-            }
-#pragma unroll
-            for (int o = 8; o > 0; o >>= 1) {
-                s1 += __shfl_xor_sync(0xffffffffu, s1, o);
-                s2 += __shfl_xor_sync(0xffffffffu, s2, o);
-            }
-            const int ped = p0 + pg_ * 4 + p;
-            if (og == 0 && ped < n) {   // human_policy.py:53-55: sigmoid / tanh heads
-                mean[2 * (size_t)ped] = 1.0f / (1.0f + expf(-(s1 + hb1)));
-                mean[2 * (size_t)ped + 1] = tanhf(s2 + hb2);
-            }
-        }
-    }
-}
-
 // ------------------------------------------------------------------ weight preparation
 // One CTA, run once per set of weights: folds the first convolution's three identical input
-// frames (env.py:647), transposes conv2 / fc2 for the kernels' access order, and chooses the two
-// power-of-two scales of the f16x3 scheme from bounds on the features and the fc1 weights.
+// frames (env.py:647), lays the weights out as the kernels' operands, and chooses the
+// power-of-two scales of the f16x3 scheme from bounds on the activations and the weights.
+constexpr int FC2_IN = 256 + 2 + 2;   // act_fc2's inputs: act_fc1's output, goal, speed (human_policy.py:51)
 struct policy_ws_t {   // device workspace layout (byte offsets from the workspace base)
-    size_t fh, fl, wh, wl, h, w1f, b1, w2, b2, fc1_b, w2t, fc2_b, heads, scales, conv_img, w1s, conv1_img, conv2_img,
-        hh, hl, w2h, w2l, fc2_tab, total;
+    size_t fh, fl, wh, wl, w1f, b1, w2, b2, fc1_b, scales, conv1_img, conv2_img, hh, hl, w2h, w2l, fc2_tab, total;
 };
 static policy_ws_t policy_ws_layout(int max_n)
 {
@@ -441,11 +343,9 @@ static policy_ws_t policy_ws_layout(int max_n)
     auto take = [&](size_t bytes) { size_t at = o; o += (bytes + 1023) / 1024 * 1024; return at; };
     L.fh = take(np * 4096 * 2); L.fl = take(np * 4096 * 2);
     L.wh = take((size_t)256 * 4096 * 2); L.wl = take((size_t)256 * 4096 * 2);
-    L.h = take(np * 256 * 4);
     L.w1f = take(160 * 4); L.b1 = take(32 * 4); L.w2 = take(3072 * 4); L.b2 = take(32 * 4);
-    L.fc1_b = take(256 * 4); L.w2t = take((size_t)PF2_IN * 128 * 4); L.fc2_b = take(128 * 4);
-    L.heads = take(258 * 4); L.scales = take(64);
-    L.conv_img = take(16384); L.w1s = take(256 * 4); L.conv1_img = take(6144); L.conv2_img = take(12288);
+    L.fc1_b = take(256 * 4); L.scales = take(64);
+    L.conv1_img = take(6144); L.conv2_img = take(12288);
     L.hh = take(np * 256 * 2); L.hl = take(np * 256 * 2);                       // act_fc1's output as f16 pairs
     L.w2h = take(128 * 256 * 2); L.w2l = take(128 * 256 * 2); L.fc2_tab = take(898 * 4);
     L.total = o;
@@ -465,16 +365,6 @@ __global__ void __launch_bounds__(1024) policy_prepare_kernel(const navgym_polic
     if (t < 32) { b1[t] = p.cv1_b[t]; b2[t] = p.cv2_b[t]; }
     for (int i = t; i < 3072; i += 1024) w2[i] = p.cv2_w[i];
     for (int i = t; i < 256; i += 1024) ((float *)(ws + L.fc1_b))[i] = p.fc1_b[i];
-    for (int i = t; i < PF2_IN * 128; i += 1024) {   // fc2 weight [128][260] -> [260][128]
-        const int k = i / 128, o = i % 128;
-        ((float *)(ws + L.w2t))[i] = p.fc2_w[o * PF2_IN + k];
-    }
-    if (t < 128) {
-        ((float *)(ws + L.fc2_b))[t] = p.fc2_b[t];
-        ((float *)(ws + L.heads))[t] = p.a1_w[t];
-        ((float *)(ws + L.heads))[128 + t] = p.a2_w[t];
-    }
-    if (t == 0) { ((float *)(ws + L.heads))[256] = p.a1_b[0]; ((float *)(ws + L.heads))[257] = p.a2_b[0]; }
     __syncthreads();
     // bound on conv1 outputs (inputs lie in [-0.5, 0.5]: env.py:627-629) and on the features
     if (t == 0) {
@@ -549,7 +439,7 @@ __global__ void __launch_bounds__(1024) policy_prepare_kernel(const navgym_polic
             frexpf(m, &e);
             s_h2 = ldexpf(1.0f, min(max(15 - e, -100), 100));
             float wm = 1e-30f;
-            for (int i = 0; i < 128 * PF2_IN; i++) if (i % PF2_IN < 256) wm = fmaxf(wm, fabsf(p.fc2_w[i]));
+            for (int i = 0; i < 128 * FC2_IN; i++) if (i % FC2_IN < 256) wm = fmaxf(wm, fabsf(p.fc2_w[i]));
             frexpf(wm, &e);
             s_w2fc = ldexpf(1.0f, min(max(14 - e, -100), 100));
             float *sc = (float *)(ws + L.scales);
@@ -560,7 +450,7 @@ __global__ void __launch_bounds__(1024) policy_prepare_kernel(const navgym_polic
         __half *w2h = (__half *)(ws + L.w2h), *w2l = (__half *)(ws + L.w2l);
         for (int i = t; i < 128 * 256; i += 1024) {
             const int o = i >> 8, k = i & 255;
-            const float x = p.fc2_w[o * PF2_IN + k] * s_w2fc;
+            const float x = p.fc2_w[o * FC2_IN + k] * s_w2fc;
             const __half hi = __float2half_rn(x);
             w2h[i] = hi;
             w2l[i] = __float2half_rn(x - __half2float(hi));
@@ -568,7 +458,7 @@ __global__ void __launch_bounds__(1024) policy_prepare_kernel(const navgym_polic
         float *tab = (float *)(ws + L.fc2_tab);
         if (t < 128) {
             tab[t] = p.fc2_b[t];
-            for (int e = 0; e < 4; e++) tab[128 * (1 + e) + t] = p.fc2_w[t * PF2_IN + 256 + e];
+            for (int e = 0; e < 4; e++) tab[128 * (1 + e) + t] = p.fc2_w[t * FC2_IN + 256 + e];
             tab[640 + t] = p.a1_w[t];
             tab[768 + t] = p.a2_w[t];
         }
@@ -585,11 +475,6 @@ __global__ void __launch_bounds__(1024) policy_prepare_kernel(const navgym_polic
         const __half hi = __float2half_rn(x);
         wh[i] = hi;
         wl[i] = __float2half_rn(x - __half2float(hi));
-    }
-    // conv1 taps + bias, scaled: [32][8] = w0..w3 | w4, bias, 0, 0
-    if (t < 256) {
-        const int c = t >> 3, k = t & 7;
-        ((float *)(ws + L.w1s))[t] = k < 5 ? w1f[c * 5 + k] * s_h_scale : (k == 5 ? b1[c] * s_h_scale : 0.0f);
     }
     // Operand images of policy_features_umma2_kernel, byte for byte as they sit in shared memory.
     // conv1 as a GEMM per pedestrian, D1[pos][n = 3 c + tap] = conv1 output 2 pos - 1 + tap of channel c:
@@ -629,19 +514,6 @@ __global__ void __launch_bounds__(1024) policy_prepare_kernel(const navgym_polic
             img2[(2048u + off) >> 1] = __float2half_rn(x - __half2float(hi));
         }
     }
-    // conv2's weight as the B operand of policy_features_umma_kernel, byte for byte as it sits in
-    // shared memory: hi | lo, each two K blocks of [32 co][64] f16, K index = 4 ci + tap (tap 3 =
-    // 0), K-major rows of 128 bytes in 8-row groups with the 128-byte swizzle
-    __half *img = (__half *)(ws + L.conv_img);
-    for (int i = t; i < 32 * 32 * 4; i += 1024) {
-        const int co = i >> 7, ci = (i >> 2) & 31, tap = i & 3;
-        const float x = tap < 3 ? w2[(co * 32 + ci) * 3 + tap] * s_w2_scale : 0.0f;
-        const __half hi = __float2half_rn(x);
-        const uint32_t off = (uint32_t)(ci >> 4) * 4096u + (uint32_t)(co >> 3) * 1024u + (uint32_t)(co & 7) * 128u +
-                             ((((uint32_t)(ci & 15) >> 1) ^ (uint32_t)(co & 7)) << 4) + (uint32_t)(ci & 1) * 8u + (uint32_t)tap * 2u;
-        img[off >> 1] = hi;
-        img[(8192u + off) >> 1] = __float2half_rn(x - __half2float(hi));
-    }
 }
 
 struct navgym_policy {
@@ -672,219 +544,8 @@ static int policy_make_map(CUtensorMap *m, void *base, uint64_t rows, uint32_t b
     const cuuint32_t box[2] = {(cuuint32_t)pg::BK, box_rows};
     const cuuint32_t estr[2] = {1, 1};
     const CUresult r = encode(m, CU_TENSOR_MAP_DATA_TYPE_FLOAT16, 2, base, dims, strides, box, estr, CU_TENSOR_MAP_INTERLEAVE_NONE,
-                              pg::BK == 64 ? CU_TENSOR_MAP_SWIZZLE_128B : CU_TENSOR_MAP_SWIZZLE_64B, CU_TENSOR_MAP_L2_PROMOTION_L2_256B, CU_TENSOR_MAP_FLOAT_OOB_FILL_NONE);
+                              CU_TENSOR_MAP_SWIZZLE_64B, CU_TENSOR_MAP_L2_PROMOTION_L2_256B, CU_TENSOR_MAP_FLOAT_OOB_FILL_NONE);
     return r == CUDA_SUCCESS ? 0 : -1;
-}
-
-// ------------------------------------------------------------------ convolutional front end on the tensor cores
-// conv1 (1 -> 32 channels, k 5, stride 2) stays on the CUDA cores -- 41 k FMA per pedestrian --
-// and writes its ReLU output straight into the A operand of conv2 seen as a GEMM per pedestrian:
-//   D[pos][co] = sum_{ci, tap} h1[ci][2 pos - 1 + tap] w2[co][ci][tap],   M 128 x N 32 x K 128,
-// K index = 4 ci + tap with a zero fourth tap, so that a row of A is, per input channel, four
-// consecutive conv1 outputs: thread `pos` computes the three it needs itself (each conv1 output is
-// evaluated by the two positions that read it: 2 x 41 k FMA is cheaper than exchanging them) and
-// stores them, hi/lo-split, as 16-byte pieces of the 128-byte-swizzled K-major tile a TMA load
-// would have produced.  conv2 then is 24 tcgen05.mma per pedestrian (8 K steps x the three
-// f16x3 products) instead of 393 k FMA; 128 epilogue threads read the accumulator row of their
-// position from TMEM, add the bias, ReLU, scale, split and store 2 x 64 contiguous bytes: the
-// features leave position-major ([pos][channel]; act_fc1's weight columns are permuted to match).
-// 21 warps: 2 producer groups of 8 (a pedestrian each, A operand in 3 rotating stages; within a
-// group warps 0-3 build K block 0 = input channels 0-15, warps 4-7 K block 1), 1 MMA issuer,
-// 4 epilogue warps (accumulators double-buffered in TMEM: 2 x 6 x 32 columns).  The producers are the
-// critical resource (~1400 instructions per position and pedestrian): 16 warps of them keep the
-// four schedulers issuing (8 warps: 0.73 ms for 40 960 pedestrians; the SIMT kernel: 0.97 ms).
-namespace pc {
-constexpr int THREADS = 21 * 32, MMA_WARP = 16;
-constexpr uint32_t A_HALF = 2 * 16384;             // hi (or lo) part of one A stage: 2 K blocks of [128][64] f16
-constexpr uint32_t A_STAGE = 2 * A_HALF;           // 64 KB
-constexpr uint32_t B_BYTES = 16384;                // hi + lo, 2 K blocks of [32][64] f16 each
-constexpr uint32_t XS_FLOATS = 520;
-constexpr int A_STAGES = 3;                        // a producer group never waits for the MMAs of its previous pedestrian
-constexpr uint32_t OFF_B = A_STAGES * A_STAGE, OFF_W1 = OFF_B + B_BYTES, OFF_XS = OFF_W1 + 32 * 8 * 4;
-constexpr uint32_t OFF_BAR = OFF_XS + 2 * XS_FLOATS * 4;
-constexpr uint32_t SMEM_BYTES = OFF_BAR + 128 + 1024;
-constexpr uint32_t IDESC = (1u << 4) | ((uint32_t)(32 >> 3) << 17) | ((uint32_t)(128 >> 4) << 24);
-}  // namespace pc
-
-// conv_img: the B operand exactly as it sits in shared memory (policy_prepare_kernel), w1s
-// [32][8] = 5 conv1 taps and the bias, all times s_h, 2 pad; scales: see policy_prepare_kernel
-__global__ void __launch_bounds__(pc::THREADS, 1)
-policy_features_umma_kernel(const float *__restrict__ scan, int n, const uint4 *__restrict__ conv_img,
-                            const float *__restrict__ w1s, const float *__restrict__ b2, const float *__restrict__ scales,
-                            __half *__restrict__ out_hi, __half *__restrict__ out_lo)
-{
-    using namespace pg;
-    extern __shared__ uint8_t smem_raw[];
-    uint8_t *sm = smem_raw + ((1024u - (smem_u32(smem_raw) & 1023u)) & 1023u);
-    const uint32_t base = smem_u32(sm);
-    const uint32_t bars = base + pc::OFF_BAR;
-    const uint32_t afull0 = bars, aempty0 = bars + 24, tfull0 = bars + 48, tempty0 = bars + 64, tmem_slot = bars + 80;
-    const int warp = threadIdx.x >> 5, lane = threadIdx.x & 31;
-
-    for (int i = threadIdx.x; i < (int)(pc::B_BYTES / 16); i += pc::THREADS) reinterpret_cast<uint4 *>(sm + pc::OFF_B)[i] = conv_img[i];
-    for (int i = threadIdx.x; i < 256; i += pc::THREADS) reinterpret_cast<float *>(sm + pc::OFF_W1)[i] = w1s[i];
-    if (threadIdx.x < 6) {   // the left padding of both scan buffers: x[-3 .. -1] = 0
-        reinterpret_cast<float *>(sm + pc::OFF_XS)[(threadIdx.x / 3) * pc::XS_FLOATS + threadIdx.x % 3] = 0.0f;
-    }
-    if (threadIdx.x == 0) {
-        for (int st = 0; st < pc::A_STAGES; st++) { mbar_init(afull0 + 8 * st, 256); mbar_init(aempty0 + 8 * st, 1); }
-        for (int b = 0; b < 2; b++) { mbar_init(tfull0 + 8 * b, 1); mbar_init(tempty0 + 8 * b, 128); }
-        asm volatile("fence.mbarrier_init.release.cluster;" ::: "memory");
-    }
-    if (warp == pc::MMA_WARP) {
-        asm volatile("tcgen05.alloc.cta_group::1.sync.aligned.shared::cta.b32 [%0], %1;" ::"r"(tmem_slot), "r"(512u) : "memory");
-        asm volatile("tcgen05.relinquish_alloc_permit.cta_group::1.sync.aligned;" ::: "memory");
-    }
-    asm volatile("fence.proxy.async.shared::cta;" ::: "memory");   // the B operand was written with ordinary stores
-    tc_fence_before();
-    __syncthreads();
-    tc_fence_after();
-    uint32_t tmem_base;
-    asm volatile("ld.shared.b32 %0, [%1];" : "=r"(tmem_base) : "r"(tmem_slot) : "memory");
-    const int my_count = blockIdx.x < n ? (n - 1 - blockIdx.x) / gridDim.x + 1 : 0;   // pedestrians of this CTA
-
-    if (warp < pc::MMA_WARP) {
-        // ---- producers: group g fills A stage g for this CTA's pedestrians j = g, g + 2, ...
-        const int g = warp >> 3, tg = threadIdx.x & 255, pos = tg & 127, half = tg >> 7;
-        float *xs = reinterpret_cast<float *>(sm + pc::OFF_XS) + g * pc::XS_FLOATS;   // xs[3 + i] = input i
-        const float *wt = reinterpret_cast<const float *>(sm + pc::OFF_W1) + half * 16 * 8;
-        // this thread's row of K block `half`; a 16-byte piece `chunk` of it sits at chunk ^ (row % 8)
-        uint8_t *row0 = sm + half * 16384 + (pos >> 3) * 1024 + (pos & 7) * 128;
-        const uint32_t rx = pos & 7;
-        float pre[2] = {0.0f, 0.0f};   // the next pedestrian's scan, loaded one pedestrian ahead
-        if (g < my_count) {
-#pragma unroll
-            for (int i = 0; i < 2; i++) pre[i] = scan[(size_t)(blockIdx.x + g * gridDim.x) * 512 + tg + 256 * i];
-        }
-        for (int j = g; j < my_count; j += 2) {
-            const uint32_t st = (uint32_t)j % pc::A_STAGES, use = (uint32_t)j / pc::A_STAGES;   // pedestrian j -> A stage j % 3
-            uint8_t *rowp = row0 + st * pc::A_STAGE;
-            asm volatile("bar.sync %0, 256;" ::"r"(1 + g) : "memory");   // everyone is done with the previous scan
-#pragma unroll
-            for (int i = 0; i < 2; i++) {
-                const double r = fmin(fmax((double)pre[i], 0.0), 6.0);
-                xs[3 + tg + 256 * i] = (float)(r / 6.0 - 0.5);  // env.py:627-629, 648
-            }
-            if (j + 2 < my_count) {
-#pragma unroll
-                for (int i = 0; i < 2; i++) pre[i] = scan[(size_t)(blockIdx.x + (j + 2) * gridDim.x) * 512 + tg + 256 * i];
-            }
-            asm volatile("bar.sync %0, 256;" ::"r"(1 + g) : "memory");
-            mbar_wait(aempty0 + 8 * st, (use & 1) ^ 1);                  // the MMAs have read this stage
-            // conv1 outputs q = 2 pos - 1 + tap need inputs 2 q - 1 + k = 4 pos - 3 + 2 tap + k
-            const float4 xa = *reinterpret_cast<const float4 *>(xs + 4 * pos), xb = *reinterpret_cast<const float4 *>(xs + 4 * pos + 4);
-            const float x[9] = {xa.x, xa.y, xa.z, xa.w, xb.x, xb.y, xb.z, xb.w, xs[4 * pos + 8]};
-            const bool pad0 = pos == 0, pad2 = pos == 127;   // conv2's own zero padding: q = -1 and q = 255
-#pragma unroll 2
-            for (int cp = 0; cp < 8; cp++) {   // two input channels = one 16-byte piece
-                float v[2][3];
-#pragma unroll
-                for (int h = 0; h < 2; h++) {
-                    const float4 wa = *reinterpret_cast<const float4 *>(wt + (2 * cp + h) * 8);
-                    const float2 wb = *reinterpret_cast<const float2 *>(wt + (2 * cp + h) * 8 + 4);
-#pragma unroll
-                    for (int tap = 0; tap < 3; tap++) {
-                        float a = wb.y;
-                        a = fmaf(wa.x, x[2 * tap], a); a = fmaf(wa.y, x[2 * tap + 1], a); a = fmaf(wa.z, x[2 * tap + 2], a);
-                        a = fmaf(wa.w, x[2 * tap + 3], a); a = fmaf(wb.x, x[2 * tap + 4], a);
-                        v[h][tap] = fmaxf(a, 0.0f);
-                    }
-                    if (pad0) v[h][0] = 0.0f;
-                    if (pad2) v[h][2] = 0.0f;
-                }
-                // three packed conversions (F2FP on the ALU pipe; a lone cvt.f16.f32 would go to
-                // the quarter-rate XU pipe): taps (0, 1) of either channel, and both third taps
-                uint32_t h01a, l01a, h01b, l01b, h2, l2;
-                split2(v[0][0], v[0][1], h01a, l01a);
-                split2(v[1][0], v[1][1], h01b, l01b);
-                split2(v[0][2], v[1][2], h2, l2);
-                const uint32_t hi[4] = {h01a, h2 & 0xffffu, h01b, h2 >> 16};   // the fourth tap is a zero
-                const uint32_t lo[4] = {l01a, l2 & 0xffffu, l01b, l2 >> 16};
-                const uint32_t off = ((uint32_t)cp ^ rx) << 4;
-                *reinterpret_cast<uint4 *>(rowp + off) = make_uint4(hi[0], hi[1], hi[2], hi[3]);
-                *reinterpret_cast<uint4 *>(rowp + pc::A_HALF + off) = make_uint4(lo[0], lo[1], lo[2], lo[3]);
-            }
-            asm volatile("fence.proxy.async.shared::cta;" ::: "memory");   // visible to the tensor core's reads
-            mbar_arrive(afull0 + 8 * st);
-        }
-    } else if (warp == pc::MMA_WARP) {
-        // ---- MMA issuer
-        if (lane == 0) {
-            const uint32_t bh = base + pc::OFF_B, bl = bh + 8192;
-            for (int j = 0; j < my_count; j++) {
-                const uint32_t g = j & 1, par = (j >> 1) & 1, st = (uint32_t)j % pc::A_STAGES, use = (uint32_t)j / pc::A_STAGES;
-                mbar_wait(tempty0 + 8 * g, par ^ 1);
-                mbar_wait(afull0 + 8 * st, use & 1);
-                tc_fence_after();
-                // Six accumulators of 32 columns (3 products x 2 K blocks), four chained MMAs each:
-                // an N = 32 MMA is ~30 cycles of tensor-pipe work but its result is only available
-                // to the next accumulating MMA ~170 cycles later, so 24 MMAs chained on one
-                // accumulator cost 4 000 cycles per pedestrian (measured: the whole kernel ran at
-                // that pace); six independent chains overlap.  The epilogue adds them up.
-                const uint32_t d = tmem_base + g * 256, ah = base + st * pc::A_STAGE, al = ah + pc::A_HALF;
-#pragma unroll
-                for (int k = 0; k < 4; k++) {
-#pragma unroll
-                    for (int kb = 0; kb < 2; kb++) {
-                        const uint64_t fh = umma_desc_sw128(ah + kb * 16384 + k * 32), fl = umma_desc_sw128(al + kb * 16384 + k * 32);
-                        const uint64_t wh = umma_desc_sw128(bh + kb * 4096 + k * 32), wl = umma_desc_sw128(bl + kb * 4096 + k * 32);
-                        umma_f16(d + (0 + kb) * 32, fl, wh, pc::IDESC, k != 0);
-                        umma_f16(d + (2 + kb) * 32, fh, wl, pc::IDESC, k != 0);
-                        umma_f16(d + (4 + kb) * 32, fh, wh, pc::IDESC, k != 0);
-                    }
-                }
-                umma_commit(aempty0 + 8 * st);
-                umma_commit(tfull0 + 8 * g);
-            }
-        }
-    } else {
-        // ---- epilogue: warp w owns TMEM lanes 32 (w % 4) ... = positions
-        const int q = warp & 3, pos = q * 32 + lane;
-        const float descale = scales[3], fscale = scales[0];
-        for (int j = 0; j < my_count; j++) {
-            const uint32_t g = j & 1, par = (j >> 1) & 1;
-            const int ped = blockIdx.x + j * gridDim.x;
-            mbar_wait(tfull0 + 8 * g, par);
-            tc_fence_after();
-            float acc[32];
-            {
-                uint32_t v[32];
-                const uint32_t t0 = tmem_base + ((uint32_t)(q * 32) << 16) + g * 256;
-                tmem_ld32(t0, v);
-#pragma unroll
-                for (int c = 0; c < 32; c++) acc[c] = __uint_as_float(v[c]);
-#pragma unroll
-                for (int a = 1; a < 6; a++) {   // the two small products first, hi x hi last
-                    tmem_ld32(t0 + a * 32, v);
-#pragma unroll
-                    for (int c = 0; c < 32; c++) acc[c] += __uint_as_float(v[c]);
-                }
-            }
-            tc_fence_before();
-            mbar_arrive(tempty0 + 8 * g);   // the accumulators are in registers: the next MMAs may overwrite them
-            uint32_t hi[16], lo[16];
-#pragma unroll
-            for (int c = 0; c < 32; c += 2) {
-                const float a = fmaxf(fmaf(acc[c], descale, b2[c]), 0.0f) * fscale;
-                const float b = fmaxf(fmaf(acc[c + 1], descale, b2[c + 1]), 0.0f) * fscale;
-                split2(a, b, hi[c >> 1], lo[c >> 1]);
-            }
-            uint4 *oh = reinterpret_cast<uint4 *>(out_hi + (size_t)ped * 4096 + pos * 32);
-            uint4 *ol = reinterpret_cast<uint4 *>(out_lo + (size_t)ped * 4096 + pos * 32);
-#pragma unroll
-            for (int i = 0; i < 4; i++) {
-                oh[i] = make_uint4(hi[4 * i], hi[4 * i + 1], hi[4 * i + 2], hi[4 * i + 3]);
-                ol[i] = make_uint4(lo[4 * i], lo[4 * i + 1], lo[4 * i + 2], lo[4 * i + 3]);
-            }
-        }
-    }
-    tc_fence_before();
-    __syncthreads();
-    if (warp == pc::MMA_WARP) {
-        __syncwarp();
-        tc_fence_after();
-        asm volatile("tcgen05.dealloc.cta_group::1.sync.aligned.b32 %0, %1;" ::"r"(tmem_base), "r"(512u) : "memory");
-    }
 }
 
 // ------------------------------------------------------------------ front end, both convolutions on the tensor cores
@@ -893,10 +554,10 @@ policy_features_umma_kernel(const float *__restrict__ scan, int n, const uint4 *
 // policy_prepare_kernel), so the CUDA cores only convert: scan -> A1 (preprocess, split), D1 -> A2
 // (ReLU, split: D1's column order 3 c + tap IS conv2's K order, a thread's accumulator row goes
 // straight into its A2 row), D2 -> features.  Per pedestrian 3 + 12 tcgen05.mma (f16x3) and ~1000
-// instructions per position instead of ~1750.
-// NAVGYM_PF_GROUPS (3) groups of NAVGYM_PF_GWARPS (8) worker warps + one issuing warp each take
+// instructions per position instead of ~1750 with conv1 on the CUDA cores.
+// GROUPS (3) groups of GWARPS (8) worker warps + one issuing warp each take
 // pedestrians round robin and run them start to end.  A warp reaches the TMEM lanes 32 (warp % 4) .. + 31
-// = 32 positions; with 8 worker warps the two that share a quarter split the columns.
+// = 32 positions; the two worker warps of a group that share a quarter split the columns.
 //   P1a the scan, clipped and centred (float64, env.py:627-629), into the group's staging row
 //   P1b every thread builds its piece of the A1 rows -> arrive a1full -> 3 MMAs into D1, commit d1full
 //   P2  D1 from TMEM, ReLU, hi/lo split, into the A2 rows (K = 96 in three 64-byte-swizzled K blocks;
@@ -910,16 +571,10 @@ policy_features_umma_kernel(const float *__restrict__ scan, int n, const uint4 *
 // to, and one thread issues one every ~80 cycles at best (tools/umma_probe.cu) -- so every group has
 // its own issuing thread (a single one for all groups kept the kernel at 15 MMAs x ~150 cycles per
 // pedestrian: 0.39 ms), with the operand descriptors computed once.
-#ifndef NAVGYM_PF_GROUPS
-#define NAVGYM_PF_GROUPS 3   // 3 x 8 worker warps: 0.32 ms for 40 960 pedestrians; 4 x 4: 0.34 ms
-#endif
-#ifndef NAVGYM_PF_GWARPS
-#define NAVGYM_PF_GWARPS 8
-#endif
 namespace pf {
-constexpr int GROUPS = NAVGYM_PF_GROUPS, GWARPS = NAVGYM_PF_GWARPS, SUBS = GWARPS / 4, GTHREADS = 32 * GWARPS;
+constexpr int GROUPS = 3, GWARPS = 8;   // 3 x 8 worker warps: 0.32 ms for 40 960 pedestrians; 4 x 4: 0.34 ms
+constexpr int SUBS = GWARPS / 4, GTHREADS = 32 * GWARPS;
 constexpr int WORKERS = GROUPS * GTHREADS, THREADS = WORKERS + 32 * GROUPS;   // + one issuing warp per group
-static_assert(GWARPS == 4 || GWARPS == 8, "worker warps per group");
 static_assert(THREADS <= 1024 && GROUPS * 128 <= 512, "threads / TMEM columns");
 constexpr uint32_t A2_HALF = 3 * 8192;                 // hi (or lo): 3 K blocks of [128][32] f16
 constexpr uint32_t GBUF = 2 * A2_HALF;                 // 48 KB per group; A1 = its first 8 KB (hi | lo, [128][16] f16 each)
@@ -1013,9 +668,6 @@ policy_features_umma2_kernel(const float *__restrict__ scan, int n, const uint4 
         // P1a: a scan (loaded into registers a phase earlier), clipped and centred, into the staging row
         // (barriers on both sides)
         auto load_scan = [&](int p, float (&raw)[PER]) {
-#ifdef NAVGYM_PF_NOLOAD   // timing experiment: one pedestrian's scan for all (L1-resident)
-            p = 0;
-#endif
 #pragma unroll
             for (int i = 0; i < PER; i++) raw[i] = scan[(size_t)p * 512 + tg + GT * i];
         };
@@ -1031,12 +683,12 @@ policy_features_umma2_kernel(const float *__restrict__ scan, int n, const uint4 
             }
             asm volatile("bar.sync %0, %1;" ::"r"(1 + g), "n"(GT) : "memory");
         };
-        // P1b: this thread's piece of A1 row `pos` (k 0-7 | k 8, the bias and padding columns; with 8
-        // warps one piece each) -> arrive a1full
+        // P1b: this thread's piece of A1 row `pos` (sub 0: k 0-7, sub 1: k 8, the bias and padding
+        // columns) -> arrive a1full
         auto build_a1 = [&]() {
             const uint32_t sw = ((uint32_t)pos >> 2) & 1u;
             uint8_t *rowp = gb + pos * 32;
-            if (SUBS == 1 || sub == 0) {
+            if (sub == 0) {
                 const float4 xa = *reinterpret_cast<const float4 *>(xs + 4 * pos), xb = *reinterpret_cast<const float4 *>(xs + 4 * pos + 4);
                 uint32_t h[4], l[4];
                 split2(xa.x * 2048.0f, xa.y * 2048.0f, h[0], l[0]);
@@ -1046,7 +698,7 @@ policy_features_umma2_kernel(const float *__restrict__ scan, int n, const uint4 
                 *reinterpret_cast<uint4 *>(rowp + ((0u ^ sw) << 4)) = make_uint4(h[0], h[1], h[2], h[3]);
                 *reinterpret_cast<uint4 *>(rowp + pf::A1_HALF + ((0u ^ sw) << 4)) = make_uint4(l[0], l[1], l[2], l[3]);
             }
-            if (SUBS == 1 || sub == 1) {
+            if (sub == 1) {
                 uint32_t h8, l8;
                 split2(xs[4 * pos + 8] * 2048.0f, 2048.0f, h8, l8);   // k = 8, and the bias column k = 9
                 const uint32_t padw = (pos == 0 ? 0x7800u : 0u) | (pos == 127 ? 0x78000000u : 0u);   // 32768 at k = 10 / k = 11
@@ -1151,12 +803,10 @@ policy_features_umma2_kernel(const float *__restrict__ scan, int n, const uint4 
             asm volatile("fence.proxy.async.shared::cta;" ::: "memory");
             asm volatile("bar.sync %0, %1;" ::"r"(1 + g), "n"(GT) : "memory");
             if (tg == 0) {
-#ifndef NAVGYM_PF_NOSTORE
                 asm volatile("cp.async.bulk.global.shared::cta.bulk_group [%0], [%1], 8192;"
                              ::"l"(out_hi + (size_t)ped * 4096), "r"(smem_u32(stg)) : "memory");
                 asm volatile("cp.async.bulk.global.shared::cta.bulk_group [%0], [%1], 8192;"
                              ::"l"(out_lo + (size_t)ped * 4096), "r"(smem_u32(stg + 8192)) : "memory");
-#endif
                 asm volatile("cp.async.bulk.commit_group;" ::: "memory");
             }
         }

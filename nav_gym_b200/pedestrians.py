@@ -6,15 +6,15 @@ then re-scans the world from each pedestrian's new pose.  Here the same pipeline
 over [num_envs, max_ped] on the GPU:
 
   agent_scans()            navgym_agent_scan_batch: every pedestrian's scan in one launch
-  HumanPolicy              the reference architecture in torch (the one dense-math component;
-                           its pretrained weights, human_policy.pth, are not distributed: load
+  HumanPolicy              the reference architecture in torch, which holds the weights (its
+                           pretrained weights, human_policy.pth, are not distributed: load
                            them with load_state_dict when available, else random-init)
+  NativePolicy             HumanPolicy's action mean through the library's own kernels
   PedestrianSim            device state + the per-step sequence of env.py:617-693
 
 Everything on the per-step path is a kernel of the library, the policy forward included
 (NativePolicy: both convolutions, act_fc1 and act_fc2 on the tcgen05 tensor cores, DESIGN 4.3);
-torch owns the device memory and, in the comparison modes only, runs the dense layers.  Nothing here touches the CPU
-oracle.
+torch owns the device memory.  Nothing here touches the CPU oracle.
 """
 import ctypes as C
 
@@ -156,14 +156,14 @@ class NativePolicy(object):
         (feature scale x fc1 weight scale), conv1 output scale, 1 / (conv1 output scale x conv2
         weight scale), -, -, act_fc1 output scale, 1 / (that x fc2 weight scale)): copies / views of
         the workspace (tests)."""
-        L = (C.c_uint64 * 7)()
+        L = (C.c_uint64 * 6)()
         self.lib.navgym_policy_workspace_layout(self.max_n, L)
         w = self._ws
         unperm = lambda t: t.view(torch.float16).reshape(n, 128, 32).permute(0, 2, 1).reshape(n, 4096)
         fh, fl = unperm(w[L[0]:L[0] + n * 8192]), unperm(w[L[1]:L[1] + n * 8192])
-        scales = w[L[3]:L[3] + 32].view(torch.float32)
-        hh = w[L[5]:L[5] + n * 512].view(torch.float16).reshape(n, 256)
-        hl = w[L[6]:L[6] + n * 512].view(torch.float16).reshape(n, 256)
+        scales = w[L[2]:L[2] + 32].view(torch.float32)
+        hh = w[L[4]:L[4] + n * 512].view(torch.float16).reshape(n, 256)
+        hl = w[L[5]:L[5] + n * 512].view(torch.float16).reshape(n, 256)
         h = ((hh.double() + hl.double()) / float(scales[6])).float()
         return fh, fl, h, scales
 
@@ -213,7 +213,7 @@ class PedestrianSim(object):
 
     Per step, in the reference's order (env.py:617-693):
         sim.act()            respawn for episodes that just ended -> route following
-                             (navgym_peds_plan) -> policy (torch) -> clip, Human.set_vel, leg
+                             (navgym_peds_plan) -> policy (NativePolicy) -> clip, Human.set_vel, leg
                              odometry (navgym_peds_move) -> the geometry the robot's lidar sees
                              (navgym_peds_advance: discs for legs, boxes otherwise)
         env.step(actions)    the robot's fused step, scanning against that geometry
@@ -226,12 +226,9 @@ class PedestrianSim(object):
     (the clipped policy mean, the policy's `speed` input), scan f32 [.., 512], goal_id i32,
     waypoint f64, goal_local f32.
 
-    precision: 'f16x3' (default) runs the whole policy through the library's own kernels
-    (NativePolicy: both convolutions, act_fc1 and act_fc2 on the tcgen05 tensor cores with hi/lo f16 operand splits, float32-grade:
-    the mean matches the reference's CPU forward to ~1e-5).  The other modes keep the dense layers
-    in torch / cuBLAS for comparison: 'fp32', 'tf32x3' (three TF32 products of the operands' high
-    and low halves, same tolerance), 'tf32' or 'bf16' (means move by ~1e-3, the pedestrians' paths
-    are not comparable step by step any more).
+    The policy forward runs through the library's own kernels (NativePolicy: both convolutions,
+    act_fc1 and act_fc2 on the tcgen05 tensor cores with hi/lo f16 operand splits, float32-grade:
+    the mean matches the reference's CPU forward to ~1e-5).
 
     Auto-reset: every act() also draws the pedestrians of each environment's NEXT episode (at
     least 4 m from where the robot's auto-reset will put it -- the same Philox draw the step
@@ -241,16 +238,13 @@ class PedestrianSim(object):
     """
 
     def __init__(self, env, max_ped, nped=None, policy=None, v_pref_range=(0.0, 0.6), has_legs_ratio=0.5,
-                 num_goals=32, min_goal_dist=10.0, min_robot_dist=4.0, seed=0, fold_frames=True,
-                 precision='f16x3'):
+                 num_goals=32, min_goal_dist=10.0, min_robot_dist=4.0, seed=0):
         from . import maps as M
-        assert precision in ('f16x3', 'fp32', 'tf32x3', 'tf32', 'bf16')
         self.env, self.device = env, env.device
         self.B, self.P = env.B, int(max_ped)
         if self.P > 127:  # navgym_agent_scan_batch, crowd mode: one thread per other agent
             raise ValueError('at most 127 pedestrians per environment')
         self.dt = float(env.args.dt)
-        self.precision = precision
         self.lib = _lib.load()
         dev, f64, f32, i32 = self.device, torch.float64, torch.float32, torch.int32
         B, P = self.B, self.P
@@ -258,8 +252,7 @@ class PedestrianSim(object):
         if policy is None:
             policy = HumanPolicy()
         self.policy = policy.to(dev).eval()
-        self.fold_frames = bool(fold_frames)
-        self.native = NativePolicy(self.policy, self.B * self.P, dev) if precision == 'f16x3' else None
+        self.native = NativePolicy(self.policy, self.B * self.P, dev)
         # ---- planning fields + free-cell pools per map (kept on the MapPool: a pool that is
         # reused for another episode / another sim does not rebuild them)
         cache = getattr(env.pool, '_plan_cache', None)
@@ -403,66 +396,10 @@ class PedestrianSim(object):
         if respawn is not None:
             self._scan(respawn)  # first scans of the respawned pedestrians (env.py:808-815)
         goal, speed = self.goal_local.reshape(-1, 2), self.prev_action.reshape(-1, 2)
-        if self.native is not None:   # three launches of the library, straight into the move kernel's input
-            self.native.mean(self.scan.reshape(self.B * self.P, -1), goal, speed, out=self._mean)
-        else:
-            self._mean.copy_(self._policy_mean(self.scan.reshape(self.B * self.P, -1), goal, speed).reshape(self.B, self.P, 2))
+        # three launches of the library, straight into the move kernel's input
+        self.native.mean(self.scan.reshape(self.B * self.P, -1), goal, speed, out=self._mean)
         self._call(self.lib.navgym_peds_move, self.move_args, 'peds_move')
         env._peds_emit(advance=False)
-
-    def _policy_mean(self, x, goal, speed):
-        """x: the raw scans [N, 512] in metres."""
-        if self.native is not None:
-            return self.native.mean(x.contiguous(), goal.contiguous(), speed.contiguous())
-        if self.precision == 'bf16':
-            with torch.autocast('cuda', dtype=torch.bfloat16):
-                return self._mean_fp(x, goal, speed).float()
-        if self.precision == 'tf32':
-            old = (torch.backends.cuda.matmul.allow_tf32, torch.backends.cudnn.allow_tf32)
-            torch.backends.cuda.matmul.allow_tf32 = torch.backends.cudnn.allow_tf32 = True
-            try:
-                return self._mean_fp(x, goal, speed)
-            finally:
-                torch.backends.cuda.matmul.allow_tf32, torch.backends.cudnn.allow_tf32 = old
-        return self._mean_fp(x, goal, speed)
-
-    def _mean_fp(self, x, goal, speed):
-        p = self.policy
-        if not self.fold_frames:
-            x3 = preprocess_scan(x)[:, None, :].expand(-1, 3, -1).contiguous()
-            return p.mean(x3, goal, speed)
-        # env.py:647 hands the newest scan to all three input frames, so the first convolution
-        # sees three identical channels: sum its weights over them once and convolve one.  The
-        # two convolutions run in one kernel of the library (activations never leave shared
-        # memory); the dense layers are torch / cuBLAS.
-        n = x.shape[0]
-        if getattr(self, '_feat', None) is None or self._feat.shape[0] != n:
-            self._feat = torch.empty(n, 4096, dtype=torch.float32, device=self.device)
-        w1 = p.act_fea_cv1.weight.float().sum(dim=1).contiguous()
-        self._w = (w1, p.act_fea_cv1.bias.float().contiguous(), p.act_fea_cv2.weight.float().contiguous(),
-                   p.act_fea_cv2.bias.float().contiguous())
-        with torch.cuda.device(self.device):
-            _lib.check(self.lib.navgym_policy_features(_ptr(x), n, *[_ptr(t) for t in self._w], _ptr(self._feat),
-                                                       self.env._stream()), 'policy_features')
-        if self.precision == 'tf32x3':
-            # x = xh + xl, w = wh + wl with xh, wh exactly representable in TF32 (low 13 mantissa
-            # bits cleared): x w^T = xh wh^T + xl wh^T + xh wl^T up to the dropped xl wl^T (2^-22)
-            def split(t):
-                hi = (t.contiguous().view(torch.int32) & -8192).view(torch.float32)
-                return hi, t - hi
-            xh, xl = split(self._feat)
-            wh, wl = split(p.act_fc1.weight.float())
-            old = torch.backends.cuda.matmul.allow_tf32
-            torch.backends.cuda.matmul.allow_tf32 = True   # for these three products only
-            try:
-                h = xh @ wh.t() + (xl @ wh.t() + xh @ wl.t())
-            finally:
-                torch.backends.cuda.matmul.allow_tf32 = old
-            h = F.relu(h + p.act_fc1.bias)
-        else:
-            h = F.relu(p.act_fc1(self._feat))
-        h = F.relu(p.act_fc2(torch.cat((h, goal, speed), dim=-1)))
-        return torch.cat((torch.sigmoid(p.actor1(h)), torch.tanh(p.actor2(h))), dim=-1)
 
     # ---- env.py:683-693 -------------------------------------------------------------------
     def observe(self):

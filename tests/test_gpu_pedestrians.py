@@ -184,7 +184,7 @@ def test_native_policy_reproduces_the_reference_means(name):
     assert np.allclose(m.cpu().numpy().reshape(T, P, 2), G['mean'], rtol=0, atol=2e-5)
 
 
-def _crowd(B=64, P=6, seed=0, **kw):
+def _crowd(B=64, P=6, seed=0):
     from nav_gym_b200 import maps
     from nav_gym_b200.batched_env import BatchedNavGym, MapPool, filter_spawn_pool
     from nav_gym_b200.pedestrians import PedestrianSim
@@ -194,34 +194,27 @@ def _crowd(B=64, P=6, seed=0, **kw):
     mp = MapPool([m], 'cuda:0', spawn_pools=[pool])
     env = BatchedNavGym(B, mp, seed=seed, auto_reset=True)
     env.reset_from_spawn_pool(np.random.RandomState(seed))
-    return m, env, PedestrianSim(env, P, seed=seed, **kw)
+    return m, env, PedestrianSim(env, P, seed=seed)
 
 
-@pytest.mark.parametrize('precision,tol', [('f16x3', 1e-5), ('fp32', 1e-5), ('tf32x3', 1e-5), ('tf32', 5e-3), ('bf16', 2e-2)])
-def test_policy_precisions(precision, tol):
-    """PedestrianSim's policy forward in each precision mode against torch's float32 forward."""
-    m, env, sim = _crowd(B=32, P=8, seed=3, precision=precision)
+def test_pedestrian_sim_policy_matches_the_float32_forward():
+    """PedestrianSim's policy forward (sim.native) on its own scans against torch's float32 forward."""
+    m, env, sim = _crowd(B=32, P=8, seed=3)
     from nav_gym_b200.pedestrians import preprocess_scan
     x = sim.scan.reshape(-1, 512)
     goal, speed = sim.goal_local.reshape(-1, 2), torch.rand(32 * 8, 2, device='cuda')
-    tf32 = (torch.backends.cuda.matmul.allow_tf32, torch.backends.cudnn.allow_tf32)
-    torch.backends.cuda.matmul.allow_tf32 = torch.backends.cudnn.allow_tf32 = False
-    try:
-        with torch.no_grad():
-            want = sim.policy.mean(preprocess_scan(x)[:, None, :].expand(-1, 3, -1).contiguous(), goal, speed)
-    finally:
-        torch.backends.cuda.matmul.allow_tf32, torch.backends.cudnn.allow_tf32 = tf32
-    with torch.no_grad():
-        got = sim._policy_mean(x, goal, speed)
-    assert float((got - want).abs().max()) < tol
+    want = _f32_reference(lambda: sim.policy.mean(preprocess_scan(x)[:, None, :].expand(-1, 3, -1).contiguous(), goal, speed))
+    got = sim.native.mean(x, goal, speed)
+    assert float((got - want).abs().max()) < 1e-5
 
 
-def test_pedestrian_sim_follows_the_reference_step_order():
+def test_native_pedestrian_sim_follows_the_reference_step_order():
     """One PedestrianSim step against a by-hand evaluation of env.py:617-693 on the same state:
-    policy mean from the previous scan / local goal / previous action, Human.set_vel with the
-    preferred-speed factor, leg odometry, and the new scans from the new poses."""
+    policy mean (the native forward, against torch's float32 forward) from the previous scan /
+    local goal / previous action, Human.set_vel with the preferred-speed factor, leg odometry,
+    and the new scans from the new poses."""
     from nav_gym_b200.pedestrians import human_set_vel, preprocess_scan
-    m, env, sim = _crowd(B=16, P=5, seed=1, fold_frames=False)
+    m, env, sim = _crowd(B=16, P=5, seed=1)
     g = torch.Generator(device='cuda'); g.manual_seed(0)
     for t in range(3):
         pose0, scan0, prev_a = sim.pose.clone(), sim.scan.clone(), sim.prev_action.clone()
@@ -237,8 +230,7 @@ def test_pedestrian_sim_follows_the_reference_step_order():
         loc = torch.stack((rel[..., 0] * c + rel[..., 1] * s, -rel[..., 0] * s + rel[..., 1] * c), -1)
         assert torch.allclose(loc.float(), sim.goal_local, atol=1e-5)
         x = preprocess_scan(scan0).reshape(-1, 1, 512).expand(-1, 3, -1).contiguous()
-        with torch.no_grad():
-            mean = sim.policy.mean(x, sim.goal_local.reshape(-1, 2), prev_a.reshape(-1, 2)).reshape(16, 5, 2)
+        mean = _f32_reference(lambda: sim.policy.mean(x, sim.goal_local.reshape(-1, 2), prev_a.reshape(-1, 2))).reshape(16, 5, 2)
         clipped = torch.minimum(torch.maximum(mean, torch.tensor([0., -1.], device='cuda')), torch.tensor([1., 1.], device='cuda'))
         assert torch.allclose(clipped, sim.prev_action, atol=1e-5)
         pose1, vel1 = human_set_vel(pose0, sim.prev_action.double() * sim.v_pref[..., None], 0.2)

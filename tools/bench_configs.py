@@ -28,8 +28,7 @@ def crowd(dev, steps, warmup, B=4096, P=10):
     mp = MapPool([m], dev, spawn_pools=[pool])
     env = BatchedNavGym(B, mp, device=dev, seed=8, auto_reset=True)
     env.reset_from_spawn_pool(np.random.RandomState(4))
-    precision = os.environ.get('NAVGYM_CROWD_PRECISION', 'f16x3')
-    sim = PedestrianSim(env, P, seed=8, precision=precision)
+    sim = PedestrianSim(env, P, seed=8)
     pol = random_policy(B, dev)
 
     def phase(fn, n):
@@ -44,7 +43,7 @@ def crowd(dev, steps, warmup, B=4096, P=10):
         sim.step(pol(None))
     ms = phase(lambda: sim.step(pol(None)), steps)
     parts = dict(act=phase(sim.act, 20), robot_step=phase(lambda: env.step(pol(None)), 20), observe=phase(sim.observe, 20))
-    return dict(config='crowd', envs=B, pedestrians=P, policy_precision=precision, ms_per_step=ms, env_steps_per_s=B / ms * 1e3,
+    return dict(config='crowd', envs=B, pedestrians=P, ms_per_step=ms, env_steps_per_s=B / ms * 1e3,
                 pedestrian_steps_per_s=B * P / ms * 1e3, pedestrian_rays_per_s=B * P * 512 / ms * 1e3,
                 ms_parts=parts)
 

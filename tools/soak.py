@@ -33,7 +33,7 @@ print('robot batch: %d steps x %d envs in %.1f s; episodes ended %d (success %d,
 B, P = 1024, 8
 env = BatchedNavGym(B, mp, seed=2, auto_reset=True)
 env.reset_from_spawn_pool(np.random.RandomState(2))
-sim = PedestrianSim(env, P, seed=2, precision='tf32')
+sim = PedestrianSim(env, P, seed=2)
 t0 = time.time()
 eps = 0
 for t in range(n_steps // 10):
