@@ -6,6 +6,17 @@ import golden_util as gu
 from nav_gym_b200.batched_env import BatchedNavGym
 
 
+def f32_reference(fn):
+    """Run fn with TF32 off everywhere (cuDNN / cuBLAS would round operands to TF32)."""
+    old = (torch.backends.cuda.matmul.allow_tf32, torch.backends.cudnn.allow_tf32)
+    torch.backends.cuda.matmul.allow_tf32 = torch.backends.cudnn.allow_tf32 = False
+    try:
+        with torch.no_grad():
+            return fn()
+    finally:
+        torch.backends.cuda.matmul.allow_tf32, torch.backends.cudnn.allow_tf32 = old
+
+
 class CudaStepper(object):
     def __init__(self, maps, map_id, start, goal, theta, max_disc=0, max_seg=0, early_stop=True,
                  cell_rule='numpy1', **kw):

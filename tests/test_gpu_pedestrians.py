@@ -6,6 +6,7 @@ import pytest
 import torch
 
 import golden_util as gu
+from cuda_util import f32_reference
 
 pytestmark = pytest.mark.gpu
 
@@ -112,17 +113,6 @@ def test_policy_features_kernel_and_folded_forward(name):
     assert np.allclose(m.cpu().numpy().reshape(T, P, 2), G['mean'], rtol=0, atol=2e-5)
 
 
-def _f32_reference(fn):
-    """Run fn with TF32 off everywhere (cuDNN / cuBLAS would round operands to TF32)."""
-    old = (torch.backends.cuda.matmul.allow_tf32, torch.backends.cudnn.allow_tf32)
-    torch.backends.cuda.matmul.allow_tf32 = torch.backends.cudnn.allow_tf32 = False
-    try:
-        with torch.no_grad():
-            return fn()
-    finally:
-        torch.backends.cuda.matmul.allow_tf32, torch.backends.cudnn.allow_tf32 = old
-
-
 @pytest.mark.parametrize('n', [1, 77, 128, 300, 1029, 19200])
 def test_native_policy_stage_by_stage(n):
     """navgym_policy_mean (front end -> tcgen05 act_fc1 in the f16x3 scheme -> act_fc2 + heads)
@@ -147,7 +137,7 @@ def test_native_policy_stage_by_stage(n):
     torch.cuda.synchronize()
     fh, fl, h, scales = nat.intermediates(n)
     x3 = preprocess_scan(scan)[:, None, :].expand(-1, 3, -1).contiguous()
-    feat = _f32_reference(lambda: F.relu(pol.act_fea_cv2(F.relu(pol.act_fea_cv1(x3)))).reshape(n, -1))
+    feat = f32_reference(lambda: F.relu(pol.act_fea_cv2(F.relu(pol.act_fea_cv1(x3)))).reshape(n, -1))
     s_f = float(scales[0])
     assert s_f > 0 and np.log2(s_f) == int(np.log2(s_f)) and float(fh.float().abs().max()) < 32768.0
     mine = (fh.double() + fl.double()) / s_f
@@ -159,11 +149,11 @@ def test_native_policy_stage_by_stage(n):
     with torch.no_grad():
         want_h = torch.relu(mine @ pol.act_fc1.weight.double().t() + pol.act_fc1.bias.double())
         err = float((h.double() - want_h).abs().max())
-        sgemm = _f32_reference(lambda: torch.relu(mine.float() @ pol.act_fc1.weight.t() + pol.act_fc1.bias))
+        sgemm = f32_reference(lambda: torch.relu(mine.float() @ pol.act_fc1.weight.t() + pol.act_fc1.bias))
         err_sgemm = float((sgemm.double() - want_h).abs().max())
     bar = 1e-5 * max(1.0, float(want_h.abs().max()))
     assert err < bar and err_sgemm < bar, (err, err_sgemm)
-    want = _f32_reference(lambda: pol.mean(x3, goal, speed))
+    want = f32_reference(lambda: pol.mean(x3, goal, speed))
     assert float((got - want).abs().max()) < 1e-5
 
 
@@ -203,7 +193,7 @@ def test_pedestrian_sim_policy_matches_the_float32_forward():
     from nav_gym_b200.pedestrians import preprocess_scan
     x = sim.scan.reshape(-1, 512)
     goal, speed = sim.goal_local.reshape(-1, 2), torch.rand(32 * 8, 2, device='cuda')
-    want = _f32_reference(lambda: sim.policy.mean(preprocess_scan(x)[:, None, :].expand(-1, 3, -1).contiguous(), goal, speed))
+    want = f32_reference(lambda: sim.policy.mean(preprocess_scan(x)[:, None, :].expand(-1, 3, -1).contiguous(), goal, speed))
     got = sim.native.mean(x, goal, speed)
     assert float((got - want).abs().max()) < 1e-5
 
@@ -230,7 +220,7 @@ def test_native_pedestrian_sim_follows_the_reference_step_order():
         loc = torch.stack((rel[..., 0] * c + rel[..., 1] * s, -rel[..., 0] * s + rel[..., 1] * c), -1)
         assert torch.allclose(loc.float(), sim.goal_local, atol=1e-5)
         x = preprocess_scan(scan0).reshape(-1, 1, 512).expand(-1, 3, -1).contiguous()
-        mean = _f32_reference(lambda: sim.policy.mean(x, sim.goal_local.reshape(-1, 2), prev_a.reshape(-1, 2))).reshape(16, 5, 2)
+        mean = f32_reference(lambda: sim.policy.mean(x, sim.goal_local.reshape(-1, 2), prev_a.reshape(-1, 2))).reshape(16, 5, 2)
         clipped = torch.minimum(torch.maximum(mean, torch.tensor([0., -1.], device='cuda')), torch.tensor([1., 1.], device='cuda'))
         assert torch.allclose(clipped, sim.prev_action, atol=1e-5)
         pose1, vel1 = human_set_vel(pose0, sim.prev_action.double() * sim.v_pref[..., None], 0.2)
