@@ -29,6 +29,19 @@ extern "C" {
 #define NAVGYM_MAX_SEG 128
 #define NAVGYM_SCHED_BUCKETS 32
 
+/* Observation row formats (navgym_step_args_t / navgym_her_args_t .obs_format).
+ *   NAVGYM_OBS_F32  float32 rows of obs_stride floats: [S*512 scans | 7 tail fields], obs_stride >= S*512 + 7.
+ *   NAVGYM_OBS_F16  rows of obs_stride HALVES (2-byte units): [S*512 scans as float16, round-to-nearest
+ *                   of the float32 value | the 7 tail fields as float32 (14 halves) | padding, never
+ *                   written].  obs_stride must be even and >= S*512 + 14 and the row base 4-byte
+ *                   aligned, so that the tail is aligned float32; S*512 + 16 halves gives 16-byte
+ *                   aligned rows.  The obs / obs_host pointers of every entry point stay `float *`:
+ *                   pass the row storage cast to it.
+ * Anything else (an unknown format, an odd or too short stride, a misaligned base) is
+ * cudaErrorInvalidValue. */
+#define NAVGYM_OBS_F32 0
+#define NAVGYM_OBS_F16 1
+
 /* rows of the structure-of-arrays float64 state block state[NAVGYM_NS][num_envs] */
 enum {
     NAVGYM_S_PX = 0, NAVGYM_S_PY, NAVGYM_S_TH,   /* robot pose (keti_robot.py:56-58) */
@@ -57,7 +70,9 @@ typedef struct {
  *   noise   f32 [num_envs][2][512] additive, slot 0 = the step's scan, slot 1 = the crash
  *           re-scan (parity traces); NULL -> Philox N(0, noise_std[env]) (production)
  *   obs     f32 [num_envs][obs_stride], first S*512+7 columns written per row (S = num_scan_stack;
- *           the S-1 older scans are carried over from the row's previous contents)
+ *           the S-1 older scans are carried over from the row's previous contents); with
+ *           obs_format = NAVGYM_OBS_F16 the rows are [num_envs][obs_stride] halves instead (see
+ *           NAVGYM_OBS_F16 above; the older scans are shifted as float16)
  *   tail64  f64 [num_envs][7]   (the 7 trailing observation fields in float64, env.py:455)
  *   hits    i16 [num_envs][512][2] hit cell minus origin cell of the step's first scan, or
  *           NAVGYM_HIT_NONE; NULL = not recorded
@@ -126,13 +141,18 @@ typedef struct {
     const int32_t *ndisc_reset;
     const float *segs_reset;
     const int32_t *nseg_reset;
+    /* row format of obs (and of obs_host in the host-buffer entry points): NAVGYM_OBS_F32 (0, the
+     * zero-initialised default) or NAVGYM_OBS_F16; obs_stride counts elements of that format */
+    int32_t obs_format;
+    int32_t _pad;
 } navgym_step_args_t;
 
 /* ---- fused hot path: NavGymEnv.step (env.py:591-728) over num_envs environments ------ */
 int navgym_step_batch(const navgym_step_args_t *args, void *stream);
 /* The same step for a caller whose buffers live on the HOST (the reference's own calling
  * convention: numpy in, numpy out).  actions_host f32 [num_envs][2], obs_host f32
- * [num_envs][obs_stride], reward_host f32 [num_envs], done_host u8 [num_envs] must be pinned
+ * [num_envs][obs_stride] (rows of args->obs_format, like obs), reward_host f32 [num_envs],
+ * done_host u8 [num_envs] must be pinned
  * (cudaHostAlloc / cudaHostRegister).  The batch is stepped as `chunks` launches over consecutive
  * environment ranges on prioritised streams, each followed by the device-to-host copy of its
  * rows, so the copies of early chunks overlap the raycast of later ones; args->actions, obs,
@@ -191,8 +211,9 @@ int navgym_export_env_len(int num_scan_stack);
 int navgym_export_env(const navgym_step_args_t *args, int env, double *out_dev, void *stream);
 
 /* ---- HER batch API: compute_rewards / compute_terminals / compute_info (env.py:464-589) on
- * `count` stored observation rows obs[count][obs_stride] (float32, the layout of env.py:455)
- * with goals[count][2]; any output pointer may be NULL. */
+ * `count` stored observation rows obs[count][obs_stride] (float32, the layout of env.py:455;
+ * with obs_format = NAVGYM_OBS_F16 the float16-scan rows above, obs cast to float *, obs_stride
+ * in halves) with goals[count][2]; any output pointer may be NULL. */
 typedef struct {
     double dist_thresh;
     double r_scale, r_success, r_crash, r_progress, r_forward, r_rotation, r_discomfort;
@@ -203,6 +224,8 @@ typedef struct {
     float *reward;
     uint8_t *done, *is_success, *is_crash;
     float *distance;
+    int32_t obs_format;        /* NAVGYM_OBS_F32 (0) or NAVGYM_OBS_F16 */
+    int32_t _pad2;
 } navgym_her_args_t;
 int navgym_compute_rewards(const navgym_her_args_t *args, void *stream);
 

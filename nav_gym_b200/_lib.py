@@ -25,6 +25,7 @@ HIT_NONE = -32768
 MAX_DISC = 64
 MAX_SEG = 128
 SCHED_BUCKETS = 32
+OBS_F32, OBS_F16 = 0, 1   # navgym_step_args_t.obs_format
 NS = 10
 S_PX, S_PY, S_TH, S_GX, S_GY, S_PPX, S_PPY, S_PYAW, S_PV, S_PW = range(NS)
 
@@ -98,6 +99,7 @@ class StepArgs(C.Structure):
         ('distance', _P), ('hits', _P), ('sched', _P),
         ('reward_mirror', _P), ('done_mirror', _P),
         ('discs_reset', _P), ('ndisc_reset', _P), ('segs_reset', _P), ('nseg_reset', _P),
+        ('obs_format', C.c_int32), ('_pad', C.c_int32),
     ]
 
 
@@ -108,7 +110,8 @@ class HerArgs(C.Structure):
                 ('count', C.c_int32), ('obs_stride', C.c_int32),
                 ('num_scan_stack', C.c_int32), ('_pad', C.c_int32),
                 ('obs', _P), ('goals', _P), ('thr', _P), ('dthr', _P), ('reward', _P),
-                ('done', _P), ('is_success', _P), ('is_crash', _P), ('distance', _P)]
+                ('done', _P), ('is_success', _P), ('is_crash', _P), ('distance', _P),
+                ('obs_format', C.c_int32), ('_pad2', C.c_int32)]
 
 
 class ScanArgs(C.Structure):

@@ -126,7 +126,7 @@ class BatchedNavGym(object):
                  max_disc=0, max_seg=0, seed=0, env_offset=0, auto_reset=False,
                  max_episode_steps=0, resample_map=False, scan_noise_std_range=(0.0, 0.05),
                  cell_rule='numpy1', early_stop=True, record_hits=False, longest_first=True,
-                 num_scan_stack=1, **reward):
+                 num_scan_stack=1, obs_dtype=torch.float32, **reward):
         self.lib = _lib.require_device()
         self.device = torch.device(device)
         self.B = B = int(num_envs)
@@ -145,8 +145,17 @@ class BatchedNavGym(object):
         self.map_id = torch.from_numpy(mid).to(dev)
         self.noise_std = torch.zeros(B, dtype=f32, device=dev)
         self.num_scan_stack = S = max(int(num_scan_stack), 1)
-        self.obs_dim = S * NB + 7
-        self.obs = torch.zeros(B, self.obs_dim, dtype=f32, device=dev)
+        # Observation rows: float32 [scans | 7 tail fields], or with obs_dtype=torch.float16 the
+        # S*512 scans in float16 followed by the tail as float32 in 14 halves and 2 halves of padding
+        # (1056-byte rows for S = 1; obs_parts() splits either format)
+        if obs_dtype == torch.float32:
+            obs_format, self.obs_dim = _lib.OBS_F32, S * NB + 7
+        elif obs_dtype == torch.float16:
+            obs_format, self.obs_dim = _lib.OBS_F16, S * NB + 16
+        else:
+            raise ValueError('obs_dtype must be torch.float32 or torch.float16, not %r' % (obs_dtype,))
+        self.obs_dtype = obs_dtype
+        self.obs = torch.zeros(B, self.obs_dim, dtype=obs_dtype, device=dev)
         self.tail64 = torch.zeros(B, 7, dtype=f64, device=dev)
         self.reward = torch.zeros(B, dtype=f32, device=dev)
         self.done = torch.zeros(B, dtype=u8, device=dev)
@@ -175,6 +184,7 @@ class BatchedNavGym(object):
         a.cell_rule = {'numpy1': 0, 'numpy2': 1}[cell_rule]
         a.max_disc, a.max_seg = self.max_disc, self.max_seg
         a.num_envs, a.obs_stride, a.num_scan_stack = B, self.obs_dim, S
+        a.obs_format = obs_format
         a.auto_reset, a.max_episode_steps = int(auto_reset), int(max_episode_steps)
         a.num_maps, a.resample_map = self.pool.num_maps, int(resample_map)
         a.seed, a.env_offset = int(seed), int(env_offset)
@@ -265,7 +275,8 @@ class BatchedNavGym(object):
 
     def step_host(self, actions_host, obs_host, reward_host, done_host, chunks=2):
         """The same step for callers that live on the host (the reference's calling
-        convention): pinned host actions in, pinned host obs / reward / done out, through the
+        convention): pinned host actions in, pinned host obs (rows of the env's obs_dtype and
+        width, like env.obs) / reward / done out, through the
         C ABI's navgym_step_batch_host: `chunks` launches over consecutive env ranges on
         prioritised streams, each followed by the D2H copy of its rows, so the copies of early
         chunks overlap the raycast of later ones (PCIe is the end-to-end bound: 2.1 KB per
@@ -273,7 +284,7 @@ class BatchedNavGym(object):
         for t in (actions_host, obs_host, reward_host, done_host):
             if not t.is_pinned() or not t.is_contiguous():
                 raise ValueError('step_host needs contiguous pinned host tensors')
-        assert obs_host.dtype == torch.float32 and tuple(obs_host.shape) == (self.B, self.obs_dim)
+        assert obs_host.dtype == self.obs_dtype and tuple(obs_host.shape) == (self.B, self.obs_dim)
         assert reward_host.dtype == torch.float32 and done_host.dtype == torch.uint8
         assert actions_host.dtype == torch.float32 and actions_host.numel() == 2 * self.B
         if self.peds is not None:
@@ -299,7 +310,7 @@ class BatchedNavGym(object):
         for t in (actions_host, obs_host, reward_host, done_host):
             if not t.is_pinned() or not t.is_contiguous():
                 raise ValueError('host_groups needs contiguous pinned host tensors')
-        assert obs_host.dtype == torch.float32 and tuple(obs_host.shape) == (self.B, self.obs_dim)
+        assert obs_host.dtype == self.obs_dtype and tuple(obs_host.shape) == (self.B, self.obs_dim)
         assert actions_host.dtype == torch.float32 and actions_host.numel() == 2 * self.B
         assert reward_host.dtype == torch.float32 and done_host.dtype == torch.uint8
         self._make_pipe(groups, fresh=True)
@@ -436,12 +447,33 @@ class BatchedNavGym(object):
                                is_crash=bool(sc[3]), truncated=bool(sc[4]), distance=float(np.float32(sc[5])),
                                episode=int(sc[8]), noise_std=float(np.float32(sc[9])))
 
+    def obs_parts(self, rows=None):
+        """(scans [N, S*512], tail [N, 7] float32) views of observation rows of this env's format:
+        env.obs (rows=None) or any [N, width] tensor of the same dtype laid out like it, e.g. pinned
+        host rows or a slice of a replay buffer.  float16 rows keep the tail as float32 in the 14
+        halves after the scans, seen here through .view(torch.float32); for float32 rows the two
+        are plain slices, so code written against obs_parts runs on either format."""
+        rows = self.obs if rows is None else rows
+        n = self.num_scan_stack * NB
+        if rows.dtype != self.obs_dtype:
+            raise ValueError('rows of dtype %s, the env keeps %s rows' % (rows.dtype, self.obs_dtype))
+        if self.obs_dtype == torch.float16:
+            return rows[:, :n], rows[:, n:n + 14].view(torch.float32)
+        return rows[:, :n], rows[:, n:n + 7]
+
     # ---- HER batch API (env.py:491-589) on device tensors ---------------------------------
     def compute_rewards(self, obs, goals, **reward):
         """compute_rewards / compute_terminals / compute_info for stored observations:
-        obs float32 [N, >=519] (row layout of env.py:455), goals float32 [N, 2], both on the
-        device.  Returns dict(reward, done, is_success, is_crash, distance) of device tensors."""
-        obs = obs.to(device=self.device, dtype=torch.float32)
+        obs float32 [N, >=519] (row layout of env.py:455), or float16 rows in the layout of
+        obs_dtype=torch.float16 (float16 scans, float32 tail; an even row stride, a 4-byte aligned
+        start), whatever the env's own format; goals float32 [N, 2], both on the device.  Returns
+        dict(reward, done, is_success, is_crash, distance) of device tensors."""
+        if obs.dtype == torch.float16:
+            obs_format = _lib.OBS_F16
+            obs = obs.to(device=self.device)
+        else:
+            obs_format = _lib.OBS_F32
+            obs = obs.to(device=self.device, dtype=torch.float32)
         if obs.stride(-1) != 1:
             obs = obs.contiguous()
         goals = goals.to(device=self.device, dtype=torch.float32).contiguous()
@@ -461,6 +493,7 @@ class BatchedNavGym(object):
                         'reward_forward_factor': 'r_forward', 'reward_rotation_factor': 'r_rotation',
                         'reward_discomfort_factor': 'r_discomfort'}[k], v)
         h.count, h.obs_stride, h.num_scan_stack = n, obs.stride(0), self.num_scan_stack
+        h.obs_format = obs_format
         h.obs, h.goals, h.thr, h.dthr = _ptr(obs), _ptr(goals), _ptr(self.thr), _ptr(self.dthr)
         h.reward, h.done, h.is_success = _ptr(out['reward']), _ptr(out['done']), _ptr(out['is_success'])
         h.is_crash, h.distance = _ptr(out['is_crash']), _ptr(out['distance'])

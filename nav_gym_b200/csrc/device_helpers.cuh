@@ -128,3 +128,40 @@ __device__ __forceinline__ uint4 philox4x32_10(uint4 c, uint2 k)
 }
 
 __device__ __forceinline__ float u01(uint32_t x) { return ((float)(x >> 8) + 0.5f) * (1.0f / 16777216.0f); }
+
+// The observation row layouts (include/navgym_b200.h NAVGYM_OBS_*), the one place that knows
+// them.  Element i < S*512 of p is a scan value; the 7 tail fields follow the S scans.
+//   F32: float[obs_stride].
+//   F16: __half[obs_stride]: float16 scans (round-to-nearest of the float32 value), the tail as
+//        float32 in the 14 halves after them (4-byte aligned: even stride, aligned base).
+// F = float for rows that are written, const float for rows that are only read; the row storage
+// is passed as F * in either format (the C ABI's obs pointers).  A stored scan value moves from
+// slot to slot of the stack as `p[dst] = p[src]` in both formats: float16 rounding is idempotent,
+// so a shifted float16 history equals the rounded float32 history.
+template <int FMT, typename F = float> struct ObsRow;
+template <typename F> struct ObsRow<NAVGYM_OBS_F32, F> {
+    using E = F;   // element type
+    E *p;          // the scans, then the tail
+    __device__ __forceinline__ ObsRow(F *obs, size_t row, int stride) : p(obs + row * stride) {}
+    __device__ __forceinline__ float scan(int i) const { return p[i]; }
+    __device__ __forceinline__ void set_scan(int i, float v) const { p[i] = v; }
+    __device__ __forceinline__ void set_tail(int S, int f, float v) const { p[S * NB + f] = v; }
+    // the tail, from the row's last scan
+    static __device__ __forceinline__ F *tail_after(E *last_scan) { return last_scan + NB; }
+};
+template <typename F> struct ObsRow<NAVGYM_OBS_F16, F> {
+    using E = typename std::conditional<std::is_const<F>::value, const __half, __half>::type;
+    E *p;
+    __device__ __forceinline__ ObsRow(F *obs, size_t row, int stride) : p(reinterpret_cast<E *>(obs) + row * stride) {}
+    __device__ __forceinline__ float scan(int i) const { return __half2float(p[i]); }
+    __device__ __forceinline__ void set_scan(int i, float v) const { p[i] = __float2half_rn(v); }
+    __device__ __forceinline__ void set_tail(int S, int f, float v) const { reinterpret_cast<F *>(p + S * NB)[f] = v; }
+    static __device__ __forceinline__ F *tail_after(E *last_scan) { return reinterpret_cast<F *>(last_scan + NB); }
+};
+
+// Scan value i of a row of either format (runtime format: debug / export paths only).
+__device__ __forceinline__ float obs_scan_at(const float *obs, int format, size_t row, int stride, int i)
+{
+    if (format == NAVGYM_OBS_F16) return ObsRow<NAVGYM_OBS_F16, const float>(obs, row, stride).scan(i);
+    return ObsRow<NAVGYM_OBS_F32, const float>(obs, row, stride).scan(i);
+}

@@ -5,18 +5,28 @@
 // (env.py:464-589: the reference's hindsight-relabelling entry points).  Observation row
 // [scan(512) | prev_pose(2) pose(2) vel(2) yaw(1)], goals given separately.
 //
-// HBM-bound: 2095 algorithmic bytes per row (2076 row + 8 goal in, 11 out) against ~250 instructions.
-// One warp per row at a time, warps striding over the rows: lane l owns beams l + 32 i, whose
-// thresholds stay in its registers for every row the warp handles; the 16 row loads of a lane are
-// independent streaming loads (128 contiguous bytes per warp and load; rows are consumed once and
-// should not displace anything in L2), 32 warps per SM keep 64 KB in flight.  The discomfort ratio
+// HBM-bound: 2095 algorithmic bytes per row (2076 row + 8 goal in, 11 out) against ~250 instructions;
+// with float16 scans (FMT = NAVGYM_OBS_F16) 1075 (a 1056-byte row).
+// One warp per row at a time, warps striding over the rows: lane l owns 16 beams, whose thresholds
+// stay in its registers for every row the warp handles -- beams l + 32 i of float32 rows, the two
+// beams of half2 words l + 32 i of float16 rows; the row loads of a lane are independent streaming
+// loads (128 contiguous bytes per warp and load; rows are consumed once and should not displace
+// anything in L2), 32 warps per SM keep 64 KB (float16: 32 KB) in flight.  The discomfort ratio
 // min_k (scan_k - thr_k) / (dthr_k - thr_k + 1e-6) -- 512 float64 divisions -- is only evaluated for
 // rows that are in discomfort (a warp-uniform branch), from the row already in registers; the two
-// goal distances are taken by lanes 0 and 1 side by side.
+// goal distances are taken by lanes 0 and 1 side by side.  Crash, discomfort and the minimum do not
+// depend on which lane holds which beam, so both formats give the results of the float32 values.
 #define NAVGYM_HER_THREADS 256
 #ifndef NAVGYM_HER_CTAS_PER_SM
 #define NAVGYM_HER_CTAS_PER_SM 4
 #endif
+template <int FMT>
+__device__ __forceinline__ int her_beam(int lane, int i)
+{
+    return FMT == NAVGYM_OBS_F16 ? 2 * (lane + 32 * (i >> 1)) + (i & 1) : lane + 32 * i;
+}
+
+template <int FMT>
 __global__ void __launch_bounds__(NAVGYM_HER_THREADS, NAVGYM_HER_CTAS_PER_SM) her_kernel(const navgym_her_args_t a)
 {
     constexpr int BPL = NB / 32;
@@ -28,17 +38,27 @@ __global__ void __launch_bounds__(NAVGYM_HER_THREADS, NAVGYM_HER_CTAS_PER_SM) he
     float thr[BPL], dthr[BPL];
 #pragma unroll
     for (int i = 0; i < BPL; i++) {
-        thr[i] = a.thr[lane + 32 * i];
-        dthr[i] = a.dthr[lane + 32 * i];
+        thr[i] = a.thr[her_beam<FMT>(lane, i)];
+        dthr[i] = a.dthr[her_beam<FMT>(lane, i)];
     }
     for (int n = blockIdx.x * warps_per_cta + (threadIdx.x >> 5); n < a.count; n += stride) {
-        const float *o = a.obs + (size_t)n * a.obs_stride + (size_t)(SS - 1) * NB;  // the newest scan
+        using Row = ObsRow<FMT, const float>;
+        const typename Row::E *o = Row(a.obs, (size_t)n, a.obs_stride).p + (size_t)(SS - 1) * NB;   // the newest scan
         float v[BPL];
+        if constexpr (FMT == NAVGYM_OBS_F16) {
 #pragma unroll
-        for (int i = 0; i < BPL; i++) v[i] = __ldcs(o + lane + 32 * i);
+            for (int i = 0; i < BPL / 2; i++) {
+                const float2 f = __half22float2(__ldcs(reinterpret_cast<const __half2 *>(o) + lane + 32 * i));
+                v[2 * i] = f.x;
+                v[2 * i + 1] = f.y;
+            }
+        } else {
+#pragma unroll
+            for (int i = 0; i < BPL; i++) v[i] = __ldcs(o + lane + 32 * i);
+        }
         // lanes 0..5: prev_pose(2) pose(2) vel(2); lanes 6, 7: the goal
         float tv = 0.0f;
-        if (lane < 6) tv = __ldcs(o + NB + lane);
+        if (lane < 6) tv = __ldcs(Row::tail_after(o) + lane);
         else if (lane < 8) tv = __ldcs(a.goals + 2 * (size_t)n + (lane - 6));
         bool c_any = false, d_any = false;
 #pragma unroll

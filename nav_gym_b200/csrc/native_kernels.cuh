@@ -76,7 +76,7 @@ __global__ void render_in_lidar_kernel(float *__restrict__ ranges, const float *
 // Everything the single-environment drop-in reads back per step (SURVEY 8f row 4), packed into
 // one float64 row so that the host needs ONE device-to-host copy:
 //   [0..NS) state rows | [NS..NS+7) tail64 | reward done is_success is_crash truncated distance
-//   steps map_id episode noise_std | S*512 scan values (float32 -> float64, exact)
+//   steps map_id episode noise_std | S*512 scan values (float32 or float16 -> float64, exact)
 #define NAVGYM_EXPORT_HEAD (NAVGYM_NS + NAVGYM_OBS_TAIL + 10)
 __global__ void export_env_kernel(const navgym_step_args_t a, int e, double *out)
 {
@@ -99,7 +99,7 @@ __global__ void export_env_kernel(const navgym_step_args_t a, int e, double *out
             case 8: v = a.episodes ? (double)a.episodes[e] : 0.0; break;
             case 9: v = a.noise_std ? (double)a.noise_std[e] : 0.0; break;
             }
-        } else v = (double)a.obs[(size_t)e * a.obs_stride + (i - NAVGYM_EXPORT_HEAD)];
+        } else v = (double)obs_scan_at(a.obs, a.obs_format, e, a.obs_stride, i - NAVGYM_EXPORT_HEAD);
         out[i] = v;
     }
 }

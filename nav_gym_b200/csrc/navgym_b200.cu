@@ -33,6 +33,7 @@
 #include <stdlib.h>
 #include <string.h>
 #include <mutex>
+#include <type_traits>
 
 #include "../../include/navgym_b200.h"
 
@@ -66,6 +67,13 @@ static int coop_default_max()
 }
 
 // Launch shape of the fused kernel: one 64-thread CTA per environment of the launch.
+template <bool RESET, int FMT>
+static void launch_step_fmt(const navgym_step_args_t &a, int count, bool coop, cudaStream_t st)
+{
+    if (coop) step_kernel<RESET, true, FMT><<<count, NAVGYM_CTA_THREADS, 0, st>>>(a);
+    else step_kernel<RESET, false, FMT><<<count, NAVGYM_CTA_THREADS, 0, st>>>(a);
+}
+
 template <bool RESET>
 static cudaError_t launch_step(const navgym_step_args_t &a, cudaStream_t st)
 {
@@ -75,10 +83,22 @@ static cudaError_t launch_step(const navgym_step_args_t &a, cudaStream_t st)
     // tail regime B (see step_kernel) while the launch is at most ~2.4 waves of CTAs (measured
     // crossover on B200: 5120 envs -2 %, 6144 envs +2 %); NAVGYM_COOP_MAX_ENVS overrides
     static const int coop_max = env_int("NAVGYM_COOP_MAX_ENVS", coop_default_max());
-    if (count <= coop_max) step_kernel<RESET, true><<<count, NAVGYM_CTA_THREADS, 0, st>>>(a);
-    else step_kernel<RESET, false><<<count, NAVGYM_CTA_THREADS, 0, st>>>(a);
+    if (a.obs_format == NAVGYM_OBS_F16) launch_step_fmt<RESET, NAVGYM_OBS_F16>(a, count, count <= coop_max, st);
+    else launch_step_fmt<RESET, NAVGYM_OBS_F32>(a, count, count <= coop_max, st);
     g_launches++;
     return cudaSuccess;
+}
+
+// Observation rows (include/navgym_b200.h NAVGYM_OBS_*): a known format, a stride that holds S
+// scans and the tail, and for float16 rows an even stride and a 4-byte aligned base (the tail is
+// stored as float32).  `obs` is the row storage the call reads or writes.
+static bool obs_rows_ok(int format, int stride, int num_scan_stack, const void *obs)
+{
+    const int scans = (num_scan_stack > 1 ? num_scan_stack : 1) * NB;
+    if (format == NAVGYM_OBS_F32) return stride >= scans + NAVGYM_OBS_TAIL;
+    if (format == NAVGYM_OBS_F16)
+        return stride % 2 == 0 && stride >= scans + 2 * NAVGYM_OBS_TAIL && ((uintptr_t)obs & 3) == 0;
+    return false;
 }
 
 #define CK(x) do { cudaError_t _e = (x); if (_e != cudaSuccess) return (int)_e; } while (0)
@@ -119,7 +139,8 @@ int navgym_device_count(void)
 int navgym_step_batch(const navgym_step_args_t *args, void *stream)
 {
     if (args->num_envs <= 0) return 0;
-    if (args->obs_stride < (args->num_scan_stack > 1 ? args->num_scan_stack : 1) * NB + NAVGYM_OBS_TAIL || args->env_begin < 0 || args->env_begin + args->env_count > args->num_envs)
+    if (!obs_rows_ok(args->obs_format, args->obs_stride, args->num_scan_stack, args->obs) || args->env_begin < 0 ||
+        args->env_begin + args->env_count > args->num_envs)
         return (int)cudaErrorInvalidValue;
     const cudaError_t err = launch_step<false>(*args, (cudaStream_t)stream);
     return (int)(err ? err : cudaGetLastError());
@@ -130,7 +151,7 @@ int navgym_step_batch(const navgym_step_args_t *args, void *stream)
 int navgym_reset_obs_batch(const navgym_step_args_t *args, void *stream)
 {
     if (args->num_envs <= 0) return 0;
-    if (args->obs_stride < (args->num_scan_stack > 1 ? args->num_scan_stack : 1) * NB + NAVGYM_OBS_TAIL)
+    if (!obs_rows_ok(args->obs_format, args->obs_stride, args->num_scan_stack, args->obs))
         return (int)cudaErrorInvalidValue;
     const cudaError_t err = launch_step<true>(*args, (cudaStream_t)stream);
     return (int)(err ? err : cudaGetLastError());
@@ -152,7 +173,7 @@ int navgym_export_env(const navgym_step_args_t *args, int env, double *out_dev, 
 int navgym_compute_rewards(const navgym_her_args_t *args, void *stream)
 {
     if (args->count <= 0) return 0;
-    if (args->obs_stride < (args->num_scan_stack > 1 ? args->num_scan_stack : 1) * NB + NAVGYM_OBS_TAIL)
+    if (!obs_rows_ok(args->obs_format, args->obs_stride, args->num_scan_stack, args->obs))
         return (int)cudaErrorInvalidValue;
     // warps stride over the rows: at most one full wave of CTAs
     static int sms = 0;
@@ -163,7 +184,10 @@ int navgym_compute_rewards(const navgym_her_args_t *args, void *stream)
     const int warps_per_cta = NAVGYM_HER_THREADS / 32;
     const int want = (args->count + warps_per_cta - 1) / warps_per_cta;
     const int ctas = want < sms * NAVGYM_HER_CTAS_PER_SM ? want : sms * NAVGYM_HER_CTAS_PER_SM;
-    her_kernel<<<ctas, NAVGYM_HER_THREADS, 0, (cudaStream_t)stream>>>(*args);
+    if (args->obs_format == NAVGYM_OBS_F16)
+        her_kernel<NAVGYM_OBS_F16><<<ctas, NAVGYM_HER_THREADS, 0, (cudaStream_t)stream>>>(*args);
+    else
+        her_kernel<NAVGYM_OBS_F32><<<ctas, NAVGYM_HER_THREADS, 0, (cudaStream_t)stream>>>(*args);
     g_launches++;
     return (int)cudaGetLastError();
 }

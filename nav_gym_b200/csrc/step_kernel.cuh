@@ -409,7 +409,7 @@ __device__ __forceinline__ void march_scan(EnvSmem &sm, const navgym_step_args_t
 #ifndef NAVGYM_CTAS_PER_SM
 #define NAVGYM_CTAS_PER_SM 16  // resident CTAs the register budget is tuned for (64 registers)
 #endif
-template <bool IS_RESET_KERNEL, int WPE, bool COOP>
+template <bool IS_RESET_KERNEL, int WPE, bool COOP, int FMT>
 __device__ __forceinline__ void step_body(const navgym_step_args_t &a, EnvSmem &sm, const int e, const int tid,
                                           int *sched_cnt, int *sched_list)
 {
@@ -510,7 +510,7 @@ __device__ __forceinline__ void step_body(const navgym_step_args_t &a, EnvSmem &
     int nd = a.discs ? min(a.ndisc[e], a.max_disc) : 0;
     int ns = a.segs ? min(a.nseg[e], a.max_seg) : 0;
     int pass = IS_RESET_KERNEL ? PASS_RESET : PASS_STEP;
-    float *orow = a.obs + (size_t)e * a.obs_stride;
+    const ObsRow<FMT> orow(a.obs, (size_t)e, a.obs_stride);   // the row format is a template parameter
 
     long long t_pass = t_begin;  // start of the pass that produces the returned observation
     float margin = CUDART_INF_F; // its smallest clearance over the crash thresholds [m]
@@ -699,17 +699,17 @@ __device__ __forceinline__ void step_body(const navgym_step_args_t &a, EnvSmem &
                     }
                     sm.scan[k] = __float_as_int(v);
                     if (SS == 1) {
-                        orow[k] = v;
+                        orow.set_scan(k, v);
                     } else {
                         // _stack_scan (env.py:257-279): [pads = current scan | previous scans,
                         // oldest first | current scan]; the previous observation row still holds
                         // them one slot to the right
                         const int hist = pass == PASS_RESET ? 0 : min(steps, SS - 1);
                         for (int j = 0; j < SS - 1; j++) {
-                            if (j < SS - 1 - hist) orow[j * NB + k] = v;
-                            else if (pass == PASS_STEP) orow[j * NB + k] = orow[(j + 1) * NB + k];
+                            if (j < SS - 1 - hist) orow.set_scan(j * NB + k, v);
+                            else if (pass == PASS_STEP) orow.p[j * NB + k] = orow.p[(j + 1) * NB + k];   // stored value, either format
                         }
-                        orow[(SS - 1) * NB + k] = v;
+                        orow.set_scan((SS - 1) * NB + k, v);
                     }
                     const float thr_k = a.thr[k];
                     c_any |= v < thr_k;
@@ -855,7 +855,7 @@ __device__ __forceinline__ void step_body(const navgym_step_args_t &a, EnvSmem &
         case 6: tv = yaw; break;
         }
         if (lane < 7) {
-            orow[(a.num_scan_stack > 1 ? a.num_scan_stack : 1) * NB + lane] = (float)tv;
+            orow.set_tail(a.num_scan_stack > 1 ? a.num_scan_stack : 1, lane, (float)tv);
             if (a.tail64) a.tail64[(size_t)e * 7 + lane] = tv;
         }
         double nv = 0.0;
@@ -929,8 +929,9 @@ __device__ __forceinline__ int sched_lookup(const navgym_step_args_t &a, const i
 // One CTA (2 warps) = one environment; CTA b of the launch takes the b-th environment of the
 // launch order.  COOP selects tail regime B (march_tail_dealt): it shortens the launch's slowest
 // environments at the price of ~4 % more gathers and instructions, which pays while a launch is
-// at most ~2 waves of CTAs (4096 envs: -16 %) and costs beyond (32768 envs: +7 %).
-template <bool IS_RESET_KERNEL, bool COOP>
+// at most ~2 waves of CTAs (4096 envs: -16 %) and costs beyond (32768 envs: +7 %).  FMT is the
+// observation row format (NAVGYM_OBS_F32 / F16, ObsRow): it only changes the row stores.
+template <bool IS_RESET_KERNEL, bool COOP, int FMT>
 __global__ void __launch_bounds__(NAVGYM_CTA_THREADS, NAVGYM_CTAS_PER_SM) step_kernel(const navgym_step_args_t a)
 {
     __shared__ EnvSmem sm;
@@ -938,5 +939,5 @@ __global__ void __launch_bounds__(NAVGYM_CTA_THREADS, NAVGYM_CTAS_PER_SM) step_k
     int e = a.env_begin + (int)blockIdx.x;
     int *sched_cnt = nullptr, *sched_list = nullptr;
     if (!IS_RESET_KERNEL && a.sched) e = sched_lookup(a, (int)blockIdx.x, sched_cnt, sched_list);
-    step_body<IS_RESET_KERNEL, WPE, COOP>(a, sm, e, (int)threadIdx.x, sched_cnt, sched_list);
+    step_body<IS_RESET_KERNEL, WPE, COOP, FMT>(a, sm, e, (int)threadIdx.x, sched_cnt, sched_list);
 }
