@@ -201,6 +201,34 @@ void navgym_policy_action_bank(void *user, int group, int env_begin, int env_end
                                const uint8_t *done_host, float *actions_host);
 /* first observation of an episode, NavGymEnv.reset's tail (env.py:822-831) */
 int navgym_reset_obs_batch(const navgym_step_args_t *args, void *stream);
+/* Masked device reset: new episodes for chosen environments, exactly as the step's auto-reset
+ * starts them, for callers that step with auto_reset = 0 so that they can read each ended
+ * episode's final observation row (and its goal, state[NAVGYM_S_GX / S_GY]) first.  One launch;
+ * mask u8 [num_envs] on the device.  For every environment e of the launch range [env_begin,
+ * env_begin + count) (count = env_count, 0 = through num_envs) with mask[e] != 0:
+ *   1. the next episode is drawn as the auto-reset of navgym_step_batch draws it: Philox key
+ *      (env_offset + e, episodes[e], 0x5eed, 0xfffffff0) with `seed`; a new map when
+ *      resample_map && num_maps > 1; a spawn row (start, goal, theta) of that map's pool;
+ *      noise_std = noise_lo + (noise_hi - noise_lo) * u01; then episodes[e] += 1, steps[e] = 0.
+ *      A map without a spawn pool keeps the pose and goal in `state` (and its map): the
+ *      auto-reset would restart from the pose before the ending step instead, so for such maps
+ *      the two are not equivalent;
+ *   2. the first observation is written as the auto-reset pass writes it: the obs row in
+ *      obs_format (all S stack slots hold the new scan), tail64, the state rows (previous pose =
+ *      pose, previous action 0, previous yaw = yaw), map_id, noise_std.  The scan is taken
+ *      against discs_reset / segs_reset when discs_reset != NULL, else against discs / segs, with
+ *      the same noise as the auto-reset pass (Philox, or slot 0 of `noise`);
+ *   3. hits are not written (they keep the step's first scan, as with auto-reset).
+ * Whatever the mask, reward, done, is_success, is_crash, truncated, distance, the mirrors and
+ * sched are not written (the step already filed every environment into the next launch order),
+ * and environments with mask[e] == 0 are not written at all.  auto_reset and actions are not
+ * read.  After navgym_step_batch with auto_reset = 0 and then this call with mask = done, every
+ * buffer above holds what the step with auto_reset = 1 would have left, bit for bit (pools with
+ * spawn rows).  Each draw depends only on the environment's own episodes[e], so the result does
+ * not depend on how the masked set is split across calls or env_offset shards.
+ * cudaErrorInvalidValue: mask == NULL, obs rows as navgym_step_batch rejects them, or an env range
+ * outside [0, num_envs).  num_envs <= 0 is a no-op. */
+int navgym_reset_envs(const navgym_step_args_t *args, const uint8_t *mask, void *stream);
 
 /* ---- host export of one environment (ros_env.py:69-176 reads a NavGymEnv's attributes; the
  * single-env drop-in returns numpy per step, env.py:728): everything it needs from environment

@@ -180,7 +180,7 @@ class PolicyParams(C.Structure):
 
 
 EXPORTS = [
-    'navgym_step_batch', 'navgym_reset_obs_batch', 'navgym_host_pipe_create', 'navgym_host_pipe_destroy',
+    'navgym_step_batch', 'navgym_reset_obs_batch', 'navgym_reset_envs', 'navgym_host_pipe_create', 'navgym_host_pipe_destroy',
     'navgym_step_batch_host', 'navgym_step_batch_host_submit', 'navgym_step_batch_host_wait', 'navgym_edt_build', 'navgym_calc_range_many',
     'navgym_raymarching_create_host', 'navgym_raymarching_calc_range_many_host',
     'navgym_raymarching_edt_dev', 'navgym_raymarching_edt_host', 'navgym_raymarching_destroy',
@@ -212,6 +212,7 @@ def load():
     lib = C.CDLL(SO)
     lib.navgym_step_batch.argtypes = [C.POINTER(StepArgs), _P]
     lib.navgym_reset_obs_batch.argtypes = [C.POINTER(StepArgs), _P]
+    lib.navgym_reset_envs.argtypes = [C.POINTER(StepArgs), _P, _P]
     lib.navgym_host_pipe_create.restype = _P
     lib.navgym_host_pipe_create.argtypes = [C.c_int, C.c_int, C.c_int]
     lib.navgym_host_pipe_destroy.restype = None

@@ -548,6 +548,62 @@ class BatchedNavGym(object):
             _lib.check(self.lib.navgym_reset_obs_batch(C.byref(self.args), self._stream()), 'reset')
         return self.obs
 
+    def env_mask(self, envs):
+        """u8 [B] device mask of `envs`: a bool / uint8 [B] tensor on the env's device (returned
+        as is, a bool tensor viewed as uint8: no copy), or a 1-D sequence / integer tensor of env
+        ids (a new mask).  ValueError for anything else, or for ids outside [0, B)."""
+        if torch.is_tensor(envs) and envs.dtype in (torch.bool, torch.uint8):
+            if envs.device != self.device:
+                raise ValueError('mask on %s, the env lives on %s' % (envs.device, self.device))
+            if envs.dim() != 1 or envs.shape[0] != self.B:
+                raise ValueError('mask of shape %s, expected [%d]' % (tuple(envs.shape), self.B))
+            m = envs.contiguous()
+            return m.view(torch.uint8) if m.dtype == torch.bool else m
+        if torch.is_tensor(envs):
+            if envs.dtype.is_floating_point or envs.dtype.is_complex:
+                raise ValueError('env ids of dtype %s: pass a bool / uint8 mask or integer ids' % envs.dtype)
+            if envs.device.type != 'cpu' and envs.device != self.device:
+                raise ValueError('env ids on %s, the env lives on %s' % (envs.device, self.device))
+            if envs.dim() > 1:
+                raise ValueError('env ids must be 1-D')
+            ids = envs.reshape(-1).to(device=self.device, dtype=torch.int64)
+        else:
+            arr = np.asarray(envs)
+            if arr.size and arr.dtype.kind not in 'iu':
+                raise ValueError('env ids of dtype %s: pass a bool / uint8 mask or integer ids' % arr.dtype)
+            if arr.ndim > 1:
+                raise ValueError('env ids must be 1-D')
+            ids = torch.from_numpy(arr.astype(np.int64).reshape(-1)).to(self.device)
+        if ids.numel() and (int(ids.min()) < 0 or int(ids.max()) >= self.B):
+            raise ValueError('env ids outside [0, %d)' % self.B)
+        m = torch.zeros(self.B, dtype=torch.uint8, device=self.device)
+        m[ids] = 1
+        return m
+
+    def reset_envs(self, envs):
+        """Start new episodes for the environments `envs` only, on the device, exactly as
+        auto-reset would have started them (navgym_reset_envs): the same spawn / map / noise draw
+        from each env's own episode counter, the same first observation.  Everything else is left
+        as it is.  `envs`: a bool / uint8 [B] tensor on the env's device (env.done itself works,
+        without a copy or a host sync) or a 1-D sequence / integer tensor of env ids.  Returns
+        self.obs.
+
+        Meant for auto_reset=False: step, read the rows of the ended episodes (their final
+        observations; their goals are still state[S_GX / S_GY]), then reset_envs(done).  Works with
+        auto_reset=True too.  With scripted pedestrians the first scan sees the geometry the last
+        step emitted, not advanced, as auto-reset does.  An env driven by a PedestrianSim is reset
+        through sim.reset_envs, which also respawns its pedestrians."""
+        if getattr(self, 'crowd', None) is not None:
+            raise ValueError('this env is driven by a PedestrianSim: call sim.reset_envs(envs), which also '
+                             'respawns its pedestrians')
+        return self._reset_envs(self.env_mask(envs))
+
+    def _reset_envs(self, mask):
+        self._reset_mask = mask  # kept alive until the next call; the launch is stream-ordered
+        with torch.cuda.device(self.device):
+            _lib.check(self.lib.navgym_reset_envs(C.byref(self.args), _ptr(mask), self._stream()), 'reset_envs')
+        return self.obs
+
     def step(self, actions, discs=None, ndisc=None, segs=None, nseg=None, noise=None):
         """One lockstep NavGymEnv.step.  Returned tensors are owned by the env and overwritten
         by the next call (clone to keep)."""

@@ -129,6 +129,36 @@ __device__ __forceinline__ uint4 philox4x32_10(uint4 c, uint2 k)
 
 __device__ __forceinline__ float u01(uint32_t x) { return ((float)(x >> 8) + 0.5f) * (1.0f / 16777216.0f); }
 
+// The draw that starts environment `env`'s next episode (global id, episode = its episode counter
+// BEFORE the new episode): one Philox call keyed (env, episode, 0x5eed, 0xfffffff0) with `seed`.
+// A new map when resample_map && num_maps > 1, and a spawn row of that map's pool: spawn(row, map)
+// is called with the row (start x, y, goal x, y, theta) and the drawn map, or no_pool() when that
+// map has no spawn pool.  Returns the new episode's scan-noise std.  The step kernel's auto-reset
+// and the masked reset (navgym_reset_envs) both draw through here, so the two cannot disagree on
+// where an episode starts (peds_plan spells the same draw out for the pedestrians' next-episode
+// candidates).  The argument-block fields are taken by reference and the outcomes handed to
+// callbacks, so the auto-reset branch compiles to the code it had when it spelled the draw out.
+template <typename Spawn, typename NoPool>
+__device__ __forceinline__ float draw_episode(const navgym_map_t *const &maps, const double *const &spawn_pool,
+                                              const int32_t &num_maps, const int32_t &resample_map,
+                                              const uint64_t &seed, uint32_t env, uint32_t episode, int map,
+                                              const float &noise_lo, const float &noise_hi, Spawn &&spawn,
+                                              NoPool &&no_pool)
+{
+    const uint4 rnd = philox4x32_10(make_uint4(env, episode, 0x5eedu, 0xfffffff0u),
+                                    make_uint2((uint32_t)seed, (uint32_t)(seed >> 32)));
+    int nmap = map;
+    if (resample_map && num_maps > 1) nmap = (int)(((uint64_t)rnd.y * (uint64_t)num_maps) >> 32);
+    const navgym_map_t m2 = maps[nmap];
+    if (m2.spawn_count > 0) {
+        const long long row = m2.spawn_offset + (long long)(((uint64_t)rnd.x * (uint64_t)m2.spawn_count) >> 32);
+        spawn(spawn_pool + row * 5, nmap);
+    } else {
+        no_pool();
+    }
+    return noise_lo + (noise_hi - noise_lo) * u01(rnd.z);
+}
+
 // The observation row layouts (include/navgym_b200.h NAVGYM_OBS_*), the one place that knows
 // them.  Element i < S*512 of p is a scan value; the 7 tail fields follow the S scans.
 //   F32: float[obs_stride].

@@ -67,24 +67,34 @@ static int coop_default_max()
 }
 
 // Launch shape of the fused kernel: one 64-thread CTA per environment of the launch.
-template <bool RESET, int FMT>
-static void launch_step_fmt(const navgym_step_args_t &a, int count, bool coop, cudaStream_t st)
+template <int MODE, int FMT>
+static void launch_step_fmt(const navgym_step_args_t &a, const uint8_t *mask, int count, bool coop, cudaStream_t st)
 {
-    if (coop) step_kernel<RESET, true, FMT><<<count, NAVGYM_CTA_THREADS, 0, st>>>(a);
-    else step_kernel<RESET, false, FMT><<<count, NAVGYM_CTA_THREADS, 0, st>>>(a);
+    if constexpr (MODE == MODE_MASKED_RESET) {
+        if (coop) reset_envs_kernel<true, FMT><<<count, NAVGYM_CTA_THREADS, 0, st>>>(a, mask);
+        else reset_envs_kernel<false, FMT><<<count, NAVGYM_CTA_THREADS, 0, st>>>(a, mask);
+    } else {
+        if (coop) step_kernel<MODE, true, FMT><<<count, NAVGYM_CTA_THREADS, 0, st>>>(a);
+        else step_kernel<MODE, false, FMT><<<count, NAVGYM_CTA_THREADS, 0, st>>>(a);
+    }
 }
 
-template <bool RESET>
-static cudaError_t launch_step(const navgym_step_args_t &a, cudaStream_t st)
+// MODE_STEP / MODE_RESET / MODE_MASKED_RESET (step_kernel.cuh) over the launch's env range;
+// `mask` is read by the masked reset only.
+template <int MODE>
+static cudaError_t launch_step(const navgym_step_args_t &a, cudaStream_t st, const uint8_t *mask = nullptr)
 {
     const int count = a.env_count > 0 ? a.env_count : a.num_envs - a.env_begin;
     // the obstacle windows of an environment are parked in NB / 2 shared-memory slots
     if ((a.discs ? a.max_disc : 0) + (a.segs ? a.max_seg : 0) > NB / 2) return cudaErrorInvalidValue;
+    // (the masked reset may scan the next episode's geometry alone)
+    if (MODE == MODE_MASKED_RESET && (a.discs_reset ? a.max_disc : 0) + (a.segs_reset ? a.max_seg : 0) > NB / 2)
+        return cudaErrorInvalidValue;
     // tail regime B (see step_kernel) while the launch is at most ~2.4 waves of CTAs (measured
     // crossover on B200: 5120 envs -2 %, 6144 envs +2 %); NAVGYM_COOP_MAX_ENVS overrides
     static const int coop_max = env_int("NAVGYM_COOP_MAX_ENVS", coop_default_max());
-    if (a.obs_format == NAVGYM_OBS_F16) launch_step_fmt<RESET, NAVGYM_OBS_F16>(a, count, count <= coop_max, st);
-    else launch_step_fmt<RESET, NAVGYM_OBS_F32>(a, count, count <= coop_max, st);
+    if (a.obs_format == NAVGYM_OBS_F16) launch_step_fmt<MODE, NAVGYM_OBS_F16>(a, mask, count, count <= coop_max, st);
+    else launch_step_fmt<MODE, NAVGYM_OBS_F32>(a, mask, count, count <= coop_max, st);
     g_launches++;
     return cudaSuccess;
 }
@@ -142,7 +152,7 @@ int navgym_step_batch(const navgym_step_args_t *args, void *stream)
     if (!obs_rows_ok(args->obs_format, args->obs_stride, args->num_scan_stack, args->obs) || args->env_begin < 0 ||
         args->env_begin + args->env_count > args->num_envs)
         return (int)cudaErrorInvalidValue;
-    const cudaError_t err = launch_step<false>(*args, (cudaStream_t)stream);
+    const cudaError_t err = launch_step<MODE_STEP>(*args, (cudaStream_t)stream);
     return (int)(err ? err : cudaGetLastError());
 }
 
@@ -153,7 +163,19 @@ int navgym_reset_obs_batch(const navgym_step_args_t *args, void *stream)
     if (args->num_envs <= 0) return 0;
     if (!obs_rows_ok(args->obs_format, args->obs_stride, args->num_scan_stack, args->obs))
         return (int)cudaErrorInvalidValue;
-    const cudaError_t err = launch_step<true>(*args, (cudaStream_t)stream);
+    const cudaError_t err = launch_step<MODE_RESET>(*args, (cudaStream_t)stream);
+    return (int)(err ? err : cudaGetLastError());
+}
+
+int navgym_reset_envs(const navgym_step_args_t *args, const uint8_t *mask, void *stream)
+{
+    if (args->num_envs <= 0) return 0;
+    if (!mask || !obs_rows_ok(args->obs_format, args->obs_stride, args->num_scan_stack, args->obs) ||
+        args->env_begin < 0 || args->env_count < 0 || args->env_begin + args->env_count > args->num_envs ||
+        args->env_begin > args->num_envs)
+        return (int)cudaErrorInvalidValue;
+    if (args->env_begin == args->num_envs) return 0;   // an empty range
+    const cudaError_t err = launch_step<MODE_MASKED_RESET>(*args, (cudaStream_t)stream, mask);
     return (int)(err ? err : cudaGetLastError());
 }
 

@@ -330,7 +330,9 @@ __global__ void peds_plan_kernel(const navgym_plan_args_t a)
         double rx = a.robot_state[NAVGYM_S_PX * B + e], ry = a.robot_state[NAVGYM_S_PY * B + e];
         int nmap = a.map_id[e];
         if (a.cand_next_spawn && a.robot_maps) {
-            // the spawn tuple step_kernel draws on auto-reset (keep in step with it)
+            // the spawn tuple step_kernel draws on auto-reset and navgym_reset_envs draws
+            // (draw_episode in device_helpers.cuh: keep in step with it -- spelled out here because
+            // routing this kernel through the helper changes its register allocation)
             const uint4 rnd = philox4x32_10(make_uint4(ge, (uint32_t)(a.episodes ? a.episodes[e] : 0), 0x5eedu, 0xfffffff0u),
                                             make_uint2((uint32_t)a.robot_seed, (uint32_t)(a.robot_seed >> 32)));
             int cand_map = nmap;

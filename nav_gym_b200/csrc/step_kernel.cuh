@@ -409,10 +409,20 @@ __device__ __forceinline__ void march_scan(EnvSmem &sm, const navgym_step_args_t
 #ifndef NAVGYM_CTAS_PER_SM
 #define NAVGYM_CTAS_PER_SM 16  // resident CTAs the register budget is tuned for (64 registers)
 #endif
-template <bool IS_RESET_KERNEL, int WPE, bool COOP, int FMT>
+// What one CTA of the fused kernel does to its environment:
+//   MODE_STEP          one step (navgym_step_batch), auto-reset included;
+//   MODE_RESET         the first observation of an episode from the pose in `state`
+//                      (navgym_reset_obs_batch);
+//   MODE_MASKED_RESET  a new episode drawn exactly as the step's auto-reset draws it, then its
+//                      first observation as the auto-reset pass writes it (navgym_reset_envs):
+//                      no hits recorded, no launch-order filing.
+enum { MODE_STEP = 0, MODE_RESET = 1, MODE_MASKED_RESET = 2 };
+template <int MODE, int WPE, bool COOP, int FMT>
 __device__ __forceinline__ void step_body(const navgym_step_args_t &a, EnvSmem &sm, const int e, const int tid,
                                           int *sched_cnt, int *sched_list)
 {
+    constexpr bool IS_RESET_KERNEL = MODE != MODE_STEP;   // both reset modes: no action, a new episode
+    constexpr bool MASKED = MODE == MODE_MASKED_RESET;
     constexpr int BPL = NB / (32 * WPE);  // beams per lane
     constexpr int TPB = WPE * 32;         // threads of the CTA
     const int lane = tid & 31, warp = tid >> 5;
@@ -448,14 +458,26 @@ __device__ __forceinline__ void step_body(const navgym_step_args_t &a, EnvSmem &
     if (warp == 0) {
         double sv = lane < NAVGYM_NS ? ST(lane) : 0.0;
         int steps = a.steps[e];
-        const int map0 = a.map_id[e];
+        int map0 = a.map_id[e];
         const int episode0 = a.episodes ? a.episodes[e] : 0;
-        const float noise_std0 = a.noise_std ? a.noise_std[e] : 0.0f;
+        float noise_std0 = a.noise_std ? a.noise_std[e] : 0.0f;
         float2 av = make_float2(0.f, 0.f);
         if (!IS_RESET_KERNEL) av = *reinterpret_cast<const float2 *>(a.actions + 2 * (size_t)e);
+        // masked reset: the next episode's spawn row (and map), drawn before the map descriptor is read
+        const double *spawn = nullptr;
+        if (MASKED)
+            noise_std0 = draw_episode(a.maps, a.spawn_pool, a.num_maps, a.resample_map, a.seed,
+                                      (uint32_t)(a.env_offset + e), (uint32_t)episode0, map0, a.noise_lo, a.noise_hi,
+                                      [&](const double *sp, int nmap) { spawn = sp; map0 = nmap; }, [] {});
         const navgym_map_t m0 = a.maps[map0];
         double px = __shfl_sync(FULL, sv, NAVGYM_S_PX), py = __shfl_sync(FULL, sv, NAVGYM_S_PY);
         double th0 = __shfl_sync(FULL, sv, NAVGYM_S_TH), th = th0;
+        double gx = 0.0, gy = 0.0;
+        if (MASKED) {   // without a spawn pool the pose and goal in `state` stay
+            gx = __shfl_sync(FULL, sv, NAVGYM_S_GX);
+            gy = __shfl_sync(FULL, sv, NAVGYM_S_GY);
+            if (spawn) { px = spawn[0]; py = spawn[1]; gx = spawn[2]; gy = spawn[3]; th = spawn[4]; }
+        }
         double act_v = 0, act_w = 0;
         if (!IS_RESET_KERNEL) {
             double v = (double)av.x, w = (double)av.y;
@@ -486,8 +508,8 @@ __device__ __forceinline__ void step_body(const navgym_step_args_t &a, EnvSmem &
         // a host-side reset starts a new episode: a new noise / spawn stream (the in-kernel
         // auto-reset advances the same counter)
         const int episode1 = episode0 + (IS_RESET_KERNEL ? 1 : 0);
-        if (lane == NAVGYM_S_GX) sm.gx = sv;
-        if (lane == NAVGYM_S_GY) sm.gy = sv;
+        if (!MASKED && lane == NAVGYM_S_GX) sm.gx = sv;
+        if (!MASKED && lane == NAVGYM_S_GY) sm.gy = sv;
         if (!IS_RESET_KERNEL) {
             if (lane == NAVGYM_S_PPX) sm.ppx = sv;
             if (lane == NAVGYM_S_PPY) sm.ppy = sv;
@@ -503,12 +525,17 @@ __device__ __forceinline__ void step_body(const navgym_step_args_t &a, EnvSmem &
             sm.episode = episode1;
             sm.noise_std = noise_std0;
             if (IS_RESET_KERNEL) { sm.ppx = px; sm.ppy = py; sm.pyaw = 0; sm.pv = 0; sm.pw = 0; }
+            if (MASKED) { sm.gx = gx; sm.gy = gy; }
             if (WPE == 1) sm.th_spec = CUDART_NAN;
             pass_setup(sm, m0, a);  // first pass: the map descriptor is already here
         }
     }
     int nd = a.discs ? min(a.ndisc[e], a.max_disc) : 0;
     int ns = a.segs ? min(a.nseg[e], a.max_seg) : 0;
+    if (MASKED && a.discs_reset != nullptr) {   // the first scan sees the next episode's pedestrians, if given
+        nd = min(a.ndisc_reset[e], a.max_disc);
+        ns = a.segs_reset ? min(a.nseg_reset[e], a.max_seg) : 0;
+    }
     int pass = IS_RESET_KERNEL ? PASS_RESET : PASS_STEP;
     const ObsRow<FMT> orow(a.obs, (size_t)e, a.obs_stride);   // the row format is a template parameter
 
@@ -542,7 +569,7 @@ __device__ __forceinline__ void step_body(const navgym_step_args_t &a, EnvSmem &
             march_scan<WPE, COOP>(sm, a, 0, BPL / 4, tid);
             const int ci = sm.ci, cj = sm.cj;
             // ranges (env.py:426), all lanes active: sqrt(di^2 + dj^2) * resolution
-            const bool rec = pass == (IS_RESET_KERNEL ? PASS_RESET : PASS_STEP) && a.hits;
+            const bool rec = !MASKED && pass == (IS_RESET_KERNEL ? PASS_RESET : PASS_STEP) && a.hits;
             const float max_range = sm.max_range, res32 = sm.res32;
 #pragma unroll
             for (int i = 0; i < BPL; i++) {
@@ -572,8 +599,8 @@ __device__ __forceinline__ void step_body(const navgym_step_args_t &a, EnvSmem &
         if (ns + nd > 0) {
             if (tid == 0) { sm.n_vis_seg = 0; sm.n_vis_disc = 0; }
             cta_sync<WPE>();
-            // (the first scan after an auto-reset sees the next episode's pedestrians, if given)
-            const bool nxt = !IS_RESET_KERNEL && pass == PASS_RESET && a.discs_reset != nullptr;
+            // (the first scan after an auto-reset or of a masked reset sees the next episode's pedestrians, if given)
+            const bool nxt = MODE != MODE_RESET && pass == PASS_RESET && a.discs_reset != nullptr;
             const float *discs = (nxt ? a.discs_reset : a.discs) + (size_t)e * a.max_disc * 3;
             const float *segs = (nxt ? a.segs_reset : a.segs) + (size_t)e * a.max_seg * 4;
             // The visible obstacles are listed in the survivor list's shared memory (free since the tail
@@ -775,20 +802,16 @@ __device__ __forceinline__ void step_body(const navgym_step_args_t &a, EnvSmem &
                     int next = PASS_END;
                     if (done && a.auto_reset) {
                         // auto-reset: draw a spawn tuple (and a map) for the next episode
-                        uint4 rnd = philox4x32_10(make_uint4((uint32_t)(a.env_offset + e), (uint32_t)sm.episode, 0x5eedu, 0xfffffff0u),
-                                                  make_uint2((uint32_t)a.seed, (uint32_t)(a.seed >> 32)));
-                        int nmap = sm.map;
-                        if (a.resample_map && a.num_maps > 1) nmap = (int)(((uint64_t)rnd.y * (uint64_t)a.num_maps) >> 32);
-                        const navgym_map_t m2 = a.maps[nmap];
-                        if (m2.spawn_count > 0) {
-                            const long long row = m2.spawn_offset + (long long)(((uint64_t)rnd.x * (uint64_t)m2.spawn_count) >> 32);
-                            const double *sp = a.spawn_pool + row * 5;
-                            sm.px = sp[0]; sm.py = sp[1]; sm.gx = sp[2]; sm.gy = sp[3]; sm.th = sp[4];
-                            sm.map = nmap;
-                        } else {  // no pool: restart from the rolled-back pose
-                            sm.px = sm.ppx; sm.py = sm.ppy; sm.th = sm.pyaw;
-                        }
-                        sm.noise_std = a.noise_lo + (a.noise_hi - a.noise_lo) * u01(rnd.z);
+                        sm.noise_std = draw_episode(
+                            a.maps, a.spawn_pool, a.num_maps, a.resample_map, a.seed, (uint32_t)(a.env_offset + e),
+                            (uint32_t)sm.episode, sm.map, a.noise_lo, a.noise_hi,
+                            [&](const double *sp, int nmap) {
+                                sm.px = sp[0]; sm.py = sp[1]; sm.gx = sp[2]; sm.gy = sp[3]; sm.th = sp[4];
+                                sm.map = nmap;
+                            },
+                            [&] {  // no pool: restart from the rolled-back pose
+                                sm.px = sm.ppx; sm.py = sm.ppy; sm.th = sm.pyaw;
+                            });
                         sm.episode += 1;
                         sm.steps = 0;
                         sm.ppx = sm.px; sm.ppy = sm.py; sm.pv = 0; sm.pw = 0; sm.act_v = 0; sm.act_w = 0;
@@ -931,13 +954,27 @@ __device__ __forceinline__ int sched_lookup(const navgym_step_args_t &a, const i
 // environments at the price of ~4 % more gathers and instructions, which pays while a launch is
 // at most ~2 waves of CTAs (4096 envs: -16 %) and costs beyond (32768 envs: +7 %).  FMT is the
 // observation row format (NAVGYM_OBS_F32 / F16, ObsRow): it only changes the row stores.
-template <bool IS_RESET_KERNEL, bool COOP, int FMT>
+template <int MODE, bool COOP, int FMT>
 __global__ void __launch_bounds__(NAVGYM_CTA_THREADS, NAVGYM_CTAS_PER_SM) step_kernel(const navgym_step_args_t a)
 {
+    static_assert(MODE == MODE_STEP || MODE == MODE_RESET, "the masked reset is reset_envs_kernel");
     __shared__ EnvSmem sm;
     constexpr int WPE = NAVGYM_CTA_THREADS / 32;
     int e = a.env_begin + (int)blockIdx.x;
     int *sched_cnt = nullptr, *sched_list = nullptr;
-    if (!IS_RESET_KERNEL && a.sched) e = sched_lookup(a, (int)blockIdx.x, sched_cnt, sched_list);
-    step_body<IS_RESET_KERNEL, WPE, COOP, FMT>(a, sm, e, (int)threadIdx.x, sched_cnt, sched_list);
+    if (MODE == MODE_STEP && a.sched) e = sched_lookup(a, (int)blockIdx.x, sched_cnt, sched_list);
+    step_body<MODE, WPE, COOP, FMT>(a, sm, e, (int)threadIdx.x, sched_cnt, sched_list);
+}
+
+// The masked reset (navgym_reset_envs): CTA b takes environment env_begin + b in index order and
+// returns at once when its mask byte is 0; `sched` is neither read nor written.
+template <bool COOP, int FMT>
+__global__ void __launch_bounds__(NAVGYM_CTA_THREADS, NAVGYM_CTAS_PER_SM)
+reset_envs_kernel(const navgym_step_args_t a, const uint8_t *__restrict__ mask)
+{
+    __shared__ EnvSmem sm;
+    constexpr int WPE = NAVGYM_CTA_THREADS / 32;
+    const int e = a.env_begin + (int)blockIdx.x;
+    if (!mask[e]) return;
+    step_body<MODE_MASKED_RESET, WPE, COOP, FMT>(a, sm, e, (int)threadIdx.x, nullptr, nullptr);
 }

@@ -234,7 +234,8 @@ class PedestrianSim(object):
     least 4 m from where the robot's auto-reset will put it -- the same Philox draw the step
     kernel makes) and hands their geometry to the robot's step as discs_reset / segs_reset, so the
     first observation of a new episode already sees the new pedestrians; the next act() adopts
-    them for the environments whose episode ended.
+    them for the environments whose episode ended.  Over an auto_reset=False env, step and read
+    the final observations, then sim.reset_envs(env.done) does the same for those environments.
     """
 
     def __init__(self, env, max_ped, nped=None, policy=None, v_pref_range=(0.0, 0.6), has_legs_ratio=0.5,
@@ -335,9 +336,10 @@ class PedestrianSim(object):
         cp.peds, cp.discs, cp.ndisc = _ptr(self.cand_rows), _ptr(self.cand_discs), _ptr(self.cand_nd)
         cp.segs, cp.nseg = _ptr(self.cand_segs), _ptr(self.cand_ns)
         self.cand_pargs = cp
-        if ea.auto_reset:
-            ea.discs_reset, ea.ndisc_reset = _ptr(self.cand_discs), _ptr(self.cand_nd)
-            ea.segs_reset, ea.nseg_reset = _ptr(self.cand_segs), _ptr(self.cand_ns)
+        # (the step reads them only on auto-reset; navgym_reset_envs reads them in sim.reset_envs)
+        ea.discs_reset, ea.ndisc_reset = _ptr(self.cand_discs), _ptr(self.cand_nd)
+        ea.segs_reset, ea.nseg_reset = _ptr(self.cand_segs), _ptr(self.cand_ns)
+        self._pending = None  # u8 [B]: environments sim.reset_envs restarted, respawned at the next act()
         self.plan_args = a
         self._mean = torch.zeros(B, P, 2, dtype=f32, device=dev)
         mv = _lib.MoveArgs()
@@ -364,7 +366,7 @@ class PedestrianSim(object):
         a = self.plan_args
         self._respawn = respawn  # keep the tensor alive while the launch reads it
         a.respawn = _ptr(respawn)
-        a.cand_next_spawn = int(bool(next_spawn) and bool(self.env.args.auto_reset))
+        a.cand_next_spawn = int(bool(next_spawn))
         self._call(self.lib.navgym_peds_plan, a, 'peds_plan')
         a.step += 1
         self._call(self.lib.navgym_peds_advance, self.cand_pargs, 'peds_advance')  # candidates' geometry
@@ -378,6 +380,7 @@ class PedestrianSim(object):
     def reset(self):
         """Spawn every environment's pedestrians (env.py:785-806) around the robots' current poses
         and take their first scans."""
+        self._pending = None
         self._plan(None, next_spawn=False)  # draw them ...
         self._plan(self._all)               # ... adopt them, and draw the next episode's
         rows = self.env.peds
@@ -392,6 +395,9 @@ class PedestrianSim(object):
     def act(self):
         env = self.env
         respawn = env.done if env.args.auto_reset else None
+        if self._pending is not None:
+            respawn = self._pending if respawn is None else respawn | self._pending
+            self._pending = None
         self._plan(respawn)
         if respawn is not None:
             self._scan(respawn)  # first scans of the respawned pedestrians (env.py:808-815)
@@ -400,6 +406,23 @@ class PedestrianSim(object):
         self.native.mean(self.scan.reshape(self.B * self.P, -1), goal, speed, out=self._mean)
         self._call(self.lib.navgym_peds_move, self.move_args, 'peds_move')
         env._peds_emit(advance=False)
+
+    # ---- masked reset (BatchedNavGym.reset_envs for an env this sim drives) ------------------
+    @torch.no_grad()
+    def reset_envs(self, envs):
+        """New episodes for the environments `envs` (a bool / uint8 [B] device tensor such as
+        env.done, or env ids), exactly as auto-reset starts them: the robot's new episode
+        (navgym_reset_envs) with its first scan against the next episode's pedestrians, those
+        pedestrians adopted at the next act(), and the current pedestrians' scans of these
+        environments retaken with the robot at its new pose.  After `sim.step(actions)` on an
+        auto_reset=False env, `sim.reset_envs(env.done)` leaves the robot's and the pedestrians'
+        state as an auto_reset=True run would have, bit for bit.  Returns env.obs."""
+        env = self.env
+        mask = env.env_mask(envs)
+        env._reset_envs(mask)
+        self._pending = mask.clone() if self._pending is None else self._pending | mask
+        self._scan(mask)
+        return env.obs
 
     # ---- env.py:683-693 -------------------------------------------------------------------
     def observe(self):
