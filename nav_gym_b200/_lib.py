@@ -60,8 +60,7 @@ def build(force=False, verbose=False):
     nvcc = _nvcc()
     if nvcc is None:
         raise RuntimeError('nvcc not found: cannot build %s' % SO)
-    extra = os.environ.get('NAVGYM_NVCC_EXTRA', '').split()   # tuning builds: -DNAVGYM_... switches
-    cmd = [nvcc] + NVCC_FLAGS + extra + (['-Xptxas', '-v'] if verbose else []) + ['-o', SO, SRC]
+    cmd = [nvcc] + NVCC_FLAGS + (['-Xptxas', '-v'] if verbose else []) + ['-o', SO, SRC]
     subprocess.check_call(cmd)
     return SO
 

@@ -17,9 +17,7 @@
 // goal distances are taken by lanes 0 and 1 side by side.  Crash, discomfort and the minimum do not
 // depend on which lane holds which beam, so both formats give the results of the float32 values.
 #define NAVGYM_HER_THREADS 256
-#ifndef NAVGYM_HER_CTAS_PER_SM
-#define NAVGYM_HER_CTAS_PER_SM 4
-#endif
+constexpr int HER_CTAS_PER_SM = 4;
 template <int FMT>
 __device__ __forceinline__ int her_beam(int lane, int i)
 {
@@ -27,7 +25,7 @@ __device__ __forceinline__ int her_beam(int lane, int i)
 }
 
 template <int FMT>
-__global__ void __launch_bounds__(NAVGYM_HER_THREADS, NAVGYM_HER_CTAS_PER_SM) her_kernel(const navgym_her_args_t a)
+__global__ void __launch_bounds__(NAVGYM_HER_THREADS, HER_CTAS_PER_SM) her_kernel(const navgym_her_args_t a)
 {
     constexpr int BPL = NB / 32;
     const int lane = threadIdx.x & 31;

@@ -52,13 +52,6 @@ static unsigned long long g_launches = 0;
 #include "policy_gemm.cuh"
 
 // ------------------------------------------------------------------ C ABI
-// Integer tuning knobs read from the environment (documented in README.md).
-static int env_int(const char *name, int dflt)
-{
-    const char *s = getenv(name);
-    return s ? atoi(s) : dflt;
-}
-
 static int coop_default_max()
 {
     int dev = 0, sms = 148;
@@ -91,8 +84,8 @@ static cudaError_t launch_step(const navgym_step_args_t &a, cudaStream_t st, con
     if (MODE == MODE_MASKED_RESET && (a.discs_reset ? a.max_disc : 0) + (a.segs_reset ? a.max_seg : 0) > NB / 2)
         return cudaErrorInvalidValue;
     // tail regime B (see step_kernel) while the launch is at most ~2.4 waves of CTAs (measured
-    // crossover on B200: 5120 envs -2 %, 6144 envs +2 %); NAVGYM_COOP_MAX_ENVS overrides
-    static const int coop_max = env_int("NAVGYM_COOP_MAX_ENVS", coop_default_max());
+    // crossover on B200: 5120 envs -2 %, 6144 envs +2 %)
+    static const int coop_max = coop_default_max();
     if (a.obs_format == NAVGYM_OBS_F16) launch_step_fmt<MODE, NAVGYM_OBS_F16>(a, mask, count, count <= coop_max, st);
     else launch_step_fmt<MODE, NAVGYM_OBS_F32>(a, mask, count, count <= coop_max, st);
     g_launches++;
@@ -205,7 +198,7 @@ int navgym_compute_rewards(const navgym_her_args_t *args, void *stream)
     }
     const int warps_per_cta = NAVGYM_HER_THREADS / 32;
     const int want = (args->count + warps_per_cta - 1) / warps_per_cta;
-    const int ctas = want < sms * NAVGYM_HER_CTAS_PER_SM ? want : sms * NAVGYM_HER_CTAS_PER_SM;
+    const int ctas = want < sms * HER_CTAS_PER_SM ? want : sms * HER_CTAS_PER_SM;
     if (args->obs_format == NAVGYM_OBS_F16)
         her_kernel<NAVGYM_OBS_F16><<<ctas, NAVGYM_HER_THREADS, 0, (cudaStream_t)stream>>>(*args);
     else

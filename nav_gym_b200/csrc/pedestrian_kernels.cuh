@@ -98,9 +98,7 @@ __device__ __forceinline__ int4 segment_window(const float4 sg, float lx, float 
 // table (np.linspace: what the reference builds, env.py:388-390, and what pymap2d's renderers
 // assume); more than NAVGYM_SCAN_SEGS listed segments fall back to agent_scan_generic_kernel.
 #define NAVGYM_SCAN_SEGS (4 * (NAVGYM_SCAN_AGENTS + 1))
-#ifndef NAVGYM_AGENT_MIN_CTAS
-#define NAVGYM_AGENT_MIN_CTAS 12   // 40 registers: the kernel waits on its EDT gathers, 48 resident warps beat 36 (0.406 -> 0.350 ms for 40 960 agents)
-#endif
+constexpr int AGENT_MIN_CTAS = 12;   // 40 registers: the kernel waits on its EDT gathers, 48 resident warps beat 36 (0.406 -> 0.350 ms for 40 960 agents)
 __device__ __forceinline__ void agent_scan_one(const navgym_scan_args_t &a, const int n, float4 *near_segs, int4 *near_win, int &n_near)
 {
     const int e = n / a.agents_per_env, slot = n - e * a.agents_per_env;
@@ -215,7 +213,7 @@ __device__ __forceinline__ void agent_scan_one(const navgym_scan_args_t &a, cons
 // per 128 consecutive agents that lists the masked ones and scans them in turn for the ~1 % masked
 // launches: an environment's agents are consecutive, so its ten scans ran one after the other in one
 // CTA and the crowd step lost 0.23 ms; the full grid costs 25-44 us.)
-__global__ void __launch_bounds__(128, NAVGYM_AGENT_MIN_CTAS) agent_scan_kernel(const navgym_scan_args_t a)
+__global__ void __launch_bounds__(128, AGENT_MIN_CTAS) agent_scan_kernel(const navgym_scan_args_t a)
 {
     __shared__ float4 near_segs[NAVGYM_SCAN_SEGS];
     __shared__ int4 near_win[NAVGYM_SCAN_SEGS];

@@ -11,6 +11,9 @@ __device__ unsigned long long g_prof[16];
 #define PROF_MARK(i)
 #endif
 
+#define NAVGYM_CTA_THREADS 64  // one CTA of 2 warps = one environment
+#define NAVGYM_CTAS_PER_SM 16  // resident CTAs the register budget is tuned for (64 registers)
+
 struct EnvSmem {
     int scan[NB];          // float bits of the ranges [m] (non-negative floats order like ints)
     float2 dir[NB];        // beam directions (cos, sin) of the current pass
@@ -21,7 +24,7 @@ struct EnvSmem {
     double th_spec, yaw_spec;  // heading warp 1 assumed for the final pose, and its yaw
     int map, steps, episode, next_pass;
     int n_vis_seg, n_vis_disc;  // visible box segments / discs listed by the obstacle phase
-    short alive[NB];       // beams still marching after the head phase: one list per warp, NB / WPE entries each
+    short alive[NB];       // beams still marching after the head phase: one list per warp, NB / 2 entries each
     float noise_std;
     // per-pass scan setup
     float lx, ly, lt, res32, max_range, t_stop;
@@ -30,46 +33,27 @@ struct EnvSmem {
 #ifdef NAVGYM_PROFILE
     int prof_iters_a[8], prof_rounds_b[8], prof_alive, prof_cyc_b[8], prof_walk[8];   // per warp: tail iterations / cooperative rounds
 #endif
-#ifdef NAVGYM_SMEM_WINDOW
-    // A/B build (profiles/r2_smem_window_ab.txt): the (2R)^2 EDT cells around the origin cell staged
-    // in shared memory; samples inside the window read it instead of L2
-    float win[4 * NAVGYM_SMEM_WINDOW * NAVGYM_SMEM_WINDOW];
-    int wx0, wy0;
-#endif
 };
 
-// EDT value of an in-map cell: from the staged window when it covers the cell (A/B build),
-// else through the read-only L1/L2 path.
-__device__ __forceinline__ float edt_at(const EnvSmem &sm, const float *__restrict__ dist, int cx, int cy, int W, bool valid)
+// EDT value of an in-map cell through the read-only L1/L2 path (element 0 when !valid).  Kept a
+// function: the same load written out at the three call sites compiles to a different schedule.
+__device__ __forceinline__ float edt_at(const float *__restrict__ dist, int cx, int cy, int W, bool valid)
 {
-#ifdef NAVGYM_SMEM_WINDOW
-    const unsigned ux = (unsigned)(cx - sm.wx0), uy = (unsigned)(cy - sm.wy0);
-    const bool inw = valid & (ux < 2u * NAVGYM_SMEM_WINDOW) & (uy < 2u * NAVGYM_SMEM_WINDOW);
-    float d = 0.0f;
-    if (inw) d = sm.win[uy * (2 * NAVGYM_SMEM_WINDOW) + ux];
-    else d = __ldg(dist + (valid ? (unsigned)(cy * W + cx) : 0u));
-    return d;
-#else
     return __ldg(dist + (valid ? (unsigned)(cy * W + cx) : 0u));
-#endif
 }
 
-#if !defined(NAVGYM_PROFILE) && !defined(NAVGYM_SMEM_WINDOW)
+#ifndef NAVGYM_PROFILE
 // 16 resident CTAs x (sizeof(EnvSmem) + 1 KB the system reserves per CTA) must fit the 132 KB
 // shared-memory configuration: 64 bytes more and the driver picks the 164 KB one, taking 32 KB
 // from the L1 the EDT gathers go through.
 static_assert(sizeof(EnvSmem) <= 132 * 1024 / 16 - 1024, "EnvSmem outgrew the 132 KB carve-out at 16 CTAs/SM");
 #endif
 enum { PASS_STEP = 0, PASS_RESCAN = 1, PASS_RESET = 2, PASS_END = 3 };
-#ifndef NAVGYM_HEAD_STEPS
-#define NAVGYM_HEAD_STEPS 4  // samples every beam marches in the lockstep head phase
-#endif
-#ifndef NAVGYM_HEAD_STEPS_LARGE
+constexpr int HEAD_STEPS = 4;  // samples every beam marches in the lockstep head phase
 // ... in launches too large for tail regime B (COOP = false): throughput-bound, where two more
 // lockstep samples (four gathers in flight per thread) beat the tail's one per lane
 // (32 768 envs: 0.478 -> 0.468 ms; at 4096 envs the length makes no difference)
-#define NAVGYM_HEAD_STEPS_LARGE 6
-#endif
+constexpr int HEAD_STEPS_LARGE = 6;
 
 // Angular window of beams that can see an obstacle spanning bearings [phi0, phi0 + width].
 // Beam k looks along lin[k] + theta with lin[k] = ANGLE_MIN + k * step (env.py:388-390).
@@ -130,23 +114,12 @@ __device__ __forceinline__ void pass_setup(EnvSmem &sm, const navgym_map_t &m, c
     sm.t_stop = fminf(fminf(a.t_stop, sm.max_range), 8.0e6f);
 }
 
-template <int WPE>
-__device__ __forceinline__ void cta_sync()
-{
-    if (WPE > 1) __syncthreads(); else __syncwarp();
-}
-template <int WPE>
-__device__ __forceinline__ int cta_or(int pred)
-{
-    return WPE > 1 ? __syncthreads_or(pred) : __any_sync(0xffffffffu, pred);
-}
-
 // Tail phase.  Two regimes:
 //  A  dealing: every warp has its own list of the beams it marched through the head phase and
 //     that are still alive; the entries are dealt to its lanes with ballot ranks (no atomics, no
 //     cross-warp traffic): a lane whose beam ends takes the warp's next undealt entry; one beam
 //     per lane, one EDT gather per lane and round trip.
-//  B  cooperative: once the warp's entries are all dealt and at most NAVGYM_COOP_ENTER beams are
+//  B  cooperative: once the warp's entries are all dealt and at most COOP_ENTER beams are
 //     still marching, the idle lanes stop idling: the L live beams are regrouped onto G = 32 / L
 //     (power of two) lanes each, and lane j of a group fetches the cell the beam would sample
 //     at t + j -- a guess at where the march goes next (along a wall the step is max(0.999 d, 1)
@@ -158,18 +131,14 @@ __device__ __forceinline__ int cta_or(int pred)
 //     the beam at least as far as regime A would -- and the dependent-gather chain of a scan's
 //     longest beams (max 226 samples on the bench world, one L2 round trip each) shrinks 3-5x
 //     (oracle/analysis/coop_march.py).  The sequence of t values and hit cells is bit-identical.
-#ifndef NAVGYM_COOP_ENTER
-#define NAVGYM_COOP_ENTER 1
-#endif
-#ifndef NAVGYM_COOP_LOG2_WIDTH
-#define NAVGYM_COOP_LOG2_WIDTH 5   // at most 2^5 lanes fetch ahead for one beam
-#endif
-template <int WPE, bool COOP>
+constexpr int COOP_ENTER = 1;
+constexpr int COOP_LOG2_WIDTH = 5;   // at most 2^5 lanes fetch ahead for one beam
+template <bool COOP>
 __device__ __forceinline__ void march_tail_dealt(EnvSmem &sm, const float *__restrict__ dist, float x0, float y0,
                                                  int W, int H, float t_stop, int n_alive, int warp, int lane)
 {
     // every warp deals from its own survivor list
-    const short *list = sm.alive + warp * (NB / WPE);
+    const short *list = sm.alive + warp * (NB / 2);
     const unsigned FULL = 0xffffffffu;
     int next_j = 32;                       // warp-uniform: entries dealt so far
     int idx = lane;
@@ -181,13 +150,12 @@ __device__ __forceinline__ void march_tail_dealt(EnvSmem &sm, const float *__res
     // ---- regime A.  The warp's dealing state (next_j, live) and with it the switch to regime B
     // only change in an iteration in which some beam ended: all of that sits behind one
     // warp-uniform test of the ballot.
-    constexpr int coop_enter = NAVGYM_COOP_ENTER;
-    bool to_b = COOP && NAVGYM_COOP_ENTER != 0 && !(next_j < n_alive) && __popc(live) <= coop_enter;
+    bool to_b = COOP && !(next_j < n_alive) && __popc(live) <= COOP_ENTER;
     while (!to_b) {
         const int cx = __float2int_rz(march_pos(dd.x, t, x0));
         const int cy = __float2int_rz(march_pos(dd.y, t, y0));
         const bool inb = ((unsigned)cx < (unsigned)W) & ((unsigned)cy < (unsigned)H);
-        const float d = edt_at(sm, dist, cx, cy, W, inb & (kb >= 0));
+        const float d = edt_at(dist, cx, cy, W, inb & (kb >= 0));
         const bool hit = inb & (d <= 0.0f);
         t = __fadd_rn(t, fmaxf(__fmul_rn(d, 0.999f), 1.0f));
         const bool fin = (kb >= 0) & (!inb | hit | !(t < t_stop));
@@ -210,7 +178,7 @@ __device__ __forceinline__ void march_tail_dealt(EnvSmem &sm, const float *__res
             next_j += __popc(fm);
             live = __ballot_sync(FULL, kb >= 0);
             if (!live) return;
-            to_b = COOP && NAVGYM_COOP_ENTER != 0 && !(next_j < n_alive) && __popc(live) <= coop_enter;
+            to_b = COOP && !(next_j < n_alive) && __popc(live) <= COOP_ENTER;
         }
     }
     // ---- regime B: `live` marks the lanes that hold a marching beam (kb, t, dd)
@@ -218,8 +186,8 @@ __device__ __forceinline__ void march_tail_dealt(EnvSmem &sm, const float *__res
     const long long prof_b0 = clock64();
 #endif
     while (live) {
-        const int L = __popc(live);        // <= NAVGYM_COOP_ENTER <= 16
-        const int lg = min(L > 8 ? 1 : L > 4 ? 2 : L > 2 ? 3 : L > 1 ? 4 : 5, NAVGYM_COOP_LOG2_WIDTH);   // G = 32 / L, a power of two
+        const int L = __popc(live);        // <= COOP_ENTER
+        const int lg = min(L > 8 ? 1 : L > 4 ? 2 : L > 2 ? 3 : L > 1 ? 4 : 5, COOP_LOG2_WIDTH);   // G = 32 / L, a power of two
         const int G = 1 << lg;             // lanes per beam
         const int g = lane >> lg, j = lane & (G - 1), base = lane & ~(G - 1);
         const bool act = g < L;
@@ -237,7 +205,7 @@ __device__ __forceinline__ void march_tail_dealt(EnvSmem &sm, const float *__res
             const int fy = __float2int_rz(march_pos(bdy, tj, y0));
             const bool finb = ((unsigned)fx < (unsigned)W) & ((unsigned)fy < (unsigned)H);
             const int fcell = finb ? (fy << 16 | fx) : -2;
-            const float fd = edt_at(sm, dist, fx, fy, W, finb & !fin);
+            const float fd = edt_at(dist, fx, fy, W, finb & !fin);
             // walk the true march through the fetched cells
             const float t0 = bt;
             bool walking = !fin;
@@ -288,12 +256,11 @@ __device__ __forceinline__ void march_tail_dealt(EnvSmem &sm, const float *__res
 // (round r = this thread's beams BEAM(4 r .. 4 r + 3)): beam directions, lockstep head phase,
 // survivor list, tail phase.  Leaves every beam's hit cell, (y << 16 | x) or -1, in sm.scan and
 // its direction in sm.dir; ends on a CTA barrier.  Scan set-up is read from sm (pass_setup).
-template <int WPE, bool COOP>
+template <bool COOP>
 __device__ __forceinline__ void march_scan(EnvSmem &sm, const navgym_step_args_t &a, const int r_begin, const int r_end,
                                            const int tid)
 {
-    constexpr int BPL = NB / (32 * WPE);
-    constexpr int TPB = WPE * 32;
+    constexpr int TPB = NAVGYM_CTA_THREADS;
     const unsigned FULL = 0xffffffffu;
     const int lane = tid & 31, warp = tid >> 5;
 #define BEAM(i) (tid + TPB * (i))
@@ -309,22 +276,7 @@ __device__ __forceinline__ void march_scan(EnvSmem &sm, const navgym_step_args_t
     const float d0 = o_in ? __ldg(dist + cj * W + ci) : 1.0f;
     const float t1 = fmaxf(__fmul_rn(d0, 0.999f), 1.0f);  // == 0.0f + first step
     const bool degenerate = !o_in | (d0 <= 0.0f) | !(t1 < t_stop);
-    constexpr int HB = BPL >= 4 ? 4 : BPL;   // beams in flight per thread in the head phase
-#ifdef NAVGYM_SMEM_WINDOW
-    {   // stage the window: rows of 2R cells, coalesced; cells outside the map are never read
-        constexpr int R2 = 2 * NAVGYM_SMEM_WINDOW;
-        const int wx0 = ci - NAVGYM_SMEM_WINDOW, wy0 = cj - NAVGYM_SMEM_WINDOW;
-        if (tid == 0) { sm.wx0 = wx0; sm.wy0 = wy0; }
-        if (!degenerate) {
-            for (int i = tid; i < R2 * R2; i += TPB) {
-                const int x = wx0 + (i % R2), y = wy0 + (i / R2);
-                const bool ok = ((unsigned)x < (unsigned)W) & ((unsigned)y < (unsigned)H);
-                sm.win[i] = ok ? __ldg(dist + (unsigned)(y * W + x)) : 0.0f;
-            }
-        }
-        cta_sync<WPE>();
-    }
-#endif
+    constexpr int HB = 4;   // beams in flight per thread in the head phase
     int n_mine = 0;   // warp-uniform: survivors in this warp's list
 #pragma unroll 1
     for (int r = r_begin; r < r_end; r++) {
@@ -348,7 +300,7 @@ __device__ __forceinline__ void march_scan(EnvSmem &sm, const navgym_step_args_t
         // was still alive (one compare instead of a predicate carried through the whole step:
         // 99 instead of 119 instructions per four samples).
 #pragma unroll 1
-        for (int st = 0; st < (COOP ? NAVGYM_HEAD_STEPS : NAVGYM_HEAD_STEPS_LARGE); st++) {
+        for (int st = 0; st < (COOP ? HEAD_STEPS : HEAD_STEPS_LARGE); st++) {
             float dv[HB];
             int cx[HB], cy[HB];
             bool inb[HB];
@@ -357,7 +309,7 @@ __device__ __forceinline__ void march_scan(EnvSmem &sm, const navgym_step_args_t
                 cx[j] = __float2int_rz(march_pos(dxh[j], th_[j], x0));
                 cy[j] = __float2int_rz(march_pos(dyh[j], th_[j], y0));
                 inb[j] = ((unsigned)cx[j] < (unsigned)W) & ((unsigned)cy[j] < (unsigned)H);
-                dv[j] = edt_at(sm, dist, cx[j], cy[j], W, inb[j]);
+                dv[j] = edt_at(dist, cx[j], cy[j], W, inb[j]);
             }
 #pragma unroll
             for (int j = 0; j < HB; j++) {
@@ -375,7 +327,7 @@ __device__ __forceinline__ void march_scan(EnvSmem &sm, const navgym_step_args_t
             const bool alive = th_[j] == th_[j];
             if (alive) sm.scan[k] = __float_as_int(th_[j]);
             const unsigned mk = __ballot_sync(FULL, alive);
-            if (alive) sm.alive[warp * (NB / WPE) + n_mine + __popc(mk & ((1u << lane) - 1u))] = (short)k;
+            if (alive) sm.alive[warp * (NB / 2) + n_mine + __popc(mk & ((1u << lane) - 1u))] = (short)k;
             n_mine += __popc(mk);
         }
     }
@@ -388,27 +340,21 @@ __device__ __forceinline__ void march_scan(EnvSmem &sm, const navgym_step_args_t
 #ifdef NAVGYM_PROFILE
         if (tid == 0) sm.prof_alive += n_alive;
 #endif
-        march_tail_dealt<WPE, COOP>(sm, dist, x0, y0, W, H, t_stop, n_alive, warp, lane);
+        march_tail_dealt<COOP>(sm, dist, x0, y0, W, H, t_stop, n_alive, warp, lane);
     }
-    cta_sync<WPE>();
+    __syncthreads();
 #undef BEAM
 }
 
-// One CTA of WPE warps = one environment.  Thread t of the CTA owns beams t + 32 WPE i, i = 0 ..
-// 16 / WPE - 1: the lanes of a warp work on neighbouring beams, whose EDT gathers share sectors.
+// One CTA of 2 warps = one environment.  Thread t of the CTA owns beams t + 64 i, i = 0 .. 7:
+// the lanes of a warp work on neighbouring beams, whose EDT gathers share sectors.
 // A scan marches in two phases (see the march section below): a lockstep head phase, four
 // samples per beam with four beams per thread in flight, then a tail phase in which the beams
 // still alive are dealt to lanes as lanes fall free (ballot-rank dealing, one beam per lane at a
 // time; the last beam of a warp is marched by all its lanes together).  The three scans a step
 // may need (the step's scan, the crash re-scan env.py:718, the auto-reset first scan) run
 // through ONE copy of the scan code inside a CTA-uniform pass loop.
-#ifndef NAVGYM_RISK_MARGIN
-#define NAVGYM_RISK_MARGIN 0.25f  // [m] clearance under which the next step may end the episode
-#endif
-#define NAVGYM_CTA_THREADS 64
-#ifndef NAVGYM_CTAS_PER_SM
-#define NAVGYM_CTAS_PER_SM 16  // resident CTAs the register budget is tuned for (64 registers)
-#endif
+constexpr float RISK_MARGIN = 0.25f;  // [m] clearance under which the next step may end the episode
 // What one CTA of the fused kernel does to its environment:
 //   MODE_STEP          one step (navgym_step_batch), auto-reset included;
 //   MODE_RESET         the first observation of an episode from the pose in `state`
@@ -417,14 +363,14 @@ __device__ __forceinline__ void march_scan(EnvSmem &sm, const navgym_step_args_t
 //                      first observation as the auto-reset pass writes it (navgym_reset_envs):
 //                      no hits recorded, no launch-order filing.
 enum { MODE_STEP = 0, MODE_RESET = 1, MODE_MASKED_RESET = 2 };
-template <int MODE, int WPE, bool COOP, int FMT>
+template <int MODE, bool COOP, int FMT>
 __device__ __forceinline__ void step_body(const navgym_step_args_t &a, EnvSmem &sm, const int e, const int tid,
                                           int *sched_cnt, int *sched_list)
 {
     constexpr bool IS_RESET_KERNEL = MODE != MODE_STEP;   // both reset modes: no action, a new episode
     constexpr bool MASKED = MODE == MODE_MASKED_RESET;
-    constexpr int BPL = NB / (32 * WPE);  // beams per lane
-    constexpr int TPB = WPE * 32;         // threads of the CTA
+    constexpr int TPB = NAVGYM_CTA_THREADS;  // threads of the CTA
+    constexpr int BPL = NB / TPB;            // beams per lane
     const int lane = tid & 31, warp = tid >> 5;
     const int B = a.num_envs;
     const long long t_begin = clock64();
@@ -444,7 +390,7 @@ __device__ __forceinline__ void step_body(const navgym_step_args_t &a, EnvSmem &
     // float64 kinematics.  Warp 1 meanwhile evaluates the yaw the epilogue will need (the same
     // heading arithmetic as warp 0): for every environment that neither rolls back nor resets,
     // the float64 sincos + atan2 of the final heading leave the critical path.
-    if (WPE > 1 && warp == 1) {
+    if (warp == 1) {
         double th = ST(NAVGYM_S_TH);
         if (!IS_RESET_KERNEL) {
             double th1;
@@ -526,7 +472,6 @@ __device__ __forceinline__ void step_body(const navgym_step_args_t &a, EnvSmem &
             sm.noise_std = noise_std0;
             if (IS_RESET_KERNEL) { sm.ppx = px; sm.ppy = py; sm.pyaw = 0; sm.pv = 0; sm.pw = 0; }
             if (MASKED) { sm.gx = gx; sm.gy = gy; }
-            if (WPE == 1) sm.th_spec = CUDART_NAN;
             pass_setup(sm, m0, a);  // first pass: the map descriptor is already here
         }
     }
@@ -543,11 +488,11 @@ __device__ __forceinline__ void step_body(const navgym_step_args_t &a, EnvSmem &
     float margin = CUDART_INF_F; // its smallest clearance over the crash thresholds [m]
     for (bool first = true;; first = false) {
         // ---- per-pass setup; the first pass was set up by the prologue
-        cta_sync<WPE>();
+        __syncthreads();
         if (!first) {
             t_pass = clock64();
             if (tid == 0) pass_setup(sm, a.maps[sm.map], a);
-            cta_sync<WPE>();
+            __syncthreads();
         }
         margin = CUDART_INF_F;
         PROF_MARK(0);
@@ -557,7 +502,7 @@ __device__ __forceinline__ void step_body(const navgym_step_args_t &a, EnvSmem &
         // Every beam of a scan starts on the origin cell, so that first sample (t = 0) is taken
         // once per environment: either the origin is occupied (all beams end there) or all
         // beams advance by the same first step.  The march then runs in two phases:
-        //  head: every thread marches its own beams NAVGYM_HEAD_STEPS samples, HB beams at a
+        //  head: every thread marches its own beams HEAD_STEPS samples, HB beams at a
         //        time in lockstep — almost every beam is still alive that early, and the HB
         //        independent EDT gathers per thread hide the L2 latency by ILP;
         //  tail: the surviving beams are compacted into a list and dealt out dynamically (a
@@ -566,7 +511,7 @@ __device__ __forceinline__ void step_body(const navgym_step_args_t &a, EnvSmem &
         // The loops only find each beam's hit cell (packed into sm.scan); ranges are computed
         // afterwards with all lanes active.
         {
-            march_scan<WPE, COOP>(sm, a, 0, BPL / 4, tid);
+            march_scan<COOP>(sm, a, 0, BPL / 4, tid);
             const int ci = sm.ci, cj = sm.cj;
             // ranges (env.py:426), all lanes active: sqrt(di^2 + dj^2) * resolution
             const bool rec = !MASKED && pass == (IS_RESET_KERNEL ? PASS_RESET : PASS_STEP) && a.hits;
@@ -598,7 +543,7 @@ __device__ __forceinline__ void step_body(const navgym_step_args_t &a, EnvSmem &
         // trip per obstacle and computed every window 32 times over.)
         if (ns + nd > 0) {
             if (tid == 0) { sm.n_vis_seg = 0; sm.n_vis_disc = 0; }
-            cta_sync<WPE>();
+            __syncthreads();
             // (the first scan after an auto-reset or of a masked reset sees the next episode's pedestrians, if given)
             const bool nxt = MODE != MODE_RESET && pass == PASS_RESET && a.discs_reset != nullptr;
             const float *discs = (nxt ? a.discs_reset : a.discs) + (size_t)e * a.max_disc * 3;
@@ -658,7 +603,7 @@ __device__ __forceinline__ void step_body(const navgym_step_args_t &a, EnvSmem &
                     else vis[NB / 2 - 1 - (bd + __popc(md_ & below))] = word;
                 }
             }
-            cta_sync<WPE>();
+            __syncthreads();
             // hits: 16 lanes per visible obstacle across the beams of its window (a window is typically
             // a dozen beams wide), segments first, then discs
             {
@@ -688,7 +633,7 @@ __device__ __forceinline__ void step_body(const navgym_step_args_t &a, EnvSmem &
                     }
                 }
             }
-            cta_sync<WPE>();
+            __syncthreads();
         }
         PROF_MARK(4);
         // ---- clip + noise (env.py:435-440), thresholds, observation row
@@ -698,7 +643,7 @@ __device__ __forceinline__ void step_body(const navgym_step_args_t &a, EnvSmem &
             const float noise_std = sm.noise_std;
             const int steps = sm.steps, episode = sm.episode;
             const int SS = a.num_scan_stack > 1 ? a.num_scan_stack : 1;
-            constexpr int G = BPL >= 4 ? 4 : BPL;
+            constexpr int G = 4;
             // Production noise: one Philox4x32-10 call + two Box-Muller pairs per group of four
             // CONSECUTIVE beams 4q .. 4q + 3, keyed (seed; global env, episode, step, scan slot,
             // q) -- a function of the beam index alone, whatever the launch shape.  The unit
@@ -712,7 +657,7 @@ __device__ __forceinline__ void step_body(const navgym_step_args_t &a, EnvSmem &
                             (uint32_t)pass, (uint32_t)q, z);
                     *reinterpret_cast<float4 *>(zs + 4 * q) = make_float4(z[0], z[1], z[2], z[3]);
                 }
-                cta_sync<WPE>();
+                __syncthreads();
             }
 #pragma unroll 1
             for (int g = 0; g < BPL / G; g++) {
@@ -750,8 +695,8 @@ __device__ __forceinline__ void step_body(const navgym_step_args_t &a, EnvSmem &
         if (pass == PASS_STEP) {
             // ---- reward / done / info on this observation (env.py:464-589)
             int crash, discomf;
-            crash = cta_or<WPE>(c_any);
-            discomf = cta_or<WPE>(d_any) && !crash;
+            crash = __syncthreads_or(c_any);
+            discomf = __syncthreads_or(d_any) && !crash;
             double mn = CUDART_INF;
             if (discomf) {
                 for (int i = 0; i < BPL; i++) {
@@ -762,14 +707,11 @@ __device__ __forceinline__ void step_body(const navgym_step_args_t &a, EnvSmem &
                 }
 #pragma unroll
                 for (int o = 16; o > 0; o >>= 1) mn = fmin(mn, __shfl_xor_sync(FULL, mn, o));
-                if (WPE > 1) {
-                    if (lane == 0) sm.red[warp] = mn;
-                    cta_sync<WPE>();
-                }
+                if (lane == 0) sm.red[warp] = mn;
+                __syncthreads();
             }
             if (warp == 0) {
-                if (WPE > 1 && discomf)
-                    for (int i = 0; i < WPE; i++) mn = fmin(mn, sm.red[i]);
+                if (discomf) mn = fmin(fmin(mn, sm.red[0]), sm.red[1]);
                 // lanes 0 / 1: distance to goal from pose / prev_pose
                 const double gx = sm.gx, gy = sm.gy;
                 const double qx = lane == 0 ? sm.px : sm.ppx, qy = lane == 0 ? sm.py : sm.ppy;
@@ -823,7 +765,7 @@ __device__ __forceinline__ void step_body(const navgym_step_args_t &a, EnvSmem &
                     sm.next_pass = next;
                 }
             }
-            cta_sync<WPE>();
+            __syncthreads();
             pass = sm.next_pass;
             if (pass == PASS_RESET && a.discs_reset != nullptr) {
                 nd = min(a.ndisc_reset[e], a.max_disc);
@@ -844,13 +786,13 @@ __device__ __forceinline__ void step_body(const navgym_step_args_t &a, EnvSmem &
     // overlaps the epilogue.
     int sched_pos = 0, sched_b = 0;
     if (sched_cnt) {
-        bool risky = margin < NAVGYM_RISK_MARGIN;
+        bool risky = margin < RISK_MARGIN;
         if (tid == 0) {
             const double gx = sm.gx - sm.px, gy = sm.gy - sm.py;
-            risky |= gx * gx + gy * gy < (a.dist_thresh + NAVGYM_RISK_MARGIN) * (a.dist_thresh + NAVGYM_RISK_MARGIN);
+            risky |= gx * gx + gy * gy < (a.dist_thresh + RISK_MARGIN) * (a.dist_thresh + RISK_MARGIN);
             risky |= a.max_episode_steps > 0 && sm.steps + 1 >= a.max_episode_steps;
         }
-        risky = cta_or<WPE>(risky) && a.auto_reset;
+        risky = __syncthreads_or(risky) && a.auto_reset;
         if (tid == 0) {
             const long long kc = ((clock64() - t_pass) << (risky ? 1 : 0)) >> 13;
             sched_b = NAVGYM_SCHED_BUCKETS - 1 - (int)(kc > NAVGYM_SCHED_BUCKETS - 1 ? NAVGYM_SCHED_BUCKETS - 1 : kc);
@@ -860,7 +802,7 @@ __device__ __forceinline__ void step_body(const navgym_step_args_t &a, EnvSmem &
     // ---------------- epilogue (warp 0): observation tail + state (env.py:455, 725-727) ---
     if (warp == 0) {
         double yaw;
-        if (WPE > 1 && sm.th_spec == sm.th) {
+        if (sm.th_spec == sm.th) {
             yaw = sm.yaw_spec;  // warp 1 had the final heading right
         } else {
             double sn, cn;
@@ -959,11 +901,10 @@ __global__ void __launch_bounds__(NAVGYM_CTA_THREADS, NAVGYM_CTAS_PER_SM) step_k
 {
     static_assert(MODE == MODE_STEP || MODE == MODE_RESET, "the masked reset is reset_envs_kernel");
     __shared__ EnvSmem sm;
-    constexpr int WPE = NAVGYM_CTA_THREADS / 32;
     int e = a.env_begin + (int)blockIdx.x;
     int *sched_cnt = nullptr, *sched_list = nullptr;
     if (MODE == MODE_STEP && a.sched) e = sched_lookup(a, (int)blockIdx.x, sched_cnt, sched_list);
-    step_body<MODE, WPE, COOP, FMT>(a, sm, e, (int)threadIdx.x, sched_cnt, sched_list);
+    step_body<MODE, COOP, FMT>(a, sm, e, (int)threadIdx.x, sched_cnt, sched_list);
 }
 
 // The masked reset (navgym_reset_envs): CTA b takes environment env_begin + b in index order and
@@ -973,8 +914,7 @@ __global__ void __launch_bounds__(NAVGYM_CTA_THREADS, NAVGYM_CTAS_PER_SM)
 reset_envs_kernel(const navgym_step_args_t a, const uint8_t *__restrict__ mask)
 {
     __shared__ EnvSmem sm;
-    constexpr int WPE = NAVGYM_CTA_THREADS / 32;
     const int e = a.env_begin + (int)blockIdx.x;
     if (!mask[e]) return;
-    step_body<MODE_MASKED_RESET, WPE, COOP, FMT>(a, sm, e, (int)threadIdx.x, nullptr, nullptr);
+    step_body<MODE_MASKED_RESET, COOP, FMT>(a, sm, e, (int)threadIdx.x, nullptr, nullptr);
 }

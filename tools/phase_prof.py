@@ -1,6 +1,6 @@
 """Per-phase cycle accounting of the fused step kernel (debug build with -DNAVGYM_PROFILE).
 Build here:   python tools/phase_prof.py build
-Run on GPU:   NAVGYM_LIB=tools/_prof/libnavgym_b200_prof.so python tools/phase_prof.py run"""
+Run on GPU:   python tools/phase_prof.py run"""
 import ctypes as C, os, subprocess, sys
 ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
 sys.path.insert(0, ROOT)
@@ -8,15 +8,15 @@ OUT = os.path.join(ROOT, 'tools', '_prof', 'libnavgym_b200_prof.so')
 if sys.argv[1] == 'build':
     from nav_gym_b200 import _lib
     os.makedirs(os.path.dirname(OUT), exist_ok=True)
-    for tag, extra in (('', []), ('_nocoop', ['-DNAVGYM_COOP_ENTER=0']), ('_e1', ['-DNAVGYM_COOP_ENTER=1']), ('_e2', ['-DNAVGYM_COOP_ENTER=2'])):
-        out = OUT.replace('.so', tag + '.so')
-        r = subprocess.run(['nvcc'] + _lib.NVCC_FLAGS + ['-DNAVGYM_PROFILE', '-Xptxas', '-v'] + extra + ['-o', out, _lib.SRC], capture_output=True, text=True)
-        lines = r.stderr.splitlines()
-        for i, l in enumerate(lines):
-            if 'step_kernelILb0ELi2ELi1' in l: print(tag, lines[i+1].strip(), lines[i+2].strip())
-        print('built', out)
+    r = subprocess.run([_lib._nvcc()] + _lib.NVCC_FLAGS + ['-DNAVGYM_PROFILE', '-Xptxas', '-v', '-o', OUT, _lib.SRC], capture_output=True, text=True)
+    if r.returncode:
+        sys.exit(r.stderr)
+    lines = r.stderr.splitlines()
+    for i, l in enumerate(lines):   # step_kernel<MODE_STEP, COOP, FMT>: stack / spills, registers / smem
+        if 'Function properties for _Z11step_kernelILi0E' in l: print(l.split()[-1] + ':', lines[i+1].strip() + ';', lines[i+2].split(':', 1)[1].strip())
+    print('built', OUT)
 else:
-    os.environ['NAVGYM_LIB'] = OUT.replace('.so', os.environ.get('NAVGYM_VARIANT', '') + '.so')
+    os.environ['NAVGYM_LIB'] = OUT
     import numpy as np, torch
     from nav_gym_b200 import _lib
     from nav_gym_b200.batched_env import BatchedNavGym, MapPool, filter_spawn_pool
