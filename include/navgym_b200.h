@@ -147,6 +147,15 @@ typedef struct {
     int32_t _pad;
 } navgym_step_args_t;
 
+/* navgym_step_batch, navgym_reset_obs_batch, navgym_reset_envs and navgym_export_env return
+ * cudaErrorInvalidValue, and launch nothing, for an argument block with
+ *   - obs rows that NAVGYM_OBS_F32 / NAVGYM_OBS_F16 above do not allow (format, stride, alignment);
+ *   - env_begin < 0, env_begin > num_envs, env_count < 0 or env_begin + env_count > num_envs;
+ *   - max_disc + max_seg > 256 counting the obstacle buffers given (discs, segs; for
+ *     navgym_reset_envs also discs_reset, segs_reset on their own).
+ * The three launchers return 0 without launching when num_envs <= 0 or when the range is empty
+ * (env_begin == num_envs). */
+
 /* ---- fused hot path: NavGymEnv.step (env.py:591-728) over num_envs environments ------ */
 int navgym_step_batch(const navgym_step_args_t *args, void *stream);
 /* The same step for a caller whose buffers live on the HOST (the reference's own calling
@@ -175,6 +184,7 @@ int navgym_step_batch_host_submit(navgym_host_pipe_t *pipe, const navgym_step_ar
                                   const float *actions_host, float *obs_host, float *reward_host,
                                   uint8_t *done_host);
 int navgym_step_batch_host_wait(navgym_host_pipe_t *pipe, int group);
+/* the pipe's number of groups, and group g's env range [begin, end) */
 int navgym_host_pipe_groups(const navgym_host_pipe_t *pipe);
 int navgym_host_pipe_group_bounds(const navgym_host_pipe_t *pipe, int group, int *begin, int *end);
 /* The whole host-side rollout loop in C (the reference's `while True: obs, r, d, info =
@@ -226,8 +236,7 @@ int navgym_reset_obs_batch(const navgym_step_args_t *args, void *stream);
  * buffer above holds what the step with auto_reset = 1 would have left, bit for bit (pools with
  * spawn rows).  Each draw depends only on the environment's own episodes[e], so the result does
  * not depend on how the masked set is split across calls or env_offset shards.
- * cudaErrorInvalidValue: mask == NULL, obs rows as navgym_step_batch rejects them, or an env range
- * outside [0, num_envs).  num_envs <= 0 is a no-op. */
+ * cudaErrorInvalidValue: mask == NULL, or an argument block rejected as above. */
 int navgym_reset_envs(const navgym_step_args_t *args, const uint8_t *mask, void *stream);
 
 /* ---- host export of one environment (ros_env.py:69-176 reads a NavGymEnv's attributes; the
@@ -412,23 +421,15 @@ int navgym_sizeof_move_args(void);
 int navgym_sizeof_plan_args(void);
 int navgym_sizeof_plan_map(void);
 
-/* ---- pedestrian policy, convolutional front end (human_policy.py:24-25, 45-47 fed as in
- * env.py:627-629, 647): scan[n][512] (metres) -> clip to [0, 6], / 6 - 0.5 (float64, then
- * float32) -> conv1d(1 -> 32, k 5, stride 2, pad 1; env.py:647 feeds the same scan to the
- * three input frames, so w1 is the reference's act_fea_cv1 weight summed over them) -> relu ->
- * conv1d(32 -> 32, k 3, stride 2, pad 1) -> relu -> features[n][4096], channel-major like
- * `.view(N, -1)`.  One launch, activations stay in shared memory (cuDNN writes and re-reads
- * 2 GB of them for 40 960 pedestrians).  w1 [32][5], b1 [32], w2 [32][32][3] (out, in, tap),
- * b2 [32]: float32 device pointers in torch's layout. */
-int navgym_policy_features(const float *scan, int n, const float *w1, const float *b1,
-                           const float *w2, const float *b2, float *features, void *stream);
-
-/* ---- the whole pedestrian policy, natively: HumanPolicy's deterministic action mean
+/* ---- the pedestrian policy, natively: HumanPolicy's deterministic action mean
  * (human_policy.py:38-55, the only output env.py:649-656 uses) for n pedestrians,
  *   mean = (sigmoid(actor1(a)), tanh(actor2(a))),  a = relu(act_fc2([relu(act_fc1(feat)), goal, speed])),
- *   feat = the convolutional front end of navgym_policy_features on the pedestrian's newest scan
- *          (env.py:647 feeds it to all three input frames; the fold is done here from the
- *          reference-shaped act_fea_cv1 weight).
+ *   feat = the convolutional front end (human_policy.py:24-25, 45-47 fed as in env.py:627-629,
+ *          647) on the pedestrian's newest scan[512] (metres): clip to [0, 6], / 6 - 0.5 (float64,
+ *          then float32) -> conv1d(1 -> 32, k 5, stride 2, pad 1) with act_fea_cv1's weight
+ *          summed over its three input frames (env.py:647 feeds the same scan to all three; the
+ *          fold is done here from the reference-shaped weight) -> relu -> conv1d(32 -> 32, k 3,
+ *          stride 2, pad 1) -> relu -> 4096 features, channel-major like `.view(N, -1)`.
  * Three launches, no library GEMM, every contraction on the tcgen05 tensor cores in the "f16x3"
  * scheme (hi/lo f16 splits of both operands, three MMAs per K step: float32-grade results): the
  * front end (features leave as two f16 halves), act_fc1 with TMA-fed operands and TMEM
@@ -484,15 +485,9 @@ int navgym_raymarching_edt_host(const navgym_raymarching_t *rm, float *out_host)
 void navgym_raymarching_destroy(navgym_raymarching_t *rm);
 
 /* ---- inner native boundary: pymap2d ------------------------------------------------ */
-/* render_contours_in_lidar(ranges, angles, flat, lidar_xy) (env.py:430-431) with the
- * polygons already flattened to closed segments segs[S][4]; in-place min. */
-int navgym_render_segments_in_lidar(float *ranges_dev, const float *headings_dev, int K,
-                                    const float *segs_dev, int S, float ox, float oy,
-                                    void *stream);
-/* CMap2D.render_agents_in_lidar (env.py:432) with agents reduced to discs[D][3]. */
-int navgym_render_discs_in_lidar(float *ranges_dev, const float *headings_dev, int K,
-                                 const float *discs_dev, int D, float ox, float oy,
-                                 void *stream);
+/* render_contours_in_lidar(ranges, angles, flat, lidar_xy) (env.py:430-431) with the polygons
+ * already flattened to closed segments segs[S][4], then CMap2D.render_agents_in_lidar
+ * (env.py:432) with agents reduced to discs[D][3]; in-place min into ranges[K]. */
 int navgym_render_in_lidar_host(float *ranges_host, const float *headings_host, int K,
                                 const float *segs_host, int S, const float *discs_host, int D,
                                 float ox, float oy);

@@ -183,13 +183,13 @@ EXPORTS = [
     'navgym_step_batch_host', 'navgym_step_batch_host_submit', 'navgym_step_batch_host_wait', 'navgym_edt_build', 'navgym_calc_range_many',
     'navgym_raymarching_create_host', 'navgym_raymarching_calc_range_many_host',
     'navgym_raymarching_edt_dev', 'navgym_raymarching_edt_host', 'navgym_raymarching_destroy',
-    'navgym_render_segments_in_lidar', 'navgym_render_discs_in_lidar', 'navgym_render_in_lidar_host',
+    'navgym_render_in_lidar_host',
     'navgym_error_string', 'navgym_device_count', 'navgym_abi_version', 'navgym_launch_count',
     'navgym_sizeof_step_args', 'navgym_sizeof_map', 'navgym_grid_bfs',
     'navgym_sizeof_her_args', 'navgym_sizeof_peds_args', 'navgym_compute_rewards', 'navgym_peds_advance',
     'navgym_agent_scan_batch', 'navgym_sizeof_scan_args',
     'navgym_peds_plan', 'navgym_sizeof_plan_args', 'navgym_sizeof_plan_map',
-    'navgym_peds_move', 'navgym_sizeof_move_args', 'navgym_policy_features',
+    'navgym_peds_move', 'navgym_sizeof_move_args',
     'navgym_host_pipe_groups', 'navgym_host_pipe_group_bounds', 'navgym_host_rollout',
     'navgym_policy_action_bank', 'navgym_export_env', 'navgym_export_env_len', 'navgym_march_is_fused',
     'navgym_policy_workspace_bytes', 'navgym_sizeof_policy_params', 'navgym_policy_create',
@@ -235,10 +235,6 @@ def load():
     lib.navgym_raymarching_edt_host.argtypes = [_P, _P]
     lib.navgym_raymarching_destroy.restype = None
     lib.navgym_raymarching_destroy.argtypes = [_P]
-    lib.navgym_render_segments_in_lidar.argtypes = [_P, _P, C.c_int, _P, C.c_int, C.c_float,
-                                                    C.c_float, _P]
-    lib.navgym_render_discs_in_lidar.argtypes = [_P, _P, C.c_int, _P, C.c_int, C.c_float,
-                                                 C.c_float, _P]
     lib.navgym_render_in_lidar_host.argtypes = [_P, _P, C.c_int, _P, C.c_int, _P, C.c_int,
                                                 C.c_float, C.c_float]
     lib.navgym_grid_bfs.restype = None
@@ -251,7 +247,6 @@ def load():
     lib.navgym_agent_scan_batch.argtypes = [C.POINTER(ScanArgs), _P]
     lib.navgym_peds_plan.argtypes = [C.POINTER(PlanArgs), _P]
     lib.navgym_peds_move.argtypes = [C.POINTER(MoveArgs), _P]
-    lib.navgym_policy_features.argtypes = [_P, C.c_int, _P, _P, _P, _P, _P, _P]
     lib.navgym_policy_workspace_bytes.restype = C.c_size_t
     lib.navgym_policy_workspace_bytes.argtypes = [C.c_int]
     lib.navgym_policy_create.restype = _P

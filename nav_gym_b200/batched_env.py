@@ -319,7 +319,12 @@ class BatchedNavGym(object):
         self._host_ptrs = tuple(_ptr(t) for t in self._host_bufs)
         self._args_ref = C.byref(self.args)
         torch.cuda.synchronize(self.device)
-        return [(self.B * g // groups, self.B * (g + 1) // groups) for g in range(groups)]
+        bounds = []
+        for g in range(self.lib.navgym_host_pipe_groups(self._pipe[0])):
+            b0, b1 = C.c_int(), C.c_int()
+            _lib.check(self.lib.navgym_host_pipe_group_bounds(self._pipe[0], g, C.byref(b0), C.byref(b1)), 'group_bounds')
+            bounds.append((b0.value, b1.value))
+        return bounds
 
     def _make_pipe(self, groups, fresh=False):
         """(Re)create the host pipe -- its streams, events and schedule buffers live on the env's

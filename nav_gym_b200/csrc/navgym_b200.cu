@@ -21,8 +21,8 @@
 //   device_helpers.cuh      cell mapping, canonical beam direction / march / segment / disc, Philox
 //   step_kernel.cuh         the fused step: one CTA = one environment, 2 warps, pass loop
 //   her_kernel.cuh          compute_rewards / terminals / info on stored observations
-//   pedestrian_kernels.cuh  pedestrians' lidar, routes, motion, policy front end, geometry
-//   native_kernels.cuh      EDT build, calc_range_many, render_*_in_lidar
+//   pedestrian_kernels.cuh  pedestrians' lidar, routes, motion, geometry
+//   native_kernels.cuh      EDT build, calc_range_many, render_in_lidar
 //   host_pipe.inl           host-buffer entry points (chunked / asynchronous, CUDA-graph replay)
 // and this file holds the C ABI (include/navgym_b200.h) around them.
 #include <cuda_runtime.h>
@@ -52,11 +52,14 @@ static unsigned long long g_launches = 0;
 #include "policy_gemm.cuh"
 
 // ------------------------------------------------------------------ C ABI
-static int coop_default_max()
+// SM count of the current device (a B200's 148 when the query fails).
+static int sm_count()
 {
-    int dev = 0, sms = 148;
-    if (cudaGetDevice(&dev) == cudaSuccess) cudaDeviceGetAttribute(&sms, cudaDevAttrMultiProcessorCount, dev);
-    return (int)(2.4 * sms * NAVGYM_CTAS_PER_SM);
+    int dev = 0, sms = 0;
+    if (cudaGetDevice(&dev) != cudaSuccess ||
+        cudaDeviceGetAttribute(&sms, cudaDevAttrMultiProcessorCount, dev) != cudaSuccess || sms <= 0)
+        return 148;
+    return sms;
 }
 
 // Launch shape of the fused kernel: one 64-thread CTA per environment of the launch.
@@ -72,24 +75,27 @@ static void launch_step_fmt(const navgym_step_args_t &a, const uint8_t *mask, in
     }
 }
 
-// MODE_STEP / MODE_RESET / MODE_MASKED_RESET (step_kernel.cuh) over the launch's env range;
-// `mask` is read by the masked reset only.
+// The obstacle windows of an environment are parked in NB / 2 shared-memory slots.
+static bool obstacle_slots_ok(int max_disc, int max_seg, const void *discs, const void *segs)
+{
+    return (discs ? max_disc : 0) + (segs ? max_seg : 0) <= NB / 2;
+}
+
+// MODE_STEP / MODE_RESET / MODE_MASKED_RESET (step_kernel.cuh) over the launch's env range, which
+// step_args_ok has accepted; `mask` is read by the masked reset only.  An empty range launches
+// nothing.
 template <int MODE>
 static cudaError_t launch_step(const navgym_step_args_t &a, cudaStream_t st, const uint8_t *mask = nullptr)
 {
     const int count = a.env_count > 0 ? a.env_count : a.num_envs - a.env_begin;
-    // the obstacle windows of an environment are parked in NB / 2 shared-memory slots
-    if ((a.discs ? a.max_disc : 0) + (a.segs ? a.max_seg : 0) > NB / 2) return cudaErrorInvalidValue;
-    // (the masked reset may scan the next episode's geometry alone)
-    if (MODE == MODE_MASKED_RESET && (a.discs_reset ? a.max_disc : 0) + (a.segs_reset ? a.max_seg : 0) > NB / 2)
-        return cudaErrorInvalidValue;
+    if (count == 0) return cudaSuccess;
     // tail regime B (see step_kernel) while the launch is at most ~2.4 waves of CTAs (measured
     // crossover on B200: 5120 envs -2 %, 6144 envs +2 %)
-    static const int coop_max = coop_default_max();
+    static const int coop_max = (int)(2.4 * sm_count() * NAVGYM_CTAS_PER_SM);
     if (a.obs_format == NAVGYM_OBS_F16) launch_step_fmt<MODE, NAVGYM_OBS_F16>(a, mask, count, count <= coop_max, st);
     else launch_step_fmt<MODE, NAVGYM_OBS_F32>(a, mask, count, count <= coop_max, st);
     g_launches++;
-    return cudaSuccess;
+    return cudaGetLastError();
 }
 
 // Observation rows (include/navgym_b200.h NAVGYM_OBS_*): a known format, a stride that holds S
@@ -102,6 +108,15 @@ static bool obs_rows_ok(int format, int stride, int num_scan_stack, const void *
     if (format == NAVGYM_OBS_F16)
         return stride % 2 == 0 && stride >= scans + 2 * NAVGYM_OBS_TAIL && ((uintptr_t)obs & 3) == 0;
     return false;
+}
+
+// What every entry point taking a navgym_step_args_t rejects (include/navgym_b200.h): malformed
+// obs rows, an env range outside [0, num_envs), a negative env_count, too many obstacle slots.
+static bool step_args_ok(const navgym_step_args_t *a)
+{
+    return obs_rows_ok(a->obs_format, a->obs_stride, a->num_scan_stack, a->obs) && a->env_begin >= 0 &&
+           a->env_begin <= a->num_envs && a->env_count >= 0 && a->env_count <= a->num_envs - a->env_begin &&
+           obstacle_slots_ok(a->max_disc, a->max_seg, a->discs, a->segs);
 }
 
 #define CK(x) do { cudaError_t _e = (x); if (_e != cudaSuccess) return (int)_e; } while (0)
@@ -142,11 +157,8 @@ int navgym_device_count(void)
 int navgym_step_batch(const navgym_step_args_t *args, void *stream)
 {
     if (args->num_envs <= 0) return 0;
-    if (!obs_rows_ok(args->obs_format, args->obs_stride, args->num_scan_stack, args->obs) || args->env_begin < 0 ||
-        args->env_begin + args->env_count > args->num_envs)
-        return (int)cudaErrorInvalidValue;
-    const cudaError_t err = launch_step<MODE_STEP>(*args, (cudaStream_t)stream);
-    return (int)(err ? err : cudaGetLastError());
+    if (!step_args_ok(args)) return (int)cudaErrorInvalidValue;
+    return (int)launch_step<MODE_STEP>(*args, (cudaStream_t)stream);
 }
 
 #include "host_pipe.inl"
@@ -154,22 +166,17 @@ int navgym_step_batch(const navgym_step_args_t *args, void *stream)
 int navgym_reset_obs_batch(const navgym_step_args_t *args, void *stream)
 {
     if (args->num_envs <= 0) return 0;
-    if (!obs_rows_ok(args->obs_format, args->obs_stride, args->num_scan_stack, args->obs))
-        return (int)cudaErrorInvalidValue;
-    const cudaError_t err = launch_step<MODE_RESET>(*args, (cudaStream_t)stream);
-    return (int)(err ? err : cudaGetLastError());
+    if (!step_args_ok(args)) return (int)cudaErrorInvalidValue;
+    return (int)launch_step<MODE_RESET>(*args, (cudaStream_t)stream);
 }
 
 int navgym_reset_envs(const navgym_step_args_t *args, const uint8_t *mask, void *stream)
 {
     if (args->num_envs <= 0) return 0;
-    if (!mask || !obs_rows_ok(args->obs_format, args->obs_stride, args->num_scan_stack, args->obs) ||
-        args->env_begin < 0 || args->env_count < 0 || args->env_begin + args->env_count > args->num_envs ||
-        args->env_begin > args->num_envs)
+    // (the masked reset may scan the next episode's geometry alone)
+    if (!mask || !step_args_ok(args) || !obstacle_slots_ok(args->max_disc, args->max_seg, args->discs_reset, args->segs_reset))
         return (int)cudaErrorInvalidValue;
-    if (args->env_begin == args->num_envs) return 0;   // an empty range
-    const cudaError_t err = launch_step<MODE_MASKED_RESET>(*args, (cudaStream_t)stream, mask);
-    return (int)(err ? err : cudaGetLastError());
+    return (int)launch_step<MODE_MASKED_RESET>(*args, (cudaStream_t)stream, mask);
 }
 
 int navgym_export_env_len(int num_scan_stack)
@@ -179,7 +186,7 @@ int navgym_export_env_len(int num_scan_stack)
 
 int navgym_export_env(const navgym_step_args_t *args, int env, double *out_dev, void *stream)
 {
-    if (env < 0 || env >= args->num_envs || !out_dev) return (int)cudaErrorInvalidValue;
+    if (!step_args_ok(args) || env < 0 || env >= args->num_envs || !out_dev) return (int)cudaErrorInvalidValue;
     export_env_kernel<<<1, 256, 0, (cudaStream_t)stream>>>(*args, env, out_dev);
     g_launches++;
     return (int)cudaGetLastError();
@@ -191,11 +198,7 @@ int navgym_compute_rewards(const navgym_her_args_t *args, void *stream)
     if (!obs_rows_ok(args->obs_format, args->obs_stride, args->num_scan_stack, args->obs))
         return (int)cudaErrorInvalidValue;
     // warps stride over the rows: at most one full wave of CTAs
-    static int sms = 0;
-    if (!sms) {
-        int dev = 0;
-        if (cudaGetDevice(&dev) != cudaSuccess || cudaDeviceGetAttribute(&sms, cudaDevAttrMultiProcessorCount, dev) != cudaSuccess || sms <= 0) sms = 148;
-    }
+    static const int sms = sm_count();
     const int warps_per_cta = NAVGYM_HER_THREADS / 32;
     const int want = (args->count + warps_per_cta - 1) / warps_per_cta;
     const int ctas = want < sms * HER_CTAS_PER_SM ? want : sms * HER_CTAS_PER_SM;
@@ -222,20 +225,6 @@ int navgym_sizeof_plan_args(void) { return (int)sizeof(navgym_plan_args_t); }
 int navgym_sizeof_plan_map(void) { return (int)sizeof(navgym_plan_map_t); }
 int navgym_sizeof_move_args(void) { return (int)sizeof(navgym_move_args_t); }
 
-int navgym_policy_features(const float *scan, int n, const float *w1, const float *b1, const float *w2,
-                           const float *b2, float *features, void *stream)
-{
-    if (n <= 0) return 0;
-    if (!scan || !w1 || !b1 || !w2 || !b2 || !features) return (int)cudaErrorInvalidValue;
-    int dev = 0, sms = 148;
-    cudaGetDevice(&dev);
-    cudaDeviceGetAttribute(&sms, cudaDevAttrMultiProcessorCount, dev);
-    const int grid = n < 4 * sms ? n : 4 * sms;  // 4 CTAs of 48 KB shared memory per SM
-    policy_features_kernel<<<grid, 128, 0, (cudaStream_t)stream>>>(scan, n, w1, b1, w2, b2, features);
-    g_launches++;
-    return (int)cudaGetLastError();
-}
-
 // ---- the pedestrian policy as one native pipeline (include/navgym_b200.h, navgym_policy_*)
 size_t navgym_policy_workspace_bytes(int max_n) { return policy_ws_layout(max_n).total; }
 int navgym_sizeof_policy_params(void) { return (int)sizeof(navgym_policy_params_t); }
@@ -251,9 +240,8 @@ navgym_policy_t *navgym_policy_create(const navgym_policy_params_t *p, void *str
     pol->max_n = p->max_n;
     pol->ws = (uint8_t *)p->workspace;
     pol->L = L;
-    pol->sms = 148;
     cudaGetDevice(&pol->device);
-    cudaDeviceGetAttribute(&pol->sms, cudaDevAttrMultiProcessorCount, pol->device);
+    pol->sms = sm_count();
     const uint64_t np = ((uint64_t)p->max_n + 127) / 128 * 128;
     cudaStream_t st = (cudaStream_t)stream;
     bool ok = cudaMemsetAsync(pol->ws + L.fh, 0, (size_t)np * 4096 * 2, st) == cudaSuccess &&
@@ -374,26 +362,6 @@ int navgym_calc_range_many(const float *dist_dev, int W, int H, const float *ins
     if (N <= 0) return 0;
     calc_range_many_kernel<<<(N + 127) / 128, 128, 0, (cudaStream_t)stream>>>(
         dist_dev, W, H, ins_dev, outs_dev, N, max_range, t_stop, hits_dev);
-    g_launches++;
-    return (int)cudaGetLastError();
-}
-
-int navgym_render_segments_in_lidar(float *ranges_dev, const float *headings_dev, int K,
-                                    const float *segs_dev, int S, float ox, float oy, void *stream)
-{
-    if (K <= 0) return 0;
-    render_in_lidar_kernel<<<(K + 127) / 128, 128, 0, (cudaStream_t)stream>>>(
-        ranges_dev, headings_dev, K, segs_dev, S, nullptr, 0, ox, oy);
-    g_launches++;
-    return (int)cudaGetLastError();
-}
-
-int navgym_render_discs_in_lidar(float *ranges_dev, const float *headings_dev, int K,
-                                 const float *discs_dev, int D, float ox, float oy, void *stream)
-{
-    if (K <= 0) return 0;
-    render_in_lidar_kernel<<<(K + 127) / 128, 128, 0, (cudaStream_t)stream>>>(
-        ranges_dev, headings_dev, K, nullptr, 0, discs_dev, D, ox, oy);
     g_launches++;
     return (int)cudaGetLastError();
 }

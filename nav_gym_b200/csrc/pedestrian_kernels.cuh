@@ -1,6 +1,6 @@
 // pedestrian_kernels.cuh -- part of navgym_b200.cu (included there; one translation unit).
-// The pedestrians of env.py:617-693 on the device: their lidar, route following, motion, the
-// policy network's convolutional front end, and the geometry the robot's lidar sees.
+// The pedestrians of env.py:617-693 on the device: their lidar, route following, motion, and
+// the geometry the robot's lidar sees.
 // ------------------------------------------------------------------ pedestrian lidar
 // The scan every simulated pedestrian takes of its surroundings (env.py:683-693): map raycast
 // from its own pose + the closed footprints of the robot and the other pedestrians, clipped,
@@ -439,84 +439,6 @@ __global__ void peds_move_kernel(const navgym_move_args_t a)
     q[0] = (float)x; q[1] = (float)y; q[2] = (float)th;
     q[9] = (float)d[0]; q[10] = (float)d[1]; q[11] = (float)d[2];
     q[12] = a.has_legs[n] ? 1.0f : 0.0f;
-}
-
-// ------------------------------------------------------------------ pedestrian policy front end
-// (include/navgym_b200.h, navgym_policy_features.)  128 threads; a CTA keeps the second
-// convolution's weights in shared memory and walks over pedestrians: conv1 fills h1 in shared
-// memory, then conv2 is register-tiled: warp w owns output channels 8w .. 8w + 7, lane l output
-// positions 4l .. 4l + 3 (32 accumulators); per input channel a lane reads its 9 inputs with
-// three loads and the warp's 24 weights as six broadcast LDS.128 -- 9 shared-memory loads per
-// 96 FMA, where one position per thread needed 25.
-#define PF_H1 264  // row pitch of h1 (32-byte multiple): [0] = left pad, [1 + q] = conv1 output q (q < 255), [256] = right pad
-__global__ void __launch_bounds__(128) policy_features_kernel(const float *__restrict__ scan, int n,
-                                                              const float *__restrict__ w1, const float *__restrict__ b1,
-                                                              const float *__restrict__ w2, const float *__restrict__ b2,
-                                                              float *__restrict__ out)
-{
-    __shared__ __align__(16) float w2s[32 * 3 * 32];  // [ci][tap][co]
-    __shared__ __align__(16) float h1[32 * PF_H1];
-    __shared__ float xs[516];                          // [0] = left pad, [1 + i] = input i
-    __shared__ float w1s[32 * 5], b1s[32], b2s[32];
-    const int t = threadIdx.x;
-    for (int i = t; i < 32 * 32 * 3; i += 128) {
-        const int co = i / 96, ci = (i / 3) % 32, k = i % 3;
-        w2s[(ci * 3 + k) * 32 + co] = w2[i];
-    }
-    for (int i = t; i < 160; i += 128) w1s[i] = w1[i];
-    if (t < 32) { b1s[t] = b1[t]; b2s[t] = b2[t]; }
-    for (int c = t; c < 32; c += 128) { h1[c * PF_H1] = 0.0f; h1[c * PF_H1 + 256] = 0.0f; }
-    if (t == 0) { xs[0] = 0.0f; xs[513] = 0.0f; xs[514] = 0.0f; xs[515] = 0.0f; }
-    for (int ped = blockIdx.x; ped < n; ped += gridDim.x) {
-        __syncthreads();  // weights ready / previous pedestrian's h1 no longer read
-        for (int i = t; i < 512; i += 128) {
-            const double r = fmin(fmax((double)scan[(size_t)ped * 512 + i], 0.0), 6.0);
-            xs[1 + i] = (float)(r / 6.0 - 0.5);  // env.py:627-629, 648
-        }
-        __syncthreads();
-        {   // conv1: thread t owns output positions t and t + 128 of every channel
-            float xa[5], xb[5];
-#pragma unroll
-            for (int k = 0; k < 5; k++) { xa[k] = xs[2 * t + k]; xb[k] = t < 127 ? xs[2 * (t + 128) + k] : 0.0f; }  // input 2q - 1 + k
-#pragma unroll 4
-            for (int c = 0; c < 32; c++) {
-                float a0 = b1s[c], a1 = a0;
-#pragma unroll
-                for (int k = 0; k < 5; k++) { a0 = fmaf(w1s[c * 5 + k], xa[k], a0); a1 = fmaf(w1s[c * 5 + k], xb[k], a1); }
-                h1[c * PF_H1 + 1 + t] = fmaxf(a0, 0.0f);
-                if (t < 127) h1[c * PF_H1 + 129 + t] = fmaxf(a1, 0.0f);
-            }
-        }
-        __syncthreads();
-        const int wco = (t >> 5) * 8, p0 = (t & 31) * 4;
-        float acc[8][4];
-#pragma unroll
-        for (int c = 0; c < 8; c++)
-#pragma unroll
-            for (int j = 0; j < 4; j++) acc[c][j] = b2s[wco + c];
-#pragma unroll 2
-        for (int ci = 0; ci < 32; ci++) {
-            // inputs 2 p0 - 1 .. 2 p0 + 7 = h1 row entries 2 p0 .. 2 p0 + 8
-            const float *row = h1 + ci * PF_H1 + 2 * p0;
-            const float4 i0 = *reinterpret_cast<const float4 *>(row), i1 = *reinterpret_cast<const float4 *>(row + 4);
-            const float in[9] = {i0.x, i0.y, i0.z, i0.w, i1.x, i1.y, i1.z, i1.w, row[8]};
-#pragma unroll
-            for (int k = 0; k < 3; k++) {
-                const float4 *wr = reinterpret_cast<const float4 *>(w2s + (ci * 3 + k) * 32 + wco);
-                const float4 wa = wr[0], wb = wr[1];
-                const float wv[8] = {wa.x, wa.y, wa.z, wa.w, wb.x, wb.y, wb.z, wb.w};
-#pragma unroll
-                for (int c = 0; c < 8; c++)
-#pragma unroll
-                    for (int j = 0; j < 4; j++) acc[c][j] = fmaf(in[2 * j + k], wv[c], acc[c][j]);
-            }
-        }
-        float *o = out + (size_t)ped * 4096 + p0;
-#pragma unroll
-        for (int c = 0; c < 8; c++)
-            *reinterpret_cast<float4 *>(o + (wco + c) * 128) =
-                make_float4(fmaxf(acc[c][0], 0.0f), fmaxf(acc[c][1], 0.0f), fmaxf(acc[c][2], 0.0f), fmaxf(acc[c][3], 0.0f));
-    }
 }
 
 // ------------------------------------------------------------------ scripted pedestrians

@@ -150,3 +150,37 @@ def test_every_field_offset_matches_the_header(tmp_path):
             n_checked += 1
         assert C.sizeof(cls) == [x for x in seen[s] if x[0] == '.'][0][1], s
     assert n_checked > 150
+
+
+# ---- argument checks of the entry points that take a navgym_step_args_t.  The blocks hold NULL
+# device pointers: they are refused, or found empty, before any device work, so no GPU is needed.
+def _step_args(**fields):
+    a = _lib.StepArgs()
+    a.num_envs, a.obs_stride, a.num_scan_stack = 4, _lib.OBS_DIM, 1
+    for k, v in fields.items():
+        setattr(a, k, v)
+    return a
+
+
+@pytest.mark.parametrize('fields', [dict(env_begin=-1), dict(env_begin=5), dict(env_count=-1),
+                                    dict(env_begin=1, env_count=4), dict(obs_format=7)],
+                         ids=lambda f: ','.join('%s=%d' % kv for kv in f.items()))
+def test_step_entry_points_reject_a_bad_argument_block(lib, fields):
+    a = C.byref(_step_args(**fields))
+    mask, out = (C.c_uint8 * 4)(), (C.c_double * 4096)()
+    launches = lib.navgym_launch_count()
+    assert lib.navgym_step_batch(a, None) == 1   # cudaErrorInvalidValue
+    assert lib.navgym_reset_obs_batch(a, None) == 1
+    assert lib.navgym_reset_envs(a, C.cast(mask, C.c_void_p), None) == 1
+    assert lib.navgym_export_env(a, 0, C.cast(out, C.c_void_p), None) == 1
+    assert lib.navgym_launch_count() == launches
+
+
+def test_step_entry_points_accept_an_empty_range(lib):
+    a = C.byref(_step_args(env_begin=4, env_count=0))
+    mask = (C.c_uint8 * 4)()
+    launches = lib.navgym_launch_count()
+    assert lib.navgym_step_batch(a, None) == 0
+    assert lib.navgym_reset_obs_batch(a, None) == 0
+    assert lib.navgym_reset_envs(a, C.cast(mask, C.c_void_p), None) == 0
+    assert lib.navgym_launch_count() == launches

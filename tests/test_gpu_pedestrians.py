@@ -74,45 +74,6 @@ def test_policy_forward_on_device(name):
     assert np.allclose(m.cpu().numpy().reshape(T, P, 2), G['mean'], rtol=0, atol=2e-5)
 
 
-@pytest.mark.parametrize('name', gu.human_trace_names())
-def test_policy_features_kernel_and_folded_forward(name):
-    """The fused convolutional front end (navgym_policy_features) against torch's two conv1d
-    layers on the reference's recorded policy inputs, and the whole folded forward against the
-    reference's recorded means."""
-    import ctypes as C
-    import torch.nn.functional as F
-    from nav_gym_b200 import _lib
-    from nav_gym_b200.pedestrians import HumanPolicy, preprocess_scan
-    G = gu.load(name)
-    torch.manual_seed(1234)
-    pol = HumanPolicy().cuda()
-    T, P = G['mean'].shape[:2]
-    # the raw scans the policy inputs were made from: scan0, then each step's scan_out
-    raw = np.concatenate([G['scan0'][None], G['scan_out'][:-1]]).reshape(T * P, 512)
-    x = torch.from_numpy(raw).cuda()
-    assert np.array_equal(preprocess_scan(x).cpu().numpy().reshape(T, P, 512), G['scan_in'])
-    feat = torch.empty(T * P, 4096, device='cuda')
-    w = (pol.act_fea_cv1.weight.sum(1).contiguous(), pol.act_fea_cv1.bias, pol.act_fea_cv2.weight.contiguous(), pol.act_fea_cv2.bias)
-    lib = _lib.load()
-    vp = lambda t: C.c_void_p(t.data_ptr())
-    with torch.no_grad():
-        _lib.check(lib.navgym_policy_features(vp(x), T * P, *[vp(t) for t in w], vp(feat), None), 'features')
-        x3 = preprocess_scan(x)[:, None, :].expand(-1, 3, -1).contiguous()
-        tf32 = torch.backends.cudnn.allow_tf32
-        torch.backends.cudnn.allow_tf32 = False  # cuDNN's default would round the inputs to TF32
-        try:
-            want = F.relu(pol.act_fea_cv2(F.relu(pol.act_fea_cv1(x3)))).reshape(T * P, -1)
-        finally:
-            torch.backends.cudnn.allow_tf32 = tf32
-        torch.cuda.synchronize()
-        assert torch.allclose(feat, want, rtol=0, atol=2e-6), float((feat - want).abs().max())
-        h = F.relu(pol.act_fc1(feat))
-        h = F.relu(pol.act_fc2(torch.cat((h, torch.from_numpy(G['goal_local']).cuda().reshape(-1, 2),
-                                          torch.from_numpy(G['speed']).cuda().reshape(-1, 2)), -1)))
-        m = torch.cat((torch.sigmoid(pol.actor1(h)), torch.tanh(pol.actor2(h))), -1)
-    assert np.allclose(m.cpu().numpy().reshape(T, P, 2), G['mean'], rtol=0, atol=2e-5)
-
-
 @pytest.mark.parametrize('n', [1, 77, 128, 300, 1029, 19200])
 def test_native_policy_stage_by_stage(n):
     """navgym_policy_mean (front end -> tcgen05 act_fc1 in the f16x3 scheme -> act_fc2 + heads)
@@ -160,15 +121,19 @@ def test_native_policy_stage_by_stage(n):
 @pytest.mark.parametrize('name', gu.human_trace_names())
 def test_native_policy_reproduces_the_reference_means(name):
     """The reference's recorded policy outputs (humans_*.npz `mean`, minted by running its own
-    human_policy.py on the CPU) from its recorded raw scans, through the native pipeline."""
-    from nav_gym_b200.pedestrians import HumanPolicy, NativePolicy
+    human_policy.py on the CPU) from its recorded raw scans, through the native pipeline; the
+    recorded policy inputs are those raw scans preprocessed."""
+    from nav_gym_b200.pedestrians import HumanPolicy, NativePolicy, preprocess_scan
     G = gu.load(name)
     torch.manual_seed(1234)
     pol = HumanPolicy().cuda()
     T, P = G['mean'].shape[:2]
+    # the raw scans the policy inputs were made from: scan0, then each step's scan_out
     raw = np.concatenate([G['scan0'][None], G['scan_out'][:-1]]).reshape(T * P, 512)
+    x = torch.from_numpy(raw).cuda()
+    assert np.array_equal(preprocess_scan(x).cpu().numpy().reshape(T, P, 512), G['scan_in'])
     nat = NativePolicy(pol, T * P, 'cuda:0')
-    m = nat.mean(torch.from_numpy(raw).cuda().contiguous(), torch.from_numpy(G['goal_local']).cuda().reshape(-1, 2).contiguous(),
+    m = nat.mean(x, torch.from_numpy(G['goal_local']).cuda().reshape(-1, 2).contiguous(),
                  torch.from_numpy(G['speed']).cuda().reshape(-1, 2).contiguous())
     torch.cuda.synchronize()
     assert np.allclose(m.cpu().numpy().reshape(T, P, 2), G['mean'], rtol=0, atol=2e-5)
