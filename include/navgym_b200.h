@@ -201,6 +201,17 @@ typedef void (*navgym_policy_fn)(void *user, int group, int env_begin, int env_e
 int navgym_host_rollout(navgym_host_pipe_t *pipe, const navgym_step_args_t *args, int64_t steps,
                         navgym_policy_fn policy, void *user, float *actions_host, float *obs_host,
                         float *reward_host, uint8_t *done_host);
+/* navgym_step_batch_host, navgym_step_batch_host_submit and navgym_host_rollout return
+ * cudaErrorInvalidValue for
+ *   - a NULL pipe, or args->num_envs other than the pipe's;
+ *   - a NULL args->actions (the device staging buffer of the actions);
+ *   - an argument block that navgym_step_batch rejects (see above; the pipe sets env_begin,
+ *     env_count, sched and sched_phase of each group itself);
+ *   - obs_host rows that args->obs_format does not allow (float16: a 4-byte aligned base);
+ *   - submit: a group outside [0, groups); rollout: a NULL policy or steps < 0.
+ * A rejected call enqueues nothing and leaves the pipe as it was.  So does a submit that fails
+ * (a failed copy or graph capture): a group's schedule phase and cached graphs change only once
+ * its step has been enqueued. */
 /* built-in policy: step s plays row (s mod rows) of a host action bank f32 [rows][num_envs][2] */
 typedef struct {
     const float *actions;

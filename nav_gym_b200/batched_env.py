@@ -281,19 +281,9 @@ class BatchedNavGym(object):
         prioritised streams, each followed by the D2H copy of its rows, so the copies of early
         chunks overlap the raycast of later ones (PCIe is the end-to-end bound: 2.1 KB per
         env-step).  Returns when all results have landed."""
-        for t in (actions_host, obs_host, reward_host, done_host):
-            if not t.is_pinned() or not t.is_contiguous():
-                raise ValueError('step_host needs contiguous pinned host tensors')
-        assert obs_host.dtype == self.obs_dtype and tuple(obs_host.shape) == (self.B, self.obs_dim)
-        assert reward_host.dtype == torch.float32 and done_host.dtype == torch.uint8
-        assert actions_host.dtype == torch.float32 and actions_host.numel() == 2 * self.B
-        if self.peds is not None:
-            chunks = 1
-            self._peds_emit(advance=True)
-            self._geom(self._pdiscs, self._pnd, self._psegs, self._pns, None)
-        else:
-            self._geom(None, None, None, None, None)
-        self._make_pipe(chunks)
+        self._check_host_tensors('step_host', actions_host, obs_host, reward_host, done_host)
+        self._geom(*self._obstacles(None, None, None, None, advance=True), None)
+        self._make_pipe(1 if self.peds is not None else chunks)
         with torch.cuda.device(self.device):
             _lib.check(self.lib.navgym_step_batch_host(
                 self._pipe[0], C.byref(self.args), self._stream(), _ptr(actions_host), _ptr(obs_host),
@@ -307,12 +297,7 @@ class BatchedNavGym(object):
         (begin, end) bounds."""
         if self.peds is not None:
             raise NotImplementedError('async host groups with device pedestrians')
-        for t in (actions_host, obs_host, reward_host, done_host):
-            if not t.is_pinned() or not t.is_contiguous():
-                raise ValueError('host_groups needs contiguous pinned host tensors')
-        assert obs_host.dtype == self.obs_dtype and tuple(obs_host.shape) == (self.B, self.obs_dim)
-        assert actions_host.dtype == torch.float32 and actions_host.numel() == 2 * self.B
-        assert reward_host.dtype == torch.float32 and done_host.dtype == torch.uint8
+        self._check_host_tensors('host_groups', actions_host, obs_host, reward_host, done_host)
         self._make_pipe(groups, fresh=True)
         self._geom(None, None, None, None, None)
         self._host_bufs = (actions_host, obs_host, reward_host, done_host)
@@ -325,6 +310,16 @@ class BatchedNavGym(object):
             _lib.check(self.lib.navgym_host_pipe_group_bounds(self._pipe[0], g, C.byref(b0), C.byref(b1)), 'group_bounds')
             bounds.append((b0.value, b1.value))
         return bounds
+
+    def _check_host_tensors(self, what, actions_host, obs_host, reward_host, done_host):
+        """The host-buffer calls' [B, ...] host tensors: ValueError unless pinned and contiguous,
+        AssertionError for a dtype or shape other than the env's."""
+        for t in (actions_host, obs_host, reward_host, done_host):
+            if not t.is_pinned() or not t.is_contiguous():
+                raise ValueError('%s needs contiguous pinned host tensors' % what)
+        assert obs_host.dtype == self.obs_dtype and tuple(obs_host.shape) == (self.B, self.obs_dim)
+        assert actions_host.dtype == torch.float32 and actions_host.numel() == 2 * self.B
+        assert reward_host.dtype == torch.float32 and done_host.dtype == torch.uint8
 
     def _make_pipe(self, groups, fresh=False):
         """(Re)create the host pipe -- its streams, events and schedule buffers live on the env's
@@ -540,15 +535,20 @@ class BatchedNavGym(object):
         with torch.cuda.device(self.device):
             _lib.check(self.lib.navgym_peds_advance(C.byref(self._pargs), self._stream()), 'peds_advance')
 
+    def _obstacles(self, discs, ndisc, segs, nseg, advance):
+        """The obstacle buffers a launch reads: the caller's or, with none given, the attached
+        pedestrians' geometry, emitted first (`advance`: scripted pedestrians move one step)."""
+        if self.peds is None or discs is not None or segs is not None:
+            return discs, ndisc, segs, nseg
+        self._peds_emit(advance=advance and self.peds_scripted)
+        return self._pdiscs, self._pnd, self._psegs, self._pns
+
     def _stream(self):
         return C.c_void_p(torch.cuda.current_stream(self.device).cuda_stream)
 
     def reset(self, discs=None, ndisc=None, segs=None, nseg=None, noise=None):
         """First observation of an episode from the state set by set_state (env.py:822-831)."""
-        if self.peds is not None and discs is None and segs is None:
-            self._peds_emit(advance=False)
-            discs, ndisc, segs, nseg = self._pdiscs, self._pnd, self._psegs, self._pns
-        self._geom(discs, ndisc, segs, nseg, noise)
+        self._geom(*self._obstacles(discs, ndisc, segs, nseg, advance=False), noise)
         with torch.cuda.device(self.device):
             _lib.check(self.lib.navgym_reset_obs_batch(C.byref(self.args), self._stream()), 'reset')
         return self.obs
@@ -612,10 +612,7 @@ class BatchedNavGym(object):
     def step(self, actions, discs=None, ndisc=None, segs=None, nseg=None, noise=None):
         """One lockstep NavGymEnv.step.  Returned tensors are owned by the env and overwritten
         by the next call (clone to keep)."""
-        if self.peds is not None and discs is None and segs is None:
-            self._peds_emit(advance=self.peds_scripted)
-            discs, ndisc, segs, nseg = self._pdiscs, self._pnd, self._psegs, self._pns
-        self._geom(discs, ndisc, segs, nseg, noise, actions)
+        self._geom(*self._obstacles(discs, ndisc, segs, nseg, advance=True), noise, actions)
         with torch.cuda.device(self.device):
             _lib.check(self.lib.navgym_step_batch(C.byref(self.args), self._stream()), 'step')
         if self.sched is not None:
