@@ -42,6 +42,11 @@ extern "C" {
 #define NAVGYM_OBS_F32 0
 #define NAVGYM_OBS_F16 1
 
+/* navgym_step_args_t.auto_reset: 0 = off, 1 = same-step (the launch that ends an episode writes
+ * the next episode's first observation over its final one), NAVGYM_AUTORESET_NEXT_STEP = the
+ * launch after the one that ends an episode starts the next (see navgym_step_batch). */
+#define NAVGYM_AUTORESET_NEXT_STEP 2
+
 /* rows of the structure-of-arrays float64 state block state[NAVGYM_NS][num_envs] */
 enum {
     NAVGYM_S_PX = 0, NAVGYM_S_PY, NAVGYM_S_TH,   /* robot pose (keti_robot.py:56-58) */
@@ -89,7 +94,8 @@ typedef struct {
     int32_t max_disc, max_seg;
     int32_t num_envs;
     int32_t obs_stride;      /* floats per obs row, >= 519 */
-    int32_t auto_reset;      /* 1: on done draw a spawn tuple and return the new first obs */
+    int32_t auto_reset;      /* 1: on done draw a spawn tuple and return the new first obs;
+                              * NAVGYM_AUTORESET_NEXT_STEP: draw it in the next launch */
     int32_t max_episode_steps; /* 0 = none (the reference has no time limit) */
     int32_t num_maps;
     int32_t resample_map;    /* 1: auto-reset also draws a new map id */
@@ -158,6 +164,28 @@ typedef struct {
 
 /* ---- fused hot path: NavGymEnv.step (env.py:591-728) over num_envs environments ------ */
 int navgym_step_batch(const navgym_step_args_t *args, void *stream);
+/* Next-step auto-reset (auto_reset = NAVGYM_AUTORESET_NEXT_STEP, Gymnasium's default).  `done` is
+ * then an INPUT as well.  For every environment e of the launch range:
+ *   - done[e] == 0 on entry: the step of auto_reset = 0, crash rollback and re-scan included.  The
+ *     row of an episode that ends now is its final observation, and its goal is still
+ *     state[NAVGYM_S_GX / S_GY];
+ *   - done[e] != 0 on entry: actions[e] is not read (a NaN action changes nothing), and the
+ *     environment starts its next episode bit for bit as navgym_reset_envs with mask[e] = 1 starts
+ *     it: the draw keyed by (env_offset + e, episodes[e]), episodes[e] += 1, steps[e] = 0, the
+ *     first observation in every stack slot, tail64, state, map_id, noise_std, the scan taken
+ *     against discs_reset / segs_reset when discs_reset != NULL, else against discs / segs.
+ *     Unlike navgym_reset_envs it also writes the step outputs: reward = 0, done = is_success =
+ *     is_crash = truncated = 0, distance = the distance from the new pose to the new goal (float64
+ *     rounded to float32, as the step computes it), the mirrors alike; hits of that scan; and the
+ *     environment's entry in the next launch order.
+ * navgym_reset_obs_batch and navgym_reset_envs do not write done: a caller that resets
+ * environments through them clears their done bytes, or the next step starts yet another episode.
+ * Setting done[e] = 1 has the next step start a new episode for e.  Each draw depends only on
+ * the environment's own episodes[e]: for the same per-episode actions every episode's sequence of
+ * (episode, step) records is the one of auto_reset = 0 followed by navgym_reset_envs(mask = done)
+ * after every step, whatever the sharding.  The host-buffer entry points below launch through
+ * navgym_step_batch and so follow the same contract: the final row lands in obs_host at the
+ * ending step, the next episode's first row one step later. */
 /* The same step for a caller whose buffers live on the HOST (the reference's own calling
  * convention: numpy in, numpy out).  actions_host f32 [num_envs][2], obs_host f32
  * [num_envs][obs_stride] (rows of args->obs_format, like obs), reward_host f32 [num_envs],

@@ -26,6 +26,7 @@ MAX_DISC = 64
 MAX_SEG = 128
 SCHED_BUCKETS = 32
 OBS_F32, OBS_F16 = 0, 1   # navgym_step_args_t.obs_format
+AUTORESET_NEXT_STEP = 2   # navgym_step_args_t.auto_reset: start ended episodes in the next launch
 NS = 10
 S_PX, S_PY, S_TH, S_GX, S_GY, S_PPX, S_PPY, S_PYAW, S_PV, S_PW = range(NS)
 

@@ -127,6 +127,15 @@ class BatchedNavGym(object):
                  max_episode_steps=0, resample_map=False, scan_noise_std_range=(0.0, 0.05),
                  cell_rule='numpy1', early_stop=True, record_hits=False, longest_first=True,
                  num_scan_stack=1, obs_dtype=torch.float32, **reward):
+        # auto_reset: False (off), True (same-step: the ending launch writes the next episode's first
+        # observation over the final one) or 'next_step' (the next launch starts the new episode)
+        if isinstance(auto_reset, str):
+            if auto_reset != 'next_step':
+                raise ValueError("auto_reset must be True, False or 'next_step', not %r" % (auto_reset,))
+            auto_reset = _lib.AUTORESET_NEXT_STEP
+        else:
+            auto_reset = 1 if auto_reset else 0
+        self.next_step_reset = auto_reset == _lib.AUTORESET_NEXT_STEP
         self.lib = _lib.require_device()
         self.device = torch.device(device)
         self.B = B = int(num_envs)
@@ -185,7 +194,7 @@ class BatchedNavGym(object):
         a.max_disc, a.max_seg = self.max_disc, self.max_seg
         a.num_envs, a.obs_stride, a.num_scan_stack = B, self.obs_dim, S
         a.obs_format = obs_format
-        a.auto_reset, a.max_episode_steps = int(auto_reset), int(max_episode_steps)
+        a.auto_reset, a.max_episode_steps = auto_reset, int(max_episode_steps)
         a.num_maps, a.resample_map = self.pool.num_maps, int(resample_map)
         a.seed, a.env_offset = int(seed), int(env_offset)
         a.noise_lo, a.noise_hi = scan_noise_std_range
@@ -547,10 +556,13 @@ class BatchedNavGym(object):
         return C.c_void_p(torch.cuda.current_stream(self.device).cuda_stream)
 
     def reset(self, discs=None, ndisc=None, segs=None, nseg=None, noise=None):
-        """First observation of an episode from the state set by set_state (env.py:822-831)."""
+        """First observation of an episode from the state set by set_state (env.py:822-831).
+        With auto_reset='next_step' also clears done, so that the next step steps every env."""
         self._geom(*self._obstacles(discs, ndisc, segs, nseg, advance=False), noise)
         with torch.cuda.device(self.device):
             _lib.check(self.lib.navgym_reset_obs_batch(C.byref(self.args), self._stream()), 'reset')
+            if self.next_step_reset:
+                self.done.zero_()
         return self.obs
 
     def env_mask(self, envs):
@@ -595,9 +607,11 @@ class BatchedNavGym(object):
 
         Meant for auto_reset=False: step, read the rows of the ended episodes (their final
         observations; their goals are still state[S_GX / S_GY]), then reset_envs(done).  Works with
-        auto_reset=True too.  With scripted pedestrians the first scan sees the geometry the last
-        step emitted, not advanced, as auto-reset does.  An env driven by a PedestrianSim is reset
-        through sim.reset_envs, which also respawns its pedestrians."""
+        auto_reset=True too.  With auto_reset='next_step' it clears done for `envs`, so that the
+        next step steps them instead of starting yet another episode.  With scripted pedestrians
+        the first scan sees the geometry the last step emitted, not advanced, as auto-reset does.
+        An env driven by a PedestrianSim is reset through sim.reset_envs, which also respawns its
+        pedestrians."""
         if getattr(self, 'crowd', None) is not None:
             raise ValueError('this env is driven by a PedestrianSim: call sim.reset_envs(envs), which also '
                              'respawns its pedestrians')
@@ -607,16 +621,25 @@ class BatchedNavGym(object):
         self._reset_mask = mask  # kept alive until the next call; the launch is stream-ordered
         with torch.cuda.device(self.device):
             _lib.check(self.lib.navgym_reset_envs(C.byref(self.args), _ptr(mask), self._stream()), 'reset_envs')
+            if self.next_step_reset:   # after the launch: `mask` may be done itself
+                self.done.masked_fill_(mask.bool(), 0)
         return self.obs
 
     def step(self, actions, discs=None, ndisc=None, segs=None, nseg=None, noise=None):
         """One lockstep NavGymEnv.step.  Returned tensors are owned by the env and overwritten
-        by the next call (clone to keep)."""
+        by the next call (clone to keep).
+
+        With auto_reset='next_step' an env whose last step ended its episode (done set on entry)
+        ignores its action and starts the next episode instead: its row is the first observation,
+        its reward and flags are 0.  info['autoreset'] (bool [B], a new tensor) marks those envs;
+        their transitions are not the policy's and belong in no replay buffer."""
         self._geom(*self._obstacles(discs, ndisc, segs, nseg, advance=True), noise, actions)
         with torch.cuda.device(self.device):
             _lib.check(self.lib.navgym_step_batch(C.byref(self.args), self._stream()), 'step')
+            info = dict(is_success=self.is_success, is_crash=self.is_crash, distance=self.distance,
+                        episode_step=self.steps, truncated=self.truncated)
+            if self.next_step_reset:   # a stepped env has steps >= 1
+                info['autoreset'] = self.steps == 0
         if self.sched is not None:
             self.args.sched_phase = (self.args.sched_phase + 1) % 3
-        info = dict(is_success=self.is_success, is_crash=self.is_crash, distance=self.distance,
-                    episode_step=self.steps, truncated=self.truncated)
         return self.obs, self.reward, self.done, info

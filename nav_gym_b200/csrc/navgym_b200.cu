@@ -82,8 +82,8 @@ static bool obstacle_slots_ok(int max_disc, int max_seg, const void *discs, cons
 }
 
 // MODE_STEP / MODE_RESET / MODE_MASKED_RESET (step_kernel.cuh) over the launch's env range, which
-// step_args_ok has accepted; `mask` is read by the masked reset only.  An empty range launches
-// nothing.
+// step_args_ok has accepted; `mask` is read by the masked reset only.  A step with auto_reset ==
+// NAVGYM_AUTORESET_NEXT_STEP runs MODE_NEXT_STEP.  An empty range launches nothing.
 template <int MODE>
 static cudaError_t launch_step(const navgym_step_args_t &a, cudaStream_t st, const uint8_t *mask = nullptr)
 {
@@ -92,8 +92,15 @@ static cudaError_t launch_step(const navgym_step_args_t &a, cudaStream_t st, con
     // tail regime B (see step_kernel) while the launch is at most ~2.4 waves of CTAs (measured
     // crossover on B200: 5120 envs -2 %, 6144 envs +2 %)
     static const int coop_max = (int)(2.4 * sm_count() * NAVGYM_CTAS_PER_SM);
-    if (a.obs_format == NAVGYM_OBS_F16) launch_step_fmt<MODE, NAVGYM_OBS_F16>(a, mask, count, count <= coop_max, st);
-    else launch_step_fmt<MODE, NAVGYM_OBS_F32>(a, mask, count, count <= coop_max, st);
+    const bool coop = count <= coop_max, f16 = a.obs_format == NAVGYM_OBS_F16;
+    if (MODE == MODE_STEP && a.auto_reset == NAVGYM_AUTORESET_NEXT_STEP) {
+        if (f16) launch_step_fmt<MODE_NEXT_STEP, NAVGYM_OBS_F16>(a, mask, count, coop, st);
+        else launch_step_fmt<MODE_NEXT_STEP, NAVGYM_OBS_F32>(a, mask, count, coop, st);
+    } else if (f16) {
+        launch_step_fmt<MODE, NAVGYM_OBS_F16>(a, mask, count, coop, st);
+    } else {
+        launch_step_fmt<MODE, NAVGYM_OBS_F32>(a, mask, count, coop, st);
+    }
     g_launches++;
     return cudaGetLastError();
 }

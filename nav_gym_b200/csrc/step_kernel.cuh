@@ -362,8 +362,12 @@ constexpr float RISK_MARGIN = 0.25f;  // [m] clearance under which the next step
 //   MODE_MASKED_RESET  a new episode drawn exactly as the step's auto-reset draws it, then its
 //                      first observation as the auto-reset pass writes it (navgym_reset_envs):
 //                      no hits recorded, no launch-order filing.
-enum { MODE_STEP = 0, MODE_RESET = 1, MODE_MASKED_RESET = 2 };
-template <int MODE, bool COOP, int FMT>
+// NEXT (next-step auto-reset, step_kernel<MODE_NEXT_STEP>) runs MODE_STEP with auto-reset off, or
+// MODE_MASKED_RESET extended to write what a step writes: outputs (0, and the distance from the new
+// pose to the new goal), hits and the launch-order filing.  Neither doubles the cost class of a
+// risky environment: no step of this mode runs a reset scan after its own.
+enum { MODE_STEP = 0, MODE_RESET = 1, MODE_MASKED_RESET = 2, MODE_NEXT_STEP = 3 };
+template <int MODE, bool COOP, int FMT, bool NEXT = false>
 __device__ __forceinline__ void step_body(const navgym_step_args_t &a, EnvSmem &sm, const int e, const int tid,
                                           int *sched_cnt, int *sched_list)
 {
@@ -514,7 +518,7 @@ __device__ __forceinline__ void step_body(const navgym_step_args_t &a, EnvSmem &
             march_scan<COOP>(sm, a, 0, BPL / 4, tid);
             const int ci = sm.ci, cj = sm.cj;
             // ranges (env.py:426), all lanes active: sqrt(di^2 + dj^2) * resolution
-            const bool rec = !MASKED && pass == (IS_RESET_KERNEL ? PASS_RESET : PASS_STEP) && a.hits;
+            const bool rec = (!MASKED || NEXT) && pass == (IS_RESET_KERNEL ? PASS_RESET : PASS_STEP) && a.hits;
             const float max_range = sm.max_range, res32 = sm.res32;
 #pragma unroll
             for (int i = 0; i < BPL; i++) {
@@ -742,7 +746,7 @@ __device__ __forceinline__ void step_body(const navgym_step_args_t &a, EnvSmem &
                     if (a.truncated) a.truncated[e] = (uint8_t)trunc;
                     a.distance[e] = (float)dist_g;
                     int next = PASS_END;
-                    if (done && a.auto_reset) {
+                    if (done && !NEXT && a.auto_reset) {
                         // auto-reset: draw a spawn tuple (and a map) for the next episode
                         sm.noise_std = draw_episode(
                             a.maps, a.spawn_pool, a.num_maps, a.resample_map, a.seed, (uint32_t)(a.env_offset + e),
@@ -792,7 +796,7 @@ __device__ __forceinline__ void step_body(const navgym_step_args_t &a, EnvSmem &
             risky |= gx * gx + gy * gy < (a.dist_thresh + RISK_MARGIN) * (a.dist_thresh + RISK_MARGIN);
             risky |= a.max_episode_steps > 0 && sm.steps + 1 >= a.max_episode_steps;
         }
-        risky = __syncthreads_or(risky) && a.auto_reset;
+        risky = __syncthreads_or(risky) && !NEXT && a.auto_reset;
         if (tid == 0) {
             const long long kc = ((clock64() - t_pass) << (risky ? 1 : 0)) >> 13;
             sched_b = NAVGYM_SCHED_BUCKETS - 1 - (int)(kc > NAVGYM_SCHED_BUCKETS - 1 ? NAVGYM_SCHED_BUCKETS - 1 : kc);
@@ -842,6 +846,18 @@ __device__ __forceinline__ void step_body(const navgym_step_args_t &a, EnvSmem &
             a.map_id[e] = sm.map;
             if (a.episodes) a.episodes[e] = sm.episode;
             if (a.noise_std) a.noise_std[e] = sm.noise_std;
+            if (MASKED && NEXT) {   // the outputs of a launch that started a new episode
+                const double ddx = __dsub_rn(sm.gx, sm.px), ddy = __dsub_rn(sm.gy, sm.py);
+                const double dist_g = sqrt(__dadd_rn(__dmul_rn(ddx, ddx), __dmul_rn(ddy, ddy)));
+                a.reward[e] = 0.0f;
+                a.done[e] = 0;
+                if (a.reward_mirror) a.reward_mirror[e] = 0.0f;
+                if (a.done_mirror) a.done_mirror[e] = 0;
+                a.is_success[e] = 0;
+                a.is_crash[e] = 0;
+                if (a.truncated) a.truncated[e] = 0;
+                a.distance[e] = (float)dist_g;
+            }
         }
     }
     if (sched_cnt && tid == 0) sched_list[(size_t)sched_b * B + sched_pos] = e;
@@ -896,15 +912,25 @@ __device__ __forceinline__ int sched_lookup(const navgym_step_args_t &a, const i
 // environments at the price of ~4 % more gathers and instructions, which pays while a launch is
 // at most ~2 waves of CTAs (4096 envs: -16 %) and costs beyond (32768 envs: +7 %).  FMT is the
 // observation row format (NAVGYM_OBS_F32 / F16, ObsRow): it only changes the row stores.
+// MODE_NEXT_STEP (auto_reset == NAVGYM_AUTORESET_NEXT_STEP): an environment whose done byte is
+// set on entry starts its next episode instead of stepping; the others step with auto-reset off.
+// Every thread of the CTA reads the byte before the first barrier of the body, and only this CTA
+// writes it, after that barrier: the choice is CTA-uniform.
 template <int MODE, bool COOP, int FMT>
 __global__ void __launch_bounds__(NAVGYM_CTA_THREADS, NAVGYM_CTAS_PER_SM) step_kernel(const navgym_step_args_t a)
 {
-    static_assert(MODE == MODE_STEP || MODE == MODE_RESET, "the masked reset is reset_envs_kernel");
+    static_assert(MODE == MODE_STEP || MODE == MODE_RESET || MODE == MODE_NEXT_STEP,
+                  "the masked reset is reset_envs_kernel");
     __shared__ EnvSmem sm;
     int e = a.env_begin + (int)blockIdx.x;
     int *sched_cnt = nullptr, *sched_list = nullptr;
-    if (MODE == MODE_STEP && a.sched) e = sched_lookup(a, (int)blockIdx.x, sched_cnt, sched_list);
-    step_body<MODE, COOP, FMT>(a, sm, e, (int)threadIdx.x, sched_cnt, sched_list);
+    if ((MODE == MODE_STEP || MODE == MODE_NEXT_STEP) && a.sched) e = sched_lookup(a, (int)blockIdx.x, sched_cnt, sched_list);
+    if constexpr (MODE == MODE_NEXT_STEP) {
+        if (a.done[e]) step_body<MODE_MASKED_RESET, COOP, FMT, true>(a, sm, e, (int)threadIdx.x, sched_cnt, sched_list);
+        else step_body<MODE_STEP, COOP, FMT, true>(a, sm, e, (int)threadIdx.x, sched_cnt, sched_list);
+    } else {
+        step_body<MODE, COOP, FMT>(a, sm, e, (int)threadIdx.x, sched_cnt, sched_list);
+    }
 }
 
 // The masked reset (navgym_reset_envs): CTA b takes environment env_begin + b in index order and

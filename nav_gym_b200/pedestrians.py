@@ -241,6 +241,9 @@ class PedestrianSim(object):
     def __init__(self, env, max_ped, nped=None, policy=None, v_pref_range=(0.0, 0.6), has_legs_ratio=0.5,
                  num_goals=32, min_goal_dist=10.0, min_robot_dist=4.0, seed=0):
         from . import maps as M
+        if env.args.auto_reset == _lib.AUTORESET_NEXT_STEP:
+            # act() respawns the pedestrians of an env in the launch that ends its episode
+            raise ValueError("PedestrianSim does not drive an auto_reset='next_step' env")
         self.env, self.device = env, env.device
         self.B, self.P = env.B, int(max_ped)
         if self.P > 127:  # navgym_agent_scan_batch, crowd mode: one thread per other agent

@@ -1,11 +1,13 @@
-"""Cost of the masked device reset (BatchedNavGym.reset_envs) on the C2 world, one command.
+"""Cost of the masked device reset (BatchedNavGym.reset_envs) and of next-step auto-reset on the
+C2 world, one command.
 
   python tools/reset_envs_bench.py --out DIR [--steps K] [--warmup W] [--reps R]
 
-Two arms, alternated (auto, masked, auto, masked, ...), R times each, at 4096 and 32 768 envs
-with bench.py's action law (a seeded bank of uniform actions):
+Three arms, alternated (auto, masked, next, auto, masked, next, ...), R times each, at 4096 and
+32 768 envs with bench.py's action law (a seeded bank of uniform actions):
   auto     BatchedNavGym(auto_reset=True): env.step
   masked   BatchedNavGym(auto_reset=False): env.step, then env.reset_envs(env.done)
+  next     BatchedNavGym(auto_reset='next_step'): env.step
 ms per step = CUDA events around the step (and, in the masked arm, the reset), L2 flushed
 (256 MiB memset) before every timed step, as bench.py does.  Then reset_envs alone at mask
 fractions 0, 1 %, 10 % and 100 % (random masks, fixed seed), same timing and flush.  The card's
@@ -53,11 +55,15 @@ def timed(torch, fn, K, W, flush):
     return np.array([s.elapsed_time(e) for s, e in ev])
 
 
-def run_arm(torch, masked, mp, banks, args, flush):
+ARMS = {'auto': True, 'masked': False, 'next': 'next_step'}   # arm -> auto_reset
+
+
+def run_arm(torch, arm, mp, banks, args, flush):
     from nav_gym_b200.batched_env import BatchedNavGym
+    masked = arm == 'masked'
     out = {}
     for B in SIZES:
-        env = BatchedNavGym(B, mp, device='cuda:0', seed=1234, auto_reset=not masked)
+        env = BatchedNavGym(B, mp, device='cuda:0', seed=1234, auto_reset=ARMS[arm])
         env.reset_from_spawn_pool(np.random.RandomState(100))
         bank = banks[B]
         n_bank = bank.shape[0]
@@ -130,25 +136,28 @@ def main():
     mp = MapPool([m], dev, spawn_pools=[pool])
     banks = {B: bench._bank(torch, dev, 64, B, 7) for B in SIZES}
     flush = torch.empty(256 << 20, dtype=torch.uint8, device=dev)
-    reps = {'auto': [], 'masked': []}
+    reps = {k: [] for k in ARMS}
     for r in range(args.reps):
-        for key in ('auto', 'masked'):
-            reps[key].append(run_arm(torch, key == 'masked', mp, banks, args, flush))
+        for key in ARMS:
+            reps[key].append(run_arm(torch, key, mp, banks, args, flush))
     summ = {k: summarize(v) for k, v in reps.items()}
     alone = summarize([reset_only(torch, mp, args, flush) for _ in range(args.reps)])
     med = lambda k, p: summ[k][p]['median']
     result = {
         'card': info, 'world': 'C2 (worlds.load_bench_world)', 'steps': args.steps, 'warmup': args.warmup,
-        'reps_per_arm': args.reps, 'order': 'auto, masked alternating; then reset_envs alone',
+        'reps_per_arm': args.reps, 'order': 'auto, masked, next alternating; then reset_envs alone',
         'summary': summ, 'reset_envs_alone': alone,
         'masked_minus_auto_ms_median': {B: med('masked', 'step_%d.ms_mean' % B) - med('auto', 'step_%d.ms_mean' % B)
                                         for B in SIZES},
+        'next_minus_auto_ms_median': {B: med('next', 'step_%d.ms_mean' % B) - med('auto', 'step_%d.ms_mean' % B)
+                                      for B in SIZES},
         'reps': reps,
     }
     os.makedirs(args.out, exist_ok=True)
     with open(os.path.join(args.out, 'reset_envs_bench.json'), 'w') as f:
         json.dump(result, f, indent=1)
-    print(json.dumps({k: result[k] for k in ('card', 'summary', 'reset_envs_alone', 'masked_minus_auto_ms_median')}))
+    print(json.dumps({k: result[k] for k in ('card', 'summary', 'reset_envs_alone', 'masked_minus_auto_ms_median',
+                                                   'next_minus_auto_ms_median')}))
 
 
 if __name__ == '__main__':
