@@ -435,7 +435,33 @@ typedef struct {
     uint64_t robot_seed;
     int32_t num_maps, resample_map;
     int32_t cand_next_spawn, _pad2;
+    int32_t num_humans_lo, num_humans_hi;  /* 0, 0 = off: every episode keeps nped[e] */
+    const int32_t *cand_nped_prev;  /* [num_envs] in: the previous call's cand_nped */
+    int32_t *cand_nped;             /* [num_envs] out: the count of the next episode drawn by this call */
+    int32_t *nped_out;              /* [num_envs] out: the count after this call's respawns */
 } navgym_plan_args_t;
+/* Per-episode pedestrian counts (num_humans_hi > 0): NavGym-v0 draws num_humans uniformly from
+ * [5, 15] at every reset (__init__.py:26-36, env.py:281-292).  Requires 0 <= num_humans_lo <=
+ * num_humans_hi <= max_ped and nped, cand_pose, cand_nped_prev, cand_nped, nped_out
+ * (cudaErrorInvalidValue otherwise).  Then:
+ *   1. draw: every call also draws the count of each environment's next episode into cand_nped[e]:
+ *      lo + floor(u * (hi - lo + 1)), u from the Philox counter (env_offset + e, 0, step, 0x5b0e)
+ *      under `seed`, one value per environment.  No other draw moves, so with lo == hi == k a run
+ *      is bit for bit the run with nped[e] = k everywhere;
+ *   2. candidates are drawn for every slot below that new count, whatever nped[e] is;
+ *   3. adopt: an environment with respawn[e] != 0 takes cand_nped_prev[e] (the cand_nped of the
+ *      previous call) with the candidates, the others keep nped[e]; that count goes to nped_out[e],
+ *      and adoption and route following run for the slots below it.  The state of the slots at or
+ *      beyond it is not written;
+ *   4. hazard: every thread of environment e reads nped[e] and cand_nped_prev[e], and e's slots can
+ *      span two CTAs, so the launch writes neither.  cand_nped[e] and nped_out[e] are written by
+ *      the thread of slot 0 of e only and read by no thread of the launch.  The caller copies
+ *      nped_out -> nped and cand_nped -> cand_nped_prev on the same stream after the launch,
+ *      before anything reads the counts (cudaErrorInvalidValue if nped_out == nped or
+ *      cand_nped == cand_nped_prev);
+ *   5. the navgym_peds_advance call that turns cand_rows into discs_reset / segs_reset takes the
+ *      copied candidate counts as its nped, so the first scan after an auto-reset or
+ *      navgym_reset_envs sees exactly the pedestrians the next call adopts. */
 int navgym_peds_plan(const navgym_plan_args_t *args, void *stream);
 
 /* env.py:655-662 + 237-255 for every pedestrian: clip the policy mean to [0, 1] x [-1, 1] (kept

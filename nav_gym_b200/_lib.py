@@ -144,7 +144,9 @@ class PlanArgs(C.Structure):
                 ('cand_pose', _P), ('cand_v_pref', _P), ('cand_legs', _P), ('cand_goal', _P), ('cand_rows', _P),
                 ('robot_maps', _P), ('spawn_pool', _P), ('episodes', _P), ('robot_seed', C.c_uint64),
                 ('num_maps', C.c_int32), ('resample_map', C.c_int32),
-                ('cand_next_spawn', C.c_int32), ('_pad2', C.c_int32)]
+                ('cand_next_spawn', C.c_int32), ('_pad2', C.c_int32),
+                ('num_humans_lo', C.c_int32), ('num_humans_hi', C.c_int32),
+                ('cand_nped_prev', _P), ('cand_nped', _P), ('nped_out', _P)]
 
 
 class MoveArgs(C.Structure):

@@ -331,7 +331,17 @@ int navgym_peds_plan(const navgym_plan_args_t *args, void *stream)
                             !args->dist_travelled || !args->vel || !args->prev_action || !args->cand_v_pref ||
                             !args->cand_legs || !args->cand_goal || !args->cand_rows))
         return (int)cudaErrorInvalidValue;
-    peds_plan_kernel<<<(n + 127) / 128, 128, 0, (cudaStream_t)stream>>>(*args);
+    const int lo = args->num_humans_lo, hi = args->num_humans_hi;
+    if (lo < 0 || lo > hi || hi > args->max_ped) return (int)cudaErrorInvalidValue;
+    // per-episode counts: the launch reads nped / cand_nped_prev and writes the other two
+    if (hi > 0 && (!args->nped || !args->cand_pose || !args->cand_nped_prev || !args->cand_nped || !args->nped_out ||
+                   (const void *)args->nped_out == (const void *)args->nped ||
+                   (const void *)args->cand_nped == (const void *)args->cand_nped_prev))
+        return (int)cudaErrorInvalidValue;
+    if (hi > 0)
+        peds_plan_kernel<true><<<(n + 127) / 128, 128, 0, (cudaStream_t)stream>>>(*args);
+    else
+        peds_plan_kernel<false><<<(n + 127) / 128, 128, 0, (cudaStream_t)stream>>>(*args);
     g_launches++;
     return (int)cudaGetLastError();
 }

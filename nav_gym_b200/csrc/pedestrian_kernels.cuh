@@ -256,73 +256,95 @@ __device__ __forceinline__ bool plan_advance(const uint16_t *f, const navgym_pla
     return true;
 }
 
+// COUNTS: per-episode pedestrian counts (num_humans_hi > 0); without them the kernel is the
+// fixed-count one, instruction for instruction.
+template <bool COUNTS>
 __global__ void peds_plan_kernel(const navgym_plan_args_t a)
 {
     const int n = blockIdx.x * blockDim.x + threadIdx.x;
     if (n >= a.num_envs * a.max_ped) return;
     const int e = n / a.max_ped, slot = n - e * a.max_ped;
-    if (a.nped && slot >= a.nped[e]) return;
-    const navgym_plan_map_t m = a.maps[a.map_id[e]];
-    if (a.respawn && a.respawn[e] && a.cand_pose) {
-        // env.py:785-806: the pedestrian drawn for this episode by the previous call
-        for (int i = 0; i < 3; i++) a.pose_rw[3 * (size_t)n + i] = a.cand_pose[3 * (size_t)n + i];
-        a.v_pref[n] = a.cand_v_pref[n];
-        a.has_legs[n] = a.cand_legs[n];
-        a.goal_id[n] = a.cand_goal[n];
-        a.waypoint[2 * (size_t)n] = CUDART_NAN;
-        a.waypoint[2 * (size_t)n + 1] = CUDART_NAN;
-        for (int i = 0; i < 3; i++) a.dist_travelled[3 * (size_t)n + i] = 0.0;
-        a.vel[2 * (size_t)n] = a.vel[2 * (size_t)n + 1] = 0.0;
-        a.prev_action[2 * (size_t)n] = a.prev_action[2 * (size_t)n + 1] = 0.0f;
-    }
-    const double px = a.pose[3 * (size_t)n], py = a.pose[3 * (size_t)n + 1], th = a.pose[3 * (size_t)n + 2];
-    const int cx = plan_cell(px, m.ox, m.res, m.W), cy = plan_cell(py, m.oy, m.res, m.H);
-    const size_t fsz = (size_t)m.W * m.H;
-    int g = a.goal_id[n];
-    const double *goals = a.goals + 2 * m.goal_offset;
-    double gx = goals[2 * g], gy = goals[2 * g + 1];
-    double wx = a.waypoint[2 * (size_t)n], wy = a.waypoint[2 * (size_t)n + 1];
-    // 1. arrived (env.py:666-668): a new goal, if one qualifies
-    if ((px - gx) * (px - gx) + (py - gy) * (py - gy) < 0.25) {
-        const uint4 r = philox4x32_10(make_uint4((uint32_t)(a.env_offset + e), (uint32_t)slot, (uint32_t)a.step, 0x9ed5u),
+    int live = a.max_ped, next = a.max_ped;  // slots simulated in this episode / drawn for the next
+    if constexpr (COUNTS) {
+        // An environment's slots can span two CTAs, so no thread may write what another one
+        // reads: every thread of e reads nped[e] and cand_nped_prev[e], which the launch never
+        // writes; the thread of slot 0 writes nped_out[e] and cand_nped[e], which no thread of the
+        // launch reads.  The caller copies them over nped / cand_nped_prev afterwards.
+        live = a.respawn && a.respawn[e] ? a.cand_nped_prev[e] : a.nped[e];
+        const uint4 r = philox4x32_10(make_uint4((uint32_t)(a.env_offset + e), 0u, (uint32_t)a.step, 0x5b0eu),
                                       make_uint2((uint32_t)a.seed, (uint32_t)(a.seed >> 32)));
-        const uint32_t draws[4] = {r.x, r.y, r.z, r.w};
-        for (int i = 0; i < 4; i++) {
-            const int c = (int)(((uint64_t)draws[i] * (uint64_t)m.num_goals) >> 32);
-            const double qx = goals[2 * c], qy = goals[2 * c + 1];
-            const double dd = (qx - px) * (qx - px) + (qy - py) * (qy - py);
-            if (c != g && dd > a.min_goal_dist * a.min_goal_dist &&
-                a.fields[m.field_offset + c * fsz + (size_t)cy * m.W + cx] != 65535u) {
-                g = c; gx = qx; gy = qy;
-                wx = CUDART_NAN;
-                break;
+        next = a.num_humans_lo + (int)(((uint64_t)r.x * (uint64_t)(a.num_humans_hi - a.num_humans_lo + 1)) >> 32);
+        if (slot == 0) {
+            a.nped_out[e] = live;
+            a.cand_nped[e] = next;
+        }
+        if (slot >= live && slot >= next) return;
+    } else {
+        if (a.nped && slot >= a.nped[e]) return;
+    }
+    if (!COUNTS || slot < live) {
+        const navgym_plan_map_t m = a.maps[a.map_id[e]];
+        if (a.respawn && a.respawn[e] && a.cand_pose) {
+            // env.py:785-806: the pedestrian drawn for this episode by the previous call
+            for (int i = 0; i < 3; i++) a.pose_rw[3 * (size_t)n + i] = a.cand_pose[3 * (size_t)n + i];
+            a.v_pref[n] = a.cand_v_pref[n];
+            a.has_legs[n] = a.cand_legs[n];
+            a.goal_id[n] = a.cand_goal[n];
+            a.waypoint[2 * (size_t)n] = CUDART_NAN;
+            a.waypoint[2 * (size_t)n + 1] = CUDART_NAN;
+            for (int i = 0; i < 3; i++) a.dist_travelled[3 * (size_t)n + i] = 0.0;
+            a.vel[2 * (size_t)n] = a.vel[2 * (size_t)n + 1] = 0.0;
+            a.prev_action[2 * (size_t)n] = a.prev_action[2 * (size_t)n + 1] = 0.0f;
+        }
+        const double px = a.pose[3 * (size_t)n], py = a.pose[3 * (size_t)n + 1], th = a.pose[3 * (size_t)n + 2];
+        const int cx = plan_cell(px, m.ox, m.res, m.W), cy = plan_cell(py, m.oy, m.res, m.H);
+        const size_t fsz = (size_t)m.W * m.H;
+        int g = a.goal_id[n];
+        const double *goals = a.goals + 2 * m.goal_offset;
+        double gx = goals[2 * g], gy = goals[2 * g + 1];
+        double wx = a.waypoint[2 * (size_t)n], wy = a.waypoint[2 * (size_t)n + 1];
+        // 1. arrived (env.py:666-668): a new goal, if one qualifies
+        if ((px - gx) * (px - gx) + (py - gy) * (py - gy) < 0.25) {
+            const uint4 r = philox4x32_10(make_uint4((uint32_t)(a.env_offset + e), (uint32_t)slot, (uint32_t)a.step, 0x9ed5u),
+                                          make_uint2((uint32_t)a.seed, (uint32_t)(a.seed >> 32)));
+            const uint32_t draws[4] = {r.x, r.y, r.z, r.w};
+            for (int i = 0; i < 4; i++) {
+                const int c = (int)(((uint64_t)draws[i] * (uint64_t)m.num_goals) >> 32);
+                const double qx = goals[2 * c], qy = goals[2 * c + 1];
+                const double dd = (qx - px) * (qx - px) + (qy - py) * (qy - py);
+                if (c != g && dd > a.min_goal_dist * a.min_goal_dist &&
+                    a.fields[m.field_offset + c * fsz + (size_t)cy * m.W + cx] != 65535u) {
+                    g = c; gx = qx; gy = qy;
+                    wx = CUDART_NAN;
+                    break;
+                }
             }
+            a.goal_id[n] = g;
         }
-        a.goal_id[n] = g;
-    }
-    const uint16_t *f = a.fields + m.field_offset + g * fsz;
-    // 2. / 3. the waypoint: first one from here, later ones from the previous waypoint
-    bool is_goal = (wx == gx) & (wy == gy);
-    if (wx != wx) {
-        if (!plan_advance(f, m, cx, cy, px, py, wx, wy, is_goal)) { wx = gx; wy = gy; is_goal = true; }
-        if (is_goal) { wx = gx; wy = gy; }
-    }
-    for (int it = 0; it < 8 && !is_goal && (px - wx) * (px - wx) + (py - wy) * (py - wy) < 1.0; it++) {
-        const double sx = wx, sy = wy;
-        if (!plan_advance(f, m, plan_cell(sx, m.ox, m.res, m.W), plan_cell(sy, m.oy, m.res, m.H), sx, sy, wx, wy, is_goal)) {
-            is_goal = true;
+        const uint16_t *f = a.fields + m.field_offset + g * fsz;
+        // 2. / 3. the waypoint: first one from here, later ones from the previous waypoint
+        bool is_goal = (wx == gx) & (wy == gy);
+        if (wx != wx) {
+            if (!plan_advance(f, m, cx, cy, px, py, wx, wy, is_goal)) { wx = gx; wy = gy; is_goal = true; }
+            if (is_goal) { wx = gx; wy = gy; }
         }
-        if (is_goal) { wx = gx; wy = gy; }
+        for (int it = 0; it < 8 && !is_goal && (px - wx) * (px - wx) + (py - wy) * (py - wy) < 1.0; it++) {
+            const double sx = wx, sy = wy;
+            if (!plan_advance(f, m, plan_cell(sx, m.ox, m.res, m.W), plan_cell(sy, m.oy, m.res, m.H), sx, sy, wx, wy, is_goal)) {
+                is_goal = true;
+            }
+            if (is_goal) { wx = gx; wy = gy; }
+        }
+        a.waypoint[2 * (size_t)n] = wx;
+        a.waypoint[2 * (size_t)n + 1] = wy;
+        // env.py:641-645: the goal in the pedestrian's frame
+        const double c = cos(th), s = sin(th);
+        a.goal_local[2 * (size_t)n] = (float)((wx - px) * c + (wy - py) * s);
+        a.goal_local[2 * (size_t)n + 1] = (float)(-(wx - px) * s + (wy - py) * c);
     }
-    a.waypoint[2 * (size_t)n] = wx;
-    a.waypoint[2 * (size_t)n + 1] = wy;
-    // env.py:641-645: the goal in the pedestrian's frame
-    const double c = cos(th), s = sin(th);
-    a.goal_local[2 * (size_t)n] = (float)((wx - px) * c + (wy - py) * s);
-    a.goal_local[2 * (size_t)n + 1] = (float)(-(wx - px) * s + (wy - py) * c);
 
     // ---- the pedestrian of this slot in the environment's next episode
-    if (a.cand_pose) {
+    if (a.cand_pose && (!COUNTS || slot < next)) {
         const size_t B = (size_t)a.num_envs;
         const uint32_t ge = (uint32_t)(a.env_offset + e);
         double rx = a.robot_state[NAVGYM_S_PX * B + e], ry = a.robot_state[NAVGYM_S_PY * B + e];

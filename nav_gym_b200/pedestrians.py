@@ -17,6 +17,7 @@ Everything on the per-step path is a kernel of the library, the policy forward i
 torch owns the device memory.  Nothing here touches the CPU oracle.
 """
 import ctypes as C
+import operator
 
 import numpy as np
 import torch
@@ -236,10 +237,18 @@ class PedestrianSim(object):
     first observation of a new episode already sees the new pedestrians; the next act() adopts
     them for the environments whose episode ended.  Over an auto_reset=False env, step and read
     the final observations, then sim.reset_envs(env.done) does the same for those environments.
+
+    Pedestrian counts: `nped` (int32 [num_envs], None = max_ped) fixes each environment's count
+    for the sim's whole life.  `num_humans_range=(lo, hi)` instead draws every episode's count
+    uniformly from lo..hi (inclusive), as NavGym-v0 draws num_humans: at reset(), with each
+    auto-reset and with each reset_envs().  sim.nped (= env.nped) then always holds the current
+    episodes' counts, and sim.cand_nped those of the next episodes, whose pedestrians the
+    candidates are (None without a range).  Slots at or beyond an environment's count are not
+    simulated, scanned or emitted.
     """
 
     def __init__(self, env, max_ped, nped=None, policy=None, v_pref_range=(0.0, 0.6), has_legs_ratio=0.5,
-                 num_goals=32, min_goal_dist=10.0, min_robot_dist=4.0, seed=0):
+                 num_goals=32, min_goal_dist=10.0, min_robot_dist=4.0, seed=0, num_humans_range=None):
         from . import maps as M
         if env.args.auto_reset == _lib.AUTORESET_NEXT_STEP:
             # act() respawns the pedestrians of an env in the launch that ends its episode
@@ -248,11 +257,24 @@ class PedestrianSim(object):
         self.B, self.P = env.B, int(max_ped)
         if self.P > 127:  # navgym_agent_scan_batch, crowd mode: one thread per other agent
             raise ValueError('at most 127 pedestrians per environment')
+        if num_humans_range is not None:
+            if nped is not None:
+                raise ValueError('give nped or num_humans_range, not both')
+            lo, hi = (operator.index(v) for v in num_humans_range)
+            if not 0 <= lo <= hi <= self.P:
+                raise ValueError('num_humans_range=(%d, %d): need 0 <= lo <= hi <= max_ped = %d' % (lo, hi, self.P))
         self.dt = float(env.args.dt)
         self.lib = _lib.load()
         dev, f64, f32, i32 = self.device, torch.float64, torch.float32, torch.int32
         B, P = self.B, self.P
         self.nped = None if nped is None else torch.as_tensor(nped, dtype=i32).to(dev)
+        self.cand_nped = self._counts = self._counts_out = None
+        if num_humans_range is not None:
+            # [nped; cand_nped], which navgym_peds_plan reads, and the two it writes in their
+            # place: _plan copies the second pair over the first after each launch
+            self._counts = torch.zeros(2, B, dtype=i32, device=dev)
+            self._counts_out = torch.zeros(2, B, dtype=i32, device=dev)
+            self.nped, self.cand_nped = self._counts[0], self._counts[1]
         if policy is None:
             policy = HumanPolicy()
         self.policy = policy.to(dev).eval()
@@ -325,6 +347,10 @@ class PedestrianSim(object):
         self.cand_rows = torch.zeros(B, P, _lib.PED_F, dtype=f32, device=dev)
         a.cand_pose, a.cand_v_pref, a.cand_legs = _ptr(self.cand_pose), _ptr(self.cand_v_pref), _ptr(self.cand_legs)
         a.cand_goal, a.cand_rows = _ptr(self.cand_goal), _ptr(self.cand_rows)
+        if num_humans_range is not None:
+            a.num_humans_lo, a.num_humans_hi = lo, hi
+            a.cand_nped_prev, a.cand_nped = _ptr(self.cand_nped), _ptr(self._counts_out[1])
+            a.nped_out = _ptr(self._counts_out[0])
         ea = env.args
         a.robot_maps, a.spawn_pool, a.episodes = ea.maps, ea.spawn_pool, ea.episodes
         a.robot_seed, a.num_maps, a.resample_map = ea.seed, ea.num_maps, ea.resample_map
@@ -338,6 +364,8 @@ class PedestrianSim(object):
         cp.advance = 0
         cp.peds, cp.discs, cp.ndisc = _ptr(self.cand_rows), _ptr(self.cand_discs), _ptr(self.cand_nd)
         cp.segs, cp.nseg = _ptr(self.cand_segs), _ptr(self.cand_ns)
+        if self.cand_nped is not None:
+            cp.nped = _ptr(self.cand_nped)  # the reset scan sees the next episode's count
         self.cand_pargs = cp
         # (the step reads them only on auto-reset; navgym_reset_envs reads them in sim.reset_envs)
         ea.discs_reset, ea.ndisc_reset = _ptr(self.cand_discs), _ptr(self.cand_nd)
@@ -371,6 +399,9 @@ class PedestrianSim(object):
         a.respawn = _ptr(respawn)
         a.cand_next_spawn = int(bool(next_spawn))
         self._call(self.lib.navgym_peds_plan, a, 'peds_plan')
+        if self._counts is not None:
+            with torch.cuda.device(self.device):
+                self._counts.copy_(self._counts_out)  # same stream, before anything reads the counts
         a.step += 1
         self._call(self.lib.navgym_peds_advance, self.cand_pargs, 'peds_advance')  # candidates' geometry
 
